@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA, sm_100a)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU arithmetic (oracle port)
+    python bench.py ... --dump-outputs DIR                   # also write the outputs of the last timed launch to DIR
 
 One bench "step" = ONE fused rollout launch (K4) over this rank's environments:
 2^20 envs x 64 env-steps, RECORD mode (reads float32 actions [64,N,2], writes the trajectory
@@ -66,7 +67,15 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-sample-envs", type=int, default=1 << 17)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed launches, write what the last one returned to DIR/<name>.npy (rank 0): the "
+                         "record planes and final joints of a fixed, seeded sample of envs, and the episode statistics")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 def peaks():
@@ -363,6 +372,28 @@ def time_config(args, ag, torch, dist, name, rank, world, dev, actions, rec, ste
     return res, scene
 
 
+DUMP_BYTES = 48 << 20
+
+
+def dump_outputs(path, scene, rec, K):
+    """Write what the last rollout launch handed its caller, as float32 / float64 .npy files: the [K, m] record planes
+    and the final joint angles of m envs drawn once with a fixed seed (m fits all of it in DUMP_BYTES), and the
+    cumulative episode statistics.  Two builds run with the same arguments can be compared file by file."""
+    import numpy as np
+    import torch
+    n = scene.n
+    m = min(n, 1 << 15, DUMP_BYTES // (16 * K + 16))
+    envs = torch.as_tensor(np.sort(np.random.default_rng(0).choice(n, m, replace=False)), device=scene.device)
+    out = {"joint_1": scene.robot.joint_1[envs].double(), "joint_2": scene.robot.joint_2[envs].double(),
+           "episode_stats": scene.stats.double()}
+    if rec is not None:
+        for k in ("j1", "j2", "reward", "flags"):
+            out["rec_" + k] = rec[k][:, envs].float()
+    os.makedirs(path, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
+
+
 def e2e_leg(args, ag, torch, dist, scene, rank, world, dev, actions):
     """The same metric end to end through the public API with HOST buffers, copies inside the timed region."""
     n, K = args.envs, args.rollout_steps
@@ -387,7 +418,7 @@ def e2e_leg(args, ag, torch, dist, scene, rank, world, dev, actions):
             dist.all_reduce(tt, op=dist.ReduceOp.MAX)
         return float(tt.item())
 
-    reps = max(2, min(args.steps, 5))
+    reps = args.steps
     out = {}
     # (a) full records: host actions in (8 B / env-step), all four record planes out (13 B / env-step)
     if record:
@@ -445,6 +476,8 @@ def run_ours(args, rank, world, local):
     wall_load0 = time.time()
     # ---- headline
     head, scene = time_config(args, ag, torch, dist, args.grid, rank, world, dev, actions, rec, args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, scene, rec, K)
     # one more launch with the filter diagnostics on (outside every timed region)
     scene.diag.zero_()
     scene.rollout(K, actions=actions, record=record, out=rec, diag=True)
