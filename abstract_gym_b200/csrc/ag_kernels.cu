@@ -14,6 +14,10 @@ bool rollout_lut_applies(const ag_params &P, const GridDev &G, const RolloutDev 
 ag_status launch_rollout_lut(const ag_params &P, const GridDev &G, const RolloutDev &A, size_t smem, cudaStream_t s);
 int64_t cspace_map_words(int32_t *b1, int32_t *b2);
 ag_status launch_cspace_map(const ag_params &P, const GridDev &G, uint32_t *map, cudaStream_t s);
+// ag_motion.cu: batched motion checking (ag_check_motion after argument validation)
+ag_status launch_check_motion(const ag_params &P, const GridDev &G, int32_t max_occupied, const double *j1, const double *j2,
+                              const double *goal, const int32_t *steps, int32_t *first_collision, int32_t *first_hit,
+                              double *last_free, int64_t m, int64_t env_id0, int32_t engine, size_t smem, cudaStream_t s);
 // ag_dense.cu: the warp-cooperative kernel for grids that go through the cell traversal (needs the transposed planes)
 bool rollout_coop_applies(const ag_params &P, const GridDev &G, const RolloutDev &A);
 ag_status launch_rollout_coop(const ag_params &P, const GridDev &G, const RolloutDev &A, size_t smem, cudaStream_t s);
@@ -968,6 +972,22 @@ ag_status ag_collision_check(const ag_params *p, const ag_grid *g, const double 
         }
     });
     return launched();
+}
+
+ag_status ag_check_motion(const ag_params *p, const ag_grid *g, const double *j1, const double *j2, const double *goal,
+                          const int32_t *steps, int32_t *first_collision, int32_t *first_hit, double *last_free, int64_t m,
+                          int64_t env_id0, int32_t engine, void *stream) {
+    if (m < 0) return AG_ERR_SHAPE;
+    if (!p || !g) return AG_ERR_NULL;
+    GridDev G;
+    size_t smem;
+    ag_status st = make_grid_dev(p, g, env_id0, engine, &G, &smem);
+    if (st) return st;
+    if (m == 0) return AG_OK;
+    if (!j1 || !j2 || !goal || !steps || !first_collision) return AG_ERR_NULL;
+    if (((uintptr_t)goal % 16) || ((uintptr_t)last_free % 16)) return AG_ERR_ALIGN;
+    return launch_check_motion(*p, G, g->max_occupied, j1, j2, goal, steps, first_collision, first_hit, last_free, m, env_id0,
+                               engine, smem, (cudaStream_t)stream);
 }
 
 ag_status ag_step(const ag_params *p, const ag_grid *g, double *j1, double *j2, const void *actions,

@@ -52,16 +52,7 @@ namespace {
 #define AG_LUT_BLOCKS_PER_SM 1
 #endif
 
-// configuration-space map (CMAP form of the kernel): 2^CB1 x 2^CB2 bins over (joint_1, joint_2) mod 2pi, one bit each
-#ifndef AG_CMAP_B1
-#define AG_CMAP_B1 10
-#endif
-#ifndef AG_CMAP_B2
-#define AG_CMAP_B2 8
-#endif
-constexpr int CB1 = AG_CMAP_B1, CB2 = AG_CMAP_B2;
-static_assert(CB1 >= 6 && CB2 >= 6 && CB1 + CB2 <= 20, "the map must fit shared memory");
-constexpr int CMAP_WORDS = 1 << (CB1 + CB2 - 5);
+// configuration-space map (CMAP form of the kernel): CB1, CB2, CMAP_WORDS in ag_rollout.cuh
 constexpr int CMAP_HDR_WORDS = 64;                       // 256-byte header in front of the map words
 constexpr int CMAP_SLOTS = 16;
 struct CmapHeader {
@@ -97,8 +88,6 @@ static_assert((AG_LUT_RING & (AG_LUT_RING - 1)) == 0 && AG_LUT_RING >= 4, "ring 
 #endif
 static_assert((AG_CMAP_RING & (AG_CMAP_RING - 1)) == 0 && AG_CMAP_RING >= 4, "ring slots: a power of two");
 
-constexpr double PHASE_MAGIC = 6755399441055744.0;       // 1.5 * 2^52: the add rounds to an integer in the low word
-constexpr double TWO_PI = 6.283185307179586476925;
 constexpr float RAD_PER_UNIT = (float)(TWO_PI / 4294967296.0);   // one phase unit (2^-32 turn) in radians
 // d = fma(2^23 + frac, RAD_PER_UNIT, C0): removes the 2^23 of the integer -> float trick and half a bin
 __host__ __device__ constexpr float lut_c0(int bits) { return (float)(-(8388608.0 * (double)RAD_PER_UNIT + TWO_PI / (double)(2 << bits))); }
@@ -907,7 +896,7 @@ bool rollout_lut_applies(const ag_params &P, const GridDev &G, const RolloutDev 
     // the table arm's error (2.2e-7 m per metre of link 1, 2.8e-7 per metre of link 2, 5e-8 of rounding) must stay
     // inside the float32 filter's budget AG_DELTA_P
     const bool budget = 2.2e-7 * P.link_1 + 2.8e-7 * P.link_2 + 5.0e-8 <= (double)AG_DELTA_P;
-    return !legacy && G.stage && G.n_grids == 1 && G.S <= 32 && !P.choose_j_tar && (!rec || A.zfill) && budget;
+    return !legacy && cspace_map_applies(G, A.max_occupied) && !P.choose_j_tar && (!rec || A.zfill) && budget;
 }
 
 // ---- the library-owned buffers of the configuration-space maps: up to 32 entries (33 KB each) per process, found by (device, grid
@@ -966,6 +955,23 @@ uint32_t *cmap_buffer(const ag_params &P, const GridDev &G, cudaStream_t s) {
 }
 }  // namespace
 
+bool cspace_map_applies(const GridDev &G, int32_t max_occupied) {
+    return G.stage && G.n_grids == 1 && G.S <= 32 && max_occupied >= 0 && max_occupied <= AG_LIST_MAX;
+}
+
+ag_status cspace_map_for_launch(const ag_params &P, const GridDev &G, cudaStream_t s, const uint32_t **map) {
+    *map = nullptr;
+    uint32_t *buf = cmap_buffer(P, G, s);
+    if (buf == nullptr) return AG_OK;
+    static std::atomic<unsigned> next_build{0};
+    k_cspace_build<<<CMAP_BUILD_BLOCKS, 256, 0, s>>>(P, G, buf, next_build.fetch_add(1, std::memory_order_relaxed) % CMAP_SLOTS);
+    ag_note_launch();
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return (ag_status)e;
+    *map = buf + CMAP_HDR_WORDS;
+    return AG_OK;
+}
+
 int64_t cspace_map_words(int32_t *b1, int32_t *b2) {
     if (b1) *b1 = CB1;
     if (b2) *b2 = CB2;
@@ -1004,14 +1010,9 @@ ag_status launch_rollout_lut(const ag_params &P, const GridDev &G, const Rollout
     static const bool no_cmap = std::getenv("AG_ROLLOUT_NO_CMAP") != nullptr;
     L.cmap = nullptr; L.cmap_off = 0;
     if (!no_cmap && A.targets == nullptr) {
-        uint32_t *buf = cmap_buffer(P, G, s);
-        if (buf != nullptr) {
-            static std::atomic<unsigned> next_build{0};
-            k_cspace_build<<<CMAP_BUILD_BLOCKS, 256, 0, s>>>(P, G, buf, next_build.fetch_add(1, std::memory_order_relaxed) % CMAP_SLOTS);
-            ag_note_launch();
-            cudaError_t e = cudaGetLastError();
-            if (e != cudaSuccess) return (ag_status)e;
-            L.cmap = buf + CMAP_HDR_WORDS;
+        const ag_status st = cspace_map_for_launch(P, G, s, &L.cmap);
+        if (st != AG_OK) return st;
+        if (L.cmap != nullptr) {
             L.cmap_off = (uint32_t)((smem + 15) & ~(size_t)15);
             smem = (size_t)L.cmap_off + (size_t)CMAP_WORDS * 4;
         }

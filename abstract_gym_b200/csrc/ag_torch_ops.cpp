@@ -92,6 +92,29 @@ void collision_check(const Tensor &params, const Tensor &bits, const OptTensor &
                                     (int32_t)engine, stream_of(dev)), "ag_collision_check");
 }
 
+// move_to_joint_pose with a collision check at every pose (two_joint_robot.py:49-62, scene_0.py:60-76) -> ag_check_motion
+void check_motion(const Tensor &params, const Tensor &bits, const OptTensor &bits_t, const OptTensor &hier, const Tensor &min_x,
+                  const Tensor &min_y, double side, double env_size, int64_t S, int64_t n_grids, int64_t max_occupied,
+                  int64_t envs_per_grid, const Tensor &j1, const Tensor &j2, const Tensor &goal, const Tensor &steps,
+                  Tensor first_collision, OptTensor first_hit, OptTensor last_free, int64_t env_id0, int64_t engine) {
+    const c10::Device dev = j1.device();
+    c10::cuda::CUDAGuard guard(dev);
+    need(j1, at::kDouble, "j1", dev); need(j2, at::kDouble, "j2", dev); need(goal, at::kDouble, "goal", dev);
+    need(steps, at::kInt, "steps", dev); need(first_collision, at::kInt, "first_collision", dev);
+    const int64_t m = j1.numel();
+    TORCH_CHECK(j2.numel() == m && steps.numel() == m && first_collision.numel() == m, "j1, j2, steps, first_collision must have one element per motion");
+    TORCH_CHECK(goal.numel() == 2 * m, "goal must be [M,2]");
+    if (first_hit.has_value() && first_hit->defined()) TORCH_CHECK(first_hit->numel() == m, "first_hit must be [M]");
+    if (last_free.has_value() && last_free->defined()) TORCH_CHECK(last_free->numel() == 2 * m, "last_free must be [M,2]");
+    const ag_params p = unpack_params(params);
+    const ag_grid g = make_grid(bits, bits_t, hier, min_x, min_y, side, env_size, S, n_grids, max_occupied, envs_per_grid, dev);
+    check_status(ag_check_motion(&p, &g, j1.data_ptr<double>(), j2.data_ptr<double>(), goal.data_ptr<double>(),
+                                 steps.data_ptr<int32_t>(), first_collision.data_ptr<int32_t>(),
+                                 opt_ptr<int32_t>(first_hit, at::kInt, "first_hit", dev), opt_ptr<double>(last_free, at::kDouble, "last_free", dev),
+                                 m, env_id0, (int32_t)engine, stream_of(dev)),
+                 "ag_check_motion");
+}
+
 // Scene.step (scenario/scene_0.py:88-103) -> ag_step
 void step(const Tensor &params, const Tensor &bits, const OptTensor &bits_t, const OptTensor &hier, const Tensor &min_x, const Tensor &min_y, double side,
           double env_size, int64_t S, int64_t n_grids, int64_t max_occupied, int64_t envs_per_grid, Tensor j1, Tensor j2,
@@ -225,6 +248,8 @@ void step_obs(const Tensor &params, const Tensor &bits, const OptTensor &bits_t,
 
 TORCH_LIBRARY(abstract_gym_b200, m) {
     m.def("collision_check(" AG_GRID_SCHEMA "Tensor j1, Tensor j2, Tensor(a!) hit, Tensor(b!)? first_hit, int env_id0, int engine) -> ()");
+    m.def("check_motion(" AG_GRID_SCHEMA "Tensor j1, Tensor j2, Tensor goal, Tensor steps, Tensor(a!) first_collision, "
+          "Tensor(b!)? first_hit, Tensor(c!)? last_free, int env_id0, int engine) -> ()");
     m.def("step(" AG_GRID_SCHEMA "Tensor(a!) j1, Tensor(b!) j2, Tensor actions, Tensor(c!) reward, Tensor(d!) flags, Tensor(e!)? ee, "
           "Tensor(f!)? dist, Tensor(g!)? first_hit, Tensor(h!)? stats, Tensor? targets, int env_id0, int engine) -> ()");
     m.def("reset(" AG_GRID_SCHEMA "Tensor(a!) j1, Tensor(b!) j2, Tensor(c!) reward, Tensor(d!) flags, Tensor(e!) reset_ctr, Tensor? mask, "
@@ -241,6 +266,7 @@ TORCH_LIBRARY(abstract_gym_b200, m) {
 
 TORCH_LIBRARY_IMPL(abstract_gym_b200, CUDA, m) {
     m.impl("collision_check", &collision_check);
+    m.impl("check_motion", &check_motion);
     m.impl("step", &step);
     m.impl("reset", &reset);
     m.impl("rollout", &rollout);

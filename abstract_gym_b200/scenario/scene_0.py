@@ -138,6 +138,39 @@ class BatchedScene:
                                                 stream_ptr(self.device)), "ag_collision_check")
         return (hit != 0, fh) if first_hit else hit != 0
 
+    def check_motion(self, goal, start=None, steps=100, first_hit=False, last_free=False, engine=None):
+        """robot/two_joint_robot.py:49-62 move_to_joint_pose() with collision_check() (scene_0.py:60-76) at every
+        intermediate pose, for M motions; nothing is moved.  Motion i goes from start[i] (default: the current joints,
+        M = N) to goal[i] in steps[i] increments, pose_k = pose_{k-1} + (1/steps)*(goal - start), and stops at its
+        first colliding pose; the start pose is not checked.  Motion i uses the grid of env i.
+        goal, start: [M,2] float64; steps: int or int32 [M].
+        Returns first_collision int32 [M]: the smallest colliding k, -1 if the motion is free, -2 if steps < 1; with
+        first_hit / last_free also a dict: first_hit int32 [M] (min hit cell index at that pose, -1 if none) and
+        last_free float64 [M,2] (the last pose before the first collision: RRT's "steer until blocked")."""
+        if start is None:
+            j1, j2 = self.robot.joint_1, self.robot.joint_2
+        else:
+            st = as_f64(start, self.device).reshape(-1, 2)
+            j1, j2 = st[:, 0].contiguous(), st[:, 1].contiguous()
+        m = j1.numel()
+        goal = as_f64(goal, self.device).reshape(m, 2).contiguous()
+        if isinstance(steps, torch.Tensor):
+            if steps.dtype != torch.int32 or steps.numel() != m:
+                raise ValueError("steps must be an int or an int32 tensor with one entry per motion")
+            steps = steps.to(self.device).reshape(m).contiguous()
+        else:
+            steps = torch.full((m,), int(steps), dtype=torch.int32, device=self.device)
+        fc = torch.empty(m, dtype=torch.int32, device=self.device)
+        fh = torch.empty(m, dtype=torch.int32, device=self.device) if first_hit else None
+        lf = torch.empty(m, 2, dtype=torch.float64, device=self.device) if last_free else None
+        g = self.grid.c_struct()
+        _lib.check(self._lib.ag_check_motion(self.params(), g, ptr(j1), ptr(j2), ptr(goal), ptr(steps), ptr(fc), ptr(fh),
+                                             ptr(lf), m, self.env_id0, self.engine if engine is None else _engine(engine),
+                                             stream_ptr(self.device)), "ag_check_motion")
+        if first_hit or last_free:
+            return fc, dict(first_hit=fh, last_free=lf)
+        return fc
+
     def check_target_reached(self):
         """scene_0.py:115-133 -> bool [N]"""
         eps = 2e-3

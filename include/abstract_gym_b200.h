@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define AG_ABI_VERSION 5
+#define AG_ABI_VERSION 6
 
 #if defined(__GNUC__)
 #define AG_API __attribute__((visibility("default")))
@@ -179,6 +179,25 @@ AG_API ag_status ag_move_to_joint_pose(double *j1, double *j2, const double *tar
 AG_API ag_status ag_collision_check(const ag_params *p, const ag_grid *g, const double *j1, const double *j2,
                              uint8_t *hit, int32_t *first_hit, int64_t n, int64_t env_id0,
                              int32_t engine, void *stream);
+
+/* Motion checking: robot/two_joint_robot.py:49-62 move_to_joint_pose() with scenario/scene_0.py:60-76
+ * Scene.collision_check() at every intermediate pose (the reference checks none of them).  Motion i starts at
+ * (j1[i], j2[i]) and goes to goal[i] = (g1, g2) in n = steps[i] increments: alpha = 1.0 / n, inc = alpha * (g - start),
+ * pose_k = pose_{k-1} + inc for k = 1 .. n, pose_0 = start -- float64, one rounding per operation, the k-fold SEQUENTIAL
+ * sum (not start + k * inc), so a free motion ends exactly where ag_move_to_joint_pose(start, goal, n) does.  The start
+ * pose is not checked (the arm is already there; Scene.step, too, checks only after the move); poses 1 .. n are, and a
+ * pose collides exactly when ag_collision_check with the same engine says so.  Motion i uses grid
+ * ((env_id0 + i) / envs_per_grid) % n_grids.  A motion stops at its first colliding pose.
+ * goal, last_free: [m][2] float64 (16-byte aligned); steps: [m] int32; all device arrays.  Outputs:
+ *   first_collision [m] int32: the smallest colliding k, -1 if the motion is free, -2 if steps[i] < 1 (nothing is
+ *                   checked; the reference divides by zero there);
+ *   first_hit       optional [m] int32: min(row*S+col) over the cells hit at pose first_collision (as K2 reports it),
+ *                   -1 if none;
+ *   last_free       optional [m][2] float64: the last pose before the first collision -- the start when it is pose 1
+ *                   or when steps[i] < 1, pose n when the motion is free. */
+AG_API ag_status ag_check_motion(const ag_params *p, const ag_grid *g, const double *j1, const double *j2, const double *goal,
+                                 const int32_t *steps, int32_t *first_collision, int32_t *first_hit, double *last_free,
+                                 int64_t m, int64_t env_id0, int32_t engine, void *stream);
 
 /* K1: scenario/scene_0.py:88-103  Scene.step(action).  j1,j2,reward,flags are in/out (sticky
  * semantics).  actions: [n][2] float64 (actions_f32 == 0) or float32.  Optional outputs:
