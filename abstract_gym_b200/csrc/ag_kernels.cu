@@ -2,6 +2,7 @@
 // Build: nvcc -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 (abstract_gym_b200/build.py).
 #include <atomic>
 #include <climits>
+#include <cmath>
 #include <cstdlib>
 #include <cstring>
 
@@ -18,6 +19,10 @@ ag_status launch_cspace_map(const ag_params &P, const GridDev &G, uint32_t *map,
 ag_status launch_check_motion(const ag_params &P, const GridDev &G, int32_t max_occupied, const double *j1, const double *j2,
                               const double *goal, const int32_t *steps, int32_t *first_collision, int32_t *first_hit,
                               double *last_free, int64_t m, int64_t env_id0, int32_t engine, size_t smem, cudaStream_t s);
+// ag_cspace.cu: configuration-space occupancy (ag_cspace_occupancy after argument validation)
+ag_status launch_cspace_occupancy(const ag_params &P, const GridDev &G, int32_t max_occupied, double lo1, double step1,
+                                  int32_t b1, double lo2, double step2, int32_t b2, uint32_t *bits, int64_t *free_count,
+                                  int32_t engine, size_t smem, cudaStream_t s);
 // ag_dense.cu: the warp-cooperative kernel for grids that go through the cell traversal (needs the transposed planes)
 bool rollout_coop_applies(const ag_params &P, const GridDev &G, const RolloutDev &A);
 ag_status launch_rollout_coop(const ag_params &P, const GridDev &G, const RolloutDev &A, size_t smem, cudaStream_t s);
@@ -988,6 +993,24 @@ ag_status ag_check_motion(const ag_params *p, const ag_grid *g, const double *j1
     if (((uintptr_t)goal % 16) || ((uintptr_t)last_free % 16)) return AG_ERR_ALIGN;
     return launch_check_motion(*p, G, g->max_occupied, j1, j2, goal, steps, first_collision, first_hit, last_free, m, env_id0,
                                engine, smem, (cudaStream_t)stream);
+}
+
+ag_status ag_cspace_occupancy(const ag_params *p, const ag_grid *g, double lo1, double step1, int32_t b1, double lo2,
+                              double step2, int32_t b2, uint32_t *bits, int64_t *free_count, int32_t engine, void *stream) {
+    if (b1 < 1 || b2 < 1) return AG_ERR_SHAPE;
+    if (!p || !g) return AG_ERR_NULL;
+    GridDev G;
+    size_t smem;
+    ag_status st = make_grid_dev(p, g, 0, engine, &G, &smem);   // env_id0 0: K2's staging choice for a grid's own envs
+    if (st) return st;
+    if (!std::isfinite(lo1) || !std::isfinite(step1) || !std::isfinite(lo2) || !std::isfinite(step2)) return AG_ERR_SHAPE;
+    const int64_t row_words = ((int64_t)b2 + 31) / 32;
+    if ((int64_t)b1 * row_words > INT64_MAX / g->n_grids) return AG_ERR_SHAPE;   // n_grids * b1 * W words must fit int64
+    if (!bits) return AG_ERR_NULL;
+    if (((uintptr_t)bits % 4) || ((uintptr_t)free_count % 8)) return AG_ERR_ALIGN;
+    if (engine != AG_ENGINE_EXACT && engine != AG_ENGINE_FAST && engine != AG_ENGINE_BRUTE) return AG_ERR_MODE;
+    return launch_cspace_occupancy(*p, G, g->max_occupied, lo1, step1, b1, lo2, step2, b2, bits, free_count, engine, smem,
+                                   (cudaStream_t)stream);
 }
 
 ag_status ag_step(const ag_params *p, const ag_grid *g, double *j1, double *j2, const void *actions,

@@ -15,6 +15,8 @@
 #include <c10/cuda/CUDAStream.h>
 #include <torch/library.h>
 
+#include <cstdint>
+
 #include "../../include/abstract_gym_b200.h"
 
 namespace {
@@ -113,6 +115,27 @@ void check_motion(const Tensor &params, const Tensor &bits, const OptTensor &bit
                                  opt_ptr<int32_t>(first_hit, at::kInt, "first_hit", dev), opt_ptr<double>(last_free, at::kDouble, "last_free", dev),
                                  m, env_id0, (int32_t)engine, stream_of(dev)),
                  "ag_check_motion");
+}
+
+// collision_check (scene_0.py:60-76) at every pose of a joint-angle lattice, per grid -> ag_cspace_occupancy
+void cspace_occupancy(const Tensor &params, const Tensor &bits, const OptTensor &bits_t, const OptTensor &hier, const Tensor &min_x,
+                      const Tensor &min_y, double side, double env_size, int64_t S, int64_t n_grids, int64_t max_occupied,
+                      int64_t envs_per_grid, double lo1, double step1, int64_t b1, double lo2, double step2, int64_t b2,
+                      Tensor occupancy, OptTensor free_count, int64_t engine) {
+    const c10::Device dev = occupancy.device();
+    c10::cuda::CUDAGuard guard(dev);
+    need(occupancy, at::kInt, "occupancy", dev);
+    TORCH_CHECK(b1 >= 1 && b2 >= 1 && b1 <= INT32_MAX && b2 <= INT32_MAX, "b1 and b2 must be in [1, 2^31)");
+    const int64_t grid_words = b1 * ((b2 + 31) / 32);
+    TORCH_CHECK(n_grids >= 1 && grid_words <= INT64_MAX / n_grids && occupancy.numel() == n_grids * grid_words,
+                "occupancy must be [n_grids, b1, ceil(b2/32)] int32 words");
+    if (free_count.has_value() && free_count->defined()) TORCH_CHECK(free_count->numel() == n_grids, "free_count must be [n_grids]");
+    const ag_params p = unpack_params(params);
+    const ag_grid g = make_grid(bits, bits_t, hier, min_x, min_y, side, env_size, S, n_grids, max_occupied, envs_per_grid, dev);
+    check_status(ag_cspace_occupancy(&p, &g, lo1, step1, (int32_t)b1, lo2, step2, (int32_t)b2,
+                                     reinterpret_cast<uint32_t *>(occupancy.data_ptr()),
+                                     opt_ptr<int64_t>(free_count, at::kLong, "free_count", dev), (int32_t)engine, stream_of(dev)),
+                 "ag_cspace_occupancy");
 }
 
 // Scene.step (scenario/scene_0.py:88-103) -> ag_step
@@ -250,6 +273,8 @@ TORCH_LIBRARY(abstract_gym_b200, m) {
     m.def("collision_check(" AG_GRID_SCHEMA "Tensor j1, Tensor j2, Tensor(a!) hit, Tensor(b!)? first_hit, int env_id0, int engine) -> ()");
     m.def("check_motion(" AG_GRID_SCHEMA "Tensor j1, Tensor j2, Tensor goal, Tensor steps, Tensor(a!) first_collision, "
           "Tensor(b!)? first_hit, Tensor(c!)? last_free, int env_id0, int engine) -> ()");
+    m.def("cspace_occupancy(" AG_GRID_SCHEMA "float lo1, float step1, int b1, float lo2, float step2, int b2, "
+          "Tensor(a!) occupancy, Tensor(b!)? free_count, int engine) -> ()");
     m.def("step(" AG_GRID_SCHEMA "Tensor(a!) j1, Tensor(b!) j2, Tensor actions, Tensor(c!) reward, Tensor(d!) flags, Tensor(e!)? ee, "
           "Tensor(f!)? dist, Tensor(g!)? first_hit, Tensor(h!)? stats, Tensor? targets, int env_id0, int engine) -> ()");
     m.def("reset(" AG_GRID_SCHEMA "Tensor(a!) j1, Tensor(b!) j2, Tensor(c!) reward, Tensor(d!) flags, Tensor(e!) reset_ctr, Tensor? mask, "
@@ -267,6 +292,7 @@ TORCH_LIBRARY(abstract_gym_b200, m) {
 TORCH_LIBRARY_IMPL(abstract_gym_b200, CUDA, m) {
     m.impl("collision_check", &collision_check);
     m.impl("check_motion", &check_motion);
+    m.impl("cspace_occupancy", &cspace_occupancy);
     m.impl("step", &step);
     m.impl("reset", &reset);
     m.impl("rollout", &rollout);

@@ -7,6 +7,7 @@ argument plumbing.  Visualisation (render / occ_to_patch, scene_0.py:41-58,135-1
 scope and raises.
 """
 import ctypes as C
+import math
 
 import numpy as np
 import torch
@@ -170,6 +171,32 @@ class BatchedScene:
         if first_hit or last_free:
             return fc, dict(first_hit=fh, last_free=lf)
         return fc
+
+    def cspace_occupancy(self, b1, b2=None, lo=(0.0, 0.0), step=None, packed=False, free_count=False, engine=None):
+        """collision_check() (scene_0.py:60-76) at every pose of a b1 x b2 lattice of joint angles, for every grid of the
+        scene: the exact obstacle image of the configuration-space torus.  Nothing is moved.
+        Pose (i, j) = (lo[0] + i * step[0], lo[1] + j * step[1]) in float64; its entry is True exactly when
+        collision_check with the same engine says that pose collides on that grid.  Defaults: b2 = b1, step = 2 pi / b
+        per axis, so the lattice covers the whole torus from 0.
+        Returns bool [n_grids, b1, b2], or with packed=True the int32 words [n_grids, b1, ceil(b2/32)] (pose (i, j) is bit
+        j % 32 of word j // 32, padding bits 0); with free_count=True also int64 [n_grids], the collision-free poses."""
+        b1 = int(b1)
+        b2 = b1 if b2 is None else int(b2)
+        if b1 < 1 or b2 < 1:
+            raise ValueError("the lattice needs b1, b2 >= 1, got %d x %d" % (b1, b2))
+        lo1, lo2 = (float(v) for v in lo)
+        st1, st2 = (2.0 * math.pi / b1, 2.0 * math.pi / b2) if step is None else (float(v) for v in step)
+        n_grids = int(self.grid.n_grids)
+        words = torch.empty(n_grids, b1, (b2 + 31) // 32, dtype=torch.int32, device=self.device)
+        fc = torch.empty(n_grids, dtype=torch.int64, device=self.device) if free_count else None
+        g = self.grid.c_struct()
+        _lib.check(self._lib.ag_cspace_occupancy(self.params(), g, lo1, st1, b1, lo2, st2, b2, ptr(words), ptr(fc),
+                                                 self.engine if engine is None else _engine(engine), stream_ptr(self.device)),
+                   "ag_cspace_occupancy")
+        if not packed:
+            shifts = torch.arange(32, dtype=torch.int32, device=self.device)
+            words = ((words.unsqueeze(-1) >> shifts) & 1).reshape(n_grids, b1, -1)[:, :, :b2] != 0
+        return (words, fc) if free_count else words
 
     def check_target_reached(self):
         """scene_0.py:115-133 -> bool [N]"""

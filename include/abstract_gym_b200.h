@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define AG_ABI_VERSION 6
+#define AG_ABI_VERSION 7
 
 #if defined(__GNUC__)
 #define AG_API __attribute__((visibility("default")))
@@ -198,6 +198,23 @@ AG_API ag_status ag_collision_check(const ag_params *p, const ag_grid *g, const 
 AG_API ag_status ag_check_motion(const ag_params *p, const ag_grid *g, const double *j1, const double *j2, const double *goal,
                                  const int32_t *steps, int32_t *first_collision, int32_t *first_hit, double *last_free,
                                  int64_t m, int64_t env_id0, int32_t engine, void *stream);
+
+/* Configuration-space occupancy: scenario/scene_0.py:60-76 Scene.collision_check() at every pose of a b1 x b2 lattice of
+ * joint angles, for every grid g = 0 .. n_grids-1 -- the obstacle image of the configuration-space torus, exact (unlike
+ * ag_cspace_map's conservative bins).  Pose (i, j) = (lo1 + (double)i * step1, lo2 + (double)j * step2): float64, one
+ * rounding per operation, never contracted to an FMA.  Its bit is 1 exactly when ag_collision_check with the same engine
+ * says that pose collides on grid g (a grid's staging and broad phase are those of K2 launched on that grid's own envs
+ * from an env_id0 that is a multiple of 256).
+ * bits: [n_grids][b1][W] uint32 (device), W = ceil(b2 / 32); pose (i, j) is bit j % 32 of word j / 32 of row i; the
+ *       padding bits of a row's last word are 0.  With b2 a multiple of 32 this is ag_cspace_map's bit order.
+ * free_count: optional [n_grids] int64 (device, 8-byte aligned): the collision-free poses of each grid, written (not
+ *       accumulated).
+ * Errors, before anything touches the device: b1 < 1 or b2 < 1, a non-finite lo or step, or n_grids * b1 * W beyond
+ * int64 -> AG_ERR_SHAPE; the grid checks of ag_collision_check; bits NULL -> AG_ERR_NULL; an unknown engine ->
+ * AG_ERR_MODE.  Stream-ordered (the free counts are zeroed by a memset on `stream`) and capturable in a CUDA graph. */
+AG_API ag_status ag_cspace_occupancy(const ag_params *p, const ag_grid *g, double lo1, double step1, int32_t b1, double lo2,
+                                     double step2, int32_t b2, uint32_t *bits, int64_t *free_count, int32_t engine,
+                                     void *stream);
 
 /* K1: scenario/scene_0.py:88-103  Scene.step(action).  j1,j2,reward,flags are in/out (sticky
  * semantics).  actions: [n][2] float64 (actions_f32 == 0) or float32.  Optional outputs:
