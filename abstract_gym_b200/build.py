@@ -16,8 +16,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 INCLUDE = os.path.join(HERE, "..", "include")
 LIB = os.environ.get("AG_LIB_PATH") or os.path.join(HERE, "libabstract_gym_b200.so")   # AG_LIB_PATH: A/B builds
-SOURCES = ["ag_kernels.cu", "ag_rollout_lut.cu", "ag_dense.cu", "ag_motion.cu", "ag_cspace.cu", "ag_host.cu"]
-HEADERS = ["ag_device.cuh", "ag_fast.cuh", "ag_rollout.cuh", os.path.join(INCLUDE, "abstract_gym_b200.h")]
+SOURCES = ["ag_kernels.cu", "ag_rollout_lut.cu", "ag_cmap.cu", "ag_dense.cu", "ag_motion.cu", "ag_cspace.cu", "ag_host.cu"]
+HEADERS = ["ag_device.cuh", "ag_fast.cuh", "ag_rollout.cuh", "ag_cmap.cuh", os.path.join(INCLUDE, "abstract_gym_b200.h")]
 OBJDIR = os.path.join(HERE, "build")
 DEBUG_LIB = os.path.join(HERE, "libabstract_gym_b200_debug.so")
 # the compiled torch custom-op library (torch.ops.abstract_gym_b200.*): a C++ shim over the C ABI, linked against

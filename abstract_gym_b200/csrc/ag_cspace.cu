@@ -8,9 +8,9 @@
 // on one grid, which it stages once; free counts are a popcount per word, a block sum and one atomic per block.
 //
 // Three forms, with K2's results:
-//   map form (FAST engine, grids where cspace_map_applies: scene_0 class) -- one phase DFMA per joint and one bit of
-//     the rollout's configuration-space map in shared memory.  A CLEAR bin is collision-free; poses in SET bins, and
-//     poses with |q| >= 2^20 or NaN (outside the phase's range), go to pose_collides<FAST>.
+//   map form (FAST engine, where ag_cmap.cu hands the launch a configuration-space map: scene_0-class grids) -- the
+//     test of cmap_needs_check (ag_cmap.cuh) with joint_1's phase hoisted out of the row; only the poses it flags go to
+//     pose_collides<FAST>.
 //   row form (EXACT, BRUTE) -- link 1 depends on joint_1 only, so it is tested once per unit; a unit whose link 1 hits
 //     is all ones, every other pose tests link 2 only.  Both engines' flag is exactly link 1 || link 2 (arm_collides,
 //     arm_brute), with the elbow of forward_kinematics, so the bits are K2's.
@@ -18,6 +18,7 @@
 //     (the float32 filter and the float64 re-evaluation look at the arm as a whole), so it is not factored.
 #include <climits>
 
+#include "ag_cmap.cuh"
 #include "ag_rollout.cuh"
 
 using namespace agd;
@@ -51,14 +52,6 @@ __device__ __forceinline__ bool link_hits(const GridDev &G, const GridView &V, d
     else return link_exact<false>(G, V, p0x, p0y, p1x, p1y, eps, fh, axis);
 }
 
-// collision_check of one pose, out of line: the map form's loop stays short with few live registers
-template <int ENGINE>
-__device__ __noinline__ bool pose_hit(const ag_params &P, const GridDev &G, const BlockCtx &B, const FastConst &C, double q1,
-                                      double q2) {
-    int fh = 0, axis = 0;
-    return pose_collides<ENGINE, false>(P, G, B, C, q1, q2, fh, axis);
-}
-
 // G.envs_per_grid == 1 (set by the launcher): env id g selects grid g, and no grid index overflows an env id.
 // Two blocks per SM fit the row form without spills; the FAST forms need more than 128 registers (see DESIGN.md).
 template <int ENGINE, bool MAP>
@@ -76,17 +69,11 @@ k_cspace(const __grid_constant__ ag_params P, const __grid_constant__ GridDev G,
         build_fast_list(G, B.V, &s_fl);
         B.fl = &s_fl;
     }
-    const uint32_t *cmap = nullptr;
-    if constexpr (MAP) {                                                         // the map: global -> shared, once per block
-        const uint4 *src = reinterpret_cast<const uint4 *>(D.cmap);
-        uint4 *dst = reinterpret_cast<uint4 *>(smem + D.cmap_off);
-        for (int w = threadIdx.x; w < CMAP_WORDS / 4; w += blockDim.x) dst[w] = src[w];
-        cmap = reinterpret_cast<const uint32_t *>(smem + D.cmap_off);
-    }
+    if constexpr (MAP) cmap_to_shared(smem + D.cmap_off, D.cmap, blockDim.x);   // the map: global -> shared, once per block
     if (threadIdx.x == 0) s_free = 0ull;
     __syncthreads();
     const int lane = threadIdx.x & 31;
-    const double phase_scale = 4294967296.0 / TWO_PI;
+    const uint32_t cmap_a = MAP ? smem_u32(smem + D.cmap_off) : 0u;
     unsigned long long free = 0;
     for (int64_t u = part * WARPS + (threadIdx.x >> 5); u < D.units; u += D.blocks_per_grid * WARPS) {
         const int64_t i = u / D.spans;
@@ -98,20 +85,14 @@ k_cspace(const __grid_constant__ ag_params P, const __grid_constant__ GridDev G,
             const Arm A = forward_kinematics(q1, 0.0, P.link_1, P.link_2);
             row_hit = link_hits<ENGINE>(G, B.V, 0.0, 0.0, A.ex, A.ey, P.section_eps);
         }
-        uint32_t x1 = 0u;
-        bool in1 = true;
-        if constexpr (MAP) {
-            x1 = (uint32_t)__double2loint(fma(q1, phase_scale, PHASE_MAGIC)) >> (32 - CB1);
-            in1 = fabs(q1) < 1048576.0;                                          // NaN-safe: NaN is out of range
-        }
+        const uint32_t x1 = MAP ? cmap_phase(q1) : 0u;
+        const bool in1 = cmap_in_range(q1);
         for (int w = w0; w < w1; ++w) {
             const int j = (w << 5) + lane;
             const double q2 = __dadd_rn(D.lo2, __dmul_rn((double)j, D.step2));
             bool hit;
             if constexpr (MAP) {
-                const uint32_t x2 = (uint32_t)__double2loint(fma(q2, phase_scale, PHASE_MAGIC));
-                const uint32_t bit = (x1 << CB2) | (x2 >> (32 - CB2));
-                const bool slow = ((cmap[bit >> 5] >> (bit & 31u)) & 1u) != 0 || !in1 || !(fabs(q2) < 1048576.0);
+                const bool slow = cmap_bit(cmap_a, x1, cmap_phase(q2)) || !in1 || !cmap_in_range(q2);
                 hit = slow && pose_hit<ENGINE>(P, G, B, C, q1, q2);
             } else if constexpr (ENGINE == AG_ENGINE_FAST) {
                 hit = pose_hit<ENGINE>(P, G, B, C, q1, q2);
@@ -149,15 +130,13 @@ ag_status launch(const ag_params &P, const GridDev &G, const CspaceDev &D0, size
         const cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return (ag_status)e;
     }
-    int dev = 0, sms = 0, occ = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k, AG_BLOCK, smem);
-    if (e != cudaSuccess) return (ag_status)e;
+    int slots = 0;
+    const ag_status st = resident_blocks(k, AG_BLOCK, smem, &slots);
+    if (st != AG_OK) return st;
     // Blocks per grid: one unit per warp at most; otherwise about one wave of blocks in all (map form: every block
     // copies the 32 KB map once) or four (the other forms: grids differ in cost, so finer blocks balance better).
-    // The total stays below 2^31: it is at most max(n_grids, 4 * sms * occ + n_grids).
-    const int64_t waves = MAP ? 1 : 4, want = waves * sms * (occ > 0 ? occ : 1);
+    // The total stays below 2^31: it is at most max(n_grids, 4 * slots + n_grids).
+    const int64_t waves = MAP ? 1 : 4, want = waves * (slots > 0 ? slots : 1);
     CspaceDev D = D0;
     const int64_t per_grid = (want + G.n_grids - 1) / G.n_grids, most = (D.units + WARPS - 1) / WARPS;
     D.blocks_per_grid = per_grid < most ? per_grid : most;
@@ -185,16 +164,13 @@ ag_status launch_cspace_occupancy(const ag_params &P, const GridDev &G0, int32_t
         if (e != cudaSuccess) return (ag_status)e;
     }
     switch (engine) {
-        case AG_ENGINE_FAST:
-            if (cspace_map_applies(G0, max_occupied)) {
-                const ag_status st = cspace_map_for_launch(P, G0, s, &D.cmap);
-                if (st != AG_OK) return st;
-                if (D.cmap != nullptr) {
-                    D.cmap_off = (uint32_t)((smem + 15) & ~(size_t)15);
-                    return launch<AG_ENGINE_FAST, true>(P, G, D, (size_t)D.cmap_off + (size_t)CMAP_WORDS * 4, s);
-                }
-            }
-            return launch<AG_ENGINE_FAST, false>(P, G, D, smem, s);
+        case AG_ENGINE_FAST: {
+            CmapLaunch cm;
+            const ag_status st = cspace_map_for_launch(P, G0, max_occupied, smem, s, &cm);
+            if (st != AG_OK) return st;
+            D.cmap = cm.map; D.cmap_off = cm.off;
+            return cm.map ? launch<AG_ENGINE_FAST, true>(P, G, D, cm.smem, s) : launch<AG_ENGINE_FAST, false>(P, G, D, smem, s);
+        }
         case AG_ENGINE_EXACT: return launch<AG_ENGINE_EXACT, false>(P, G, D, smem, s);
         case AG_ENGINE_BRUTE: return launch<AG_ENGINE_BRUTE, false>(P, G, D, smem, s);
         default: return AG_ERR_MODE;

@@ -1,5 +1,5 @@
 // ag_rollout.cuh -- pieces shared by the rollout kernels (ag_kernels.cu: K1..K5 and the general K4;
-// ag_rollout_lut.cu: the persistent scene_0-class K4).
+// ag_rollout_lut.cu: the persistent scene_0-class K4), motion checking (ag_motion.cu) and occupancy (ag_cspace.cu).
 #pragma once
 #include <climits>
 
@@ -10,6 +10,18 @@ namespace agd {
 
 constexpr int AG_BLOCK = 256;
 static_assert(AG_BLOCK <= AG_TILEQ_COLS, "the tile queue of arm_fast_hier has one column per thread");
+
+// the grid of a persistent launch: blocks of `kernel` resident at once (SM count x blocks per SM at `block` threads and
+// `smem` bytes of dynamic shared memory)
+template <typename Kernel>
+ag_status resident_blocks(Kernel kernel, int block, size_t smem, int *blocks) {
+    int dev = 0, sms = 0, occ = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, block, smem);
+    *blocks = sms * occ;
+    return (ag_status)e;
+}
 
 struct RolloutDev {
     int64_t n, env_id0, row_stride;
@@ -109,6 +121,15 @@ __device__ __forceinline__ bool pose_collides(const ag_params &P, const GridDev 
     }
 }
 
+// collision_check of one pose, out of line: the map forms of k_check_motion and k_cspace keep their loops short,
+// with few live registers
+template <int ENGINE, int BP = BP_ANY>
+static __device__ __noinline__ bool pose_hit(const ag_params &P, const GridDev &G, const BlockCtx &B, const FastConst &C, double q1,
+                                      double q2) {
+    int fh = 0, axis = 0;
+    return pose_collides<ENGINE, false, BP>(P, G, B, C, q1, q2, fh, axis);
+}
+
 // shared by K3 and K4: scenario/scene_0.py:174-181 with a bound.  `colliding` is the
 // collision_check() of the current pose.
 template <int ENGINE, bool HAS_RESET_U, int BP = BP_ANY>
@@ -204,42 +225,11 @@ __device__ __forceinline__ void zero_fill_warp(const RolloutDev &A, int64_t warp
     __syncwarp();                                       // orders these stores before the owners' later rewrites
 }
 
-
-// ------------------------------------------------------------------------- configuration-space map (ag_rollout_lut.cu)
-// 2^CB1 x 2^CB2 bins over (joint_1, joint_2) mod 2pi, one bit each.  The bin of a pose with |q| < 2^20 comes from the
-// joint phases x = low word of fma(q, 2^32/2pi, PHASE_MAGIC): bit ((x1 >> (32 - CB1)) << CB2) | (x2 >> (32 - CB2)) of
-// the map, word bit >> 5.  CLEAR: no pose of the bin collides or reaches the target (k_cspace_build); SET: evaluate.
-#ifndef AG_CMAP_B1
-#define AG_CMAP_B1 10
-#endif
-#ifndef AG_CMAP_B2
-#define AG_CMAP_B2 8
-#endif
-constexpr int CB1 = AG_CMAP_B1, CB2 = AG_CMAP_B2;
-static_assert(CB1 >= 6 && CB2 >= 6 && CB1 + CB2 <= 20, "the map must fit shared memory");
-constexpr int CMAP_WORDS = 1 << (CB1 + CB2 - 5);
-constexpr double PHASE_MAGIC = 6755399441055744.0;       // 1.5 * 2^52: the add rounds to an integer in the low word
-constexpr double TWO_PI = 6.283185307179586476925;
-
-}  // namespace agd
-
-// ag_rollout_lut.cu: the map for one launch.  cspace_map_applies: the grid is one staged grid with an obstacle list
-// (S <= 32, at most AG_LIST_MAX occupied cells by ag_grid.max_occupied), the only grids the map is built for.
-// cspace_map_for_launch: the library's cached map of this grid and these parameters, after enqueuing on `s` the
-// k_cspace_build launch that checks it against the grid's current content on the device (and rebuilds it if it
-// differs); *map = nullptr when no cache entry can be had (inside a stream capture before the grid's first uncaptured
-// launch, or an allocation failure) -- the caller then takes its general form, whose results are identical.
-bool cspace_map_applies(const agd::GridDev &G, int32_t max_occupied);
-ag_status cspace_map_for_launch(const ag_params &P, const agd::GridDev &G, cudaStream_t s, const uint32_t **map);
-
-namespace agd {
-
 __device__ __forceinline__ void cp_async8(uint32_t smem_dst, const void *gsrc) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_dst), "l"(gsrc) : "memory");
 }
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-
 
 }  // namespace agd

@@ -9,8 +9,8 @@
 //
 // CMAP form (the default; scene-wide target): one bit of a configuration-space map in shared memory, indexed by the top
 //   bits of (x1, x2), says whether ANY pose of that bin can touch an obstacle or the target box -- no forward kinematics
-//   in the hot loop at all (k_cspace_build below explains how the map is made conservative, and how it is cached and
-//   validated against the current grid on the device at every launch).
+//   in the hot loop at all (ag_cmap.cuh: the map's layout and test; ag_cmap.cu: how the map is made conservative, and
+//   how it is cached and validated against the current grid on the device at every launch).
 // table-arm form (per-env targets, or no map available): the float32 arm comes from two shared-memory tables,
 //   entry  = lut[x >> (32-B)]                            (c, s) * length at the bin centre, 8 bytes
 //   d      = (x mod 2^(32-B)) * 2pi/2^32 - pi/2^B        angle from the bin centre, one LOP3 + one FFMA
@@ -31,9 +31,8 @@
 //   action (cp.async ring, RING - 1 rows ahead) -> 2 DADD -> test -> record (2 F2F + 2 STG) -> vote.
 #include <atomic>
 #include <cstdlib>
-#include <cstring>
-#include <mutex>
 
+#include "ag_cmap.cuh"
 #include "ag_rollout.cuh"
 
 using namespace agd;
@@ -51,15 +50,6 @@ namespace {
 #ifndef AG_LUT_BLOCKS_PER_SM
 #define AG_LUT_BLOCKS_PER_SM 1
 #endif
-
-// configuration-space map (CMAP form of the kernel): CB1, CB2, CMAP_WORDS in ag_rollout.cuh
-constexpr int CMAP_HDR_WORDS = 64;                       // 256-byte header in front of the map words
-constexpr int CMAP_SLOTS = 16;
-struct CmapHeader {
-    unsigned long long key;                              // hash of everything the map depends on; 0 = never built
-    unsigned int done[CMAP_SLOTS];                       // blocks finished, one counter per in-flight build
-};
-static_assert(sizeof(CmapHeader) <= CMAP_HDR_WORDS * 4, "header");
 
 constexpr int B1 = AG_LUT_B1, B2 = AG_LUT_B2;            // bins: 2^B1 for link 1 (also the resolution of its hazard bit), 2^B2 for link 2
 constexpr int N1 = 1 << B1, N2 = 1 << B2;
@@ -100,7 +90,7 @@ struct LutConst {
     uint32_t ss_off;        // byte offset of SlowShared in dynamic shared memory (after the staged grid)
     uint32_t slot;          // this launch's pair of tile / done counters (g_tile_sched)
     uint32_t cmap_off;      // CMAP: byte offset of the map's shared-memory copy in the dynamic segment
-    const uint32_t *cmap;   // CMAP: the map words in global memory (k_cspace_build)
+    const uint32_t *cmap;   // CMAP: the map words in global memory (cspace_map_for_launch)
 };
 
 // Dynamic tile scheduling: warps draw 32-env tiles from a device-global counter, so no warp idles while tiles remain
@@ -148,13 +138,7 @@ struct PoseDraw {
 };
 enum { PD_VALID = 1, PD_DREW = 2, PD_STUCK = 4 };
 
-__device__ __forceinline__ uint32_t lds_u32(uint32_t addr) {
-    uint32_t v;
-    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(addr));
-    return v;
-}
-
-// cmap_a: shared-window address of the configuration-space map, or 0.  A candidate whose bin is CLEAR is certainly
+// cmap_a: shared-window address of the configuration-space map, or 0.  A candidate cmap_needs_check clears is certainly
 // collision-free (the map's guarantee): accepted without any arithmetic on the arm.
 AG_COLD PoseDraw draw_valid_pose(const ag_params &P, const GridDev &G, const FastConst &C,
                                                  const unsigned char *smem_grid, const FastList *fl, uint32_t rc,
@@ -177,12 +161,7 @@ AG_COLD PoseDraw draw_valid_pose(const ag_params &P, const GridDev &G, const Fas
         ++rc; ++tries;
         o.j1 = __dmul_rn(__dmul_rn(u0, 3.141592653589793), 2.0);    // scene_0.py:180  rand()*pi*2.0
         o.j2 = __dmul_rn(__dmul_rn(u1, 3.141592653589793), 2.0);    // :181
-        if (cmap_a != 0u && o.j1 < 1048576.0 && o.j2 < 1048576.0) {        // candidates are in [0, 2 pi) unless scripted
-            const uint32_t x1 = (uint32_t)__double2loint(fma(o.j1, 4294967296.0 / TWO_PI, PHASE_MAGIC));
-            const uint32_t x2 = (uint32_t)__double2loint(fma(o.j2, 4294967296.0 / TWO_PI, PHASE_MAGIC));
-            const uint32_t bit = ((x1 >> (32 - CB1)) << CB2) | (x2 >> (32 - CB2));
-            if (((lds_u32(cmap_a + ((bit >> 3) & ~3u)) >> (bit & 31u)) & 1u) == 0u) { colliding = false; continue; }
-        }
+        if (cmap_a != 0u && !cmap_needs_check(cmap_a, o.j1, o.j2)) { colliding = false; continue; }
         const int d = fast_decide<BP_LIST>(P, G, V, fl, C, o.j1, o.j2, false);
         axis += d >> 2;
         colliding = (d & 1) != 0;
@@ -274,45 +253,9 @@ __device__ __forceinline__ float2 taylor_turn(float2 t, float d) {
     return make_float2(fmaf(-d, t.y, ut.x), fmaf(d, t.x, ut.y));
 }
 
-// The directions in which link 1 (origin -> length l1) comes within `mg` of the closed square sq = (min_x, min_y, max_x,
-// max_y): the angular extent of (inflated square) n (disc of radius l1) seen from the origin.  That set is convex and,
-// unless the origin lies inside the inflated square, does not contain the origin, so its extent is spanned by its
-// vertices: corners inside the disc and circle / edge crossings (a ray from the centre is never tangent to the circle).
-// half < 0: never; half >= pi: always.
-__device__ void hazard_interval(double X0, double Y0, double X1, double Y1, double l1, float &mid, float &half);
+// hazard_interval (ag_cmap.cuh) of the square sq = (min_x, min_y, max_x, max_y) inflated by mg
 __device__ void hazard_interval(float4 sq, double l1, double mg, float &mid, float &half) {
-    hazard_interval((double)sq.x - mg, (double)sq.y - mg, (double)sq.z + mg, (double)sq.w + mg, l1, mid, half);
-}
-// the same for an (already inflated) box X0..X1 x Y0..Y1
-__device__ void hazard_interval(double X0, double Y0, double X1, double Y1, double l1, float &mid, float &half) {
-    if (X0 <= 0.0 && X1 >= 0.0 && Y0 <= 0.0 && Y1 >= 0.0) { mid = 0.0f; half = 4.0f; return; }
-    const double r2 = l1 * l1;
-    const double ref = atan2(0.5 * (Y0 + Y1), 0.5 * (X0 + X1));
-    double lo = 1.0e9, hi = -1.0e9;
-    auto take = [&](double px, double py) {
-        double a = atan2(py, px) - ref;
-        a -= TWO_PI * rint(a / TWO_PI);
-        lo = fmin(lo, a); hi = fmax(hi, a);
-    };
-    const double XS[2] = {X0, X1}, YS[2] = {Y0, Y1};
-    for (int i = 0; i < 2; ++i)
-        for (int j = 0; j < 2; ++j)
-            if (XS[i] * XS[i] + YS[j] * YS[j] <= r2) take(XS[i], YS[j]);
-    for (int i = 0; i < 2; ++i) {
-        if (fabs(XS[i]) <= l1) {
-            const double y = sqrt(r2 - XS[i] * XS[i]);
-            if (y >= Y0 && y <= Y1) take(XS[i], y);
-            if (-y >= Y0 && -y <= Y1) take(XS[i], -y);
-        }
-        if (fabs(YS[i]) <= l1) {
-            const double xx = sqrt(r2 - YS[i] * YS[i]);
-            if (xx >= X0 && xx <= X1) take(xx, YS[i]);
-            if (-xx >= X0 && -xx <= X1) take(-xx, YS[i]);
-        }
-    }
-    if (hi < lo) { mid = 0.0f; half = -1.0f; return; }
-    mid = (float)(ref + 0.5 * (lo + hi));
-    half = (float)(0.5 * (hi - lo));
+    agd::hazard_interval((double)sq.x - mg, (double)sq.y - mg, (double)sq.z + mg, (double)sq.w + mg, l1, mid, half);
 }
 
 // Fill a table of n bins with (c, s) * len at the bin centres (b + 1/2) * 2pi/n, eight symmetric entries per
@@ -346,176 +289,10 @@ __device__ void fill_table(float2 *lut, int n, double len, const float *hz, int 
     }
 }
 
-// ------------------------------------------------------------------------- configuration-space map (CMAP)
-// One bit per bin of (joint_1, joint_2) mod 2pi: CLEAR = for every pose of the bin both links stay farther than CMAP_MG
-// from every occupied square and the end effector stays outside the target box (scene_0.py:129-130) by more than
-// CMAP_MG, i.e. the step is certainly uneventful and the hot loop needs no forward kinematics at all -- two DFMA for
-// the phases, one shared-memory word, one bit test.  SET = "look closer": the lane takes the slow path, which decides
-// exactly as before.  So the map only has to be CONSERVATIVE; it is built from lower bounds of distances:
-//   * over a bin, joint_1 in [a1-d1, a1+d1] and joint_2 in [a2-d2, a2+d2], the elbow stays within the sagitta
-//     l1(1-cos d1) of the chord Ea..Eb and link 2's direction vector within l2(1-cos d2) of the triangle 0, Ua, Ub, so
-//     link 2 sweeps a subset of the convex polygon hull({Ea,Eb} + {0,Ua,Ub}) inflated by the two sagittas;
-//   * the distance from that polygon to a square is bounded from below by the largest separation along a finite set
-//     of unit axes (every axis gives a valid lower bound; the set -- box normals, the link normals at the bin's centre
-//     and edges, the chord normal, and the directions from the square's corners to the centre pose's elbow and end
-//     effector -- makes the bound tight for edge/vertex and vertex/vertex contacts);
-//   * link 1 depends on joint_1 only and uses the exact angular intervals of hazard_interval().
-// 2.0e-6 m covers the rounding of the phase (< 1e-9 rad), of this float64 construction, and the reference's own
-// rounding noise (< 1e-12 m): the same margin the float32 broad phase uses.
-// The map depends on the grid, the link lengths, the target and its tolerance.  It lives in a library-owned device
-// buffer that is reused between launches: every launch re-derives a 64-bit key from the CURRENT grid words and
-// parameters on the device (thread 0 of each block, ~100 words) and rebuilds the map only when the stored key differs.
-constexpr double CMAP_MG = 2.0e-6;
-constexpr int CMAP_BUILD_BLOCKS = 128;
-constexpr uint32_t CMAP_VERSION = 1;
-
-struct V2 { double x, y; };
-
-__device__ __forceinline__ unsigned long long mix64(unsigned long long h, unsigned long long v) {
-    h ^= v;
-    h *= 0x100000001B3ull;                                                       // FNV-1a over 64-bit words
-    return h ^ (h >> 29);
-}
-
-// separation of the point set P and the box (centre c, half extents hx, hy) along the unit axis n (negative: overlap)
-template <int NP>
-__device__ __forceinline__ double axis_gap(V2 n, const V2 (&P)[NP], V2 c, double hx, double hy) {
-    double lo = 1.0e300, hi = -1.0e300;
-#pragma unroll
-    for (int i = 0; i < NP; ++i) {
-        const double d = n.x * P[i].x + n.y * P[i].y;
-        lo = fmin(lo, d); hi = fmax(hi, d);
-    }
-    const double cc = n.x * c.x + n.y * c.y, r = fabs(n.x) * hx + fabs(n.y) * hy;
-    return fmax(lo - (cc + r), (cc - r) - hi);
-}
-
-__global__ void __launch_bounds__(256)
-k_cspace_build(const __grid_constant__ ag_params P, const __grid_constant__ GridDev G, uint32_t *buf, uint32_t slot) {
-    __shared__ unsigned long long s_key;
-    __shared__ int s_skip, s_m;
-    __shared__ double s_sq[AG_LIST_MAX][4];
-    __shared__ float s_hz[2 * AG_LIST_MAX];
-    CmapHeader *H = reinterpret_cast<CmapHeader *>(buf);
-    if (threadIdx.x == 0) {
-        unsigned long long h = 0xCBF29CE484222325ull;
-        h = mix64(h, ((unsigned long long)CMAP_VERSION << 48) | ((unsigned long long)CB1 << 40) | ((unsigned long long)CB2 << 32) | (unsigned)G.S);
-        const double par[6] = {P.link_1, P.link_2, P.target_x, P.target_y, P.reach_eps, G.side};
-        for (int i = 0; i < 6; ++i) h = mix64(h, (unsigned long long)__double_as_longlong(par[i]));
-        int m = 0;
-        for (int r = 0; r < G.S; ++r) {
-            h = mix64(h, (unsigned long long)__double_as_longlong(G.min_y[r]));
-            h = mix64(h, (unsigned long long)__double_as_longlong(G.min_x[r]));
-            for (int w = 0; w < G.wpr; ++w) {
-                uint32_t word = G.bits[r * G.wpr + w];
-                h = mix64(h, word);
-                while (word) {
-                    const int c = (w << 5) + __ffs(word) - 1;
-                    word &= word - 1;
-                    if (m < AG_LIST_MAX && c < G.S) {
-                        const double mnx = G.min_x[c], mny = G.min_y[r];
-                        s_sq[m][0] = mnx; s_sq[m][1] = mny;
-                        s_sq[m][2] = __dadd_rn(mnx, G.side); s_sq[m][3] = __dadd_rn(mny, G.side);   // occupancy_grid.py:66-67
-                    }
-                    ++m;
-                }
-            }
-        }
-        h |= 1ull;                                                               // 0 means "never built"
-        s_key = h;
-        s_m = m > AG_LIST_MAX ? -1 : m;                                          // no obstacle list: every bin is slow
-        s_skip = (*reinterpret_cast<volatile unsigned long long *>(&H->key) == h) ? 1 : 0;
-    }
-    __syncthreads();
-    if (!s_skip) {
-        const int m = s_m;
-        if ((int)threadIdx.x < m)
-            hazard_interval(s_sq[threadIdx.x][0] - CMAP_MG, s_sq[threadIdx.x][1] - CMAP_MG, s_sq[threadIdx.x][2] + CMAP_MG,
-                            s_sq[threadIdx.x][3] + CMAP_MG, P.link_1, s_hz[2 * threadIdx.x], s_hz[2 * threadIdx.x + 1]);
-        __syncthreads();
-        constexpr int N1c = 1 << CB1, N2c = 1 << CB2;
-        const double l1 = P.link_1, l2 = P.link_2;
-        double sd, cd;
-        sincospi(1.0 / (double)N1c, &sd, &cd);
-        const double sag1 = l1 * (1.0 - cd);
-        sincospi(1.0 / (double)N2c, &sd, &cd);
-        const double sag2 = l2 * (1.0 - cd);
-        const double infl = sag1 + sag2 + CMAP_MG;
-        const float hw1 = (float)(TWO_PI / (double)(2 * N1c)) + 2.0e-6f;          // half a bin of joint_1 + rounding
-        for (int bin = blockIdx.x * 256 + threadIdx.x; bin < N1c * N2c; bin += gridDim.x * 256) {   // a warp = 32 bins of joint_2
-            const int b1 = bin >> CB2, b2 = bin & (N2c - 1);
-            bool haz = m < 0;
-            // ---- link 1: exact angular intervals
-            const float th1 = ((float)b1 + 0.5f) * (float)(TWO_PI / (double)N1c);
-            for (int k = 0; k < m; ++k) {
-                float dlt = th1 - s_hz[2 * k];
-                dlt -= (float)TWO_PI * rintf(dlt * (float)(1.0 / TWO_PI));
-                if (fabsf(dlt) <= s_hz[2 * k + 1] + hw1) haz = true;
-            }
-            // ---- link 2: the swept polygon against every square
-            V2 Ea, Eb, Ec, Ua, Ub, Uc;
-            sincospi(2.0 * (double)b1 / (double)N1c, &Ea.y, &Ea.x);
-            sincospi(2.0 * (double)(b1 + 1) / (double)N1c, &Eb.y, &Eb.x);
-            sincospi((2.0 * (double)b1 + 1.0) / (double)N1c, &Ec.y, &Ec.x);
-            sincospi(2.0 * (double)b2 / (double)N2c, &Ua.y, &Ua.x);
-            sincospi(2.0 * (double)(b2 + 1) / (double)N2c, &Ub.y, &Ub.x);
-            sincospi((2.0 * (double)b2 + 1.0) / (double)N2c, &Uc.y, &Uc.x);
-            const V2 n1c = {Ec.x, Ec.y};                                          // normal of the elbow chord = link 1's direction
-            const V2 n2a = {-Ua.y, Ua.x}, n2b = {-Ub.y, Ub.x}, n2c = {-Uc.y, Uc.x};   // link 2's normals at the bin's edges / centre
-            const V2 ea = {l1 * Ea.x, l1 * Ea.y}, eb = {l1 * Eb.x, l1 * Eb.y}, ec = {l1 * Ec.x, l1 * Ec.y};
-            const V2 ua = {l2 * Ua.x, l2 * Ua.y}, ub = {l2 * Ub.x, l2 * Ub.y};
-            const V2 gc = {ec.x + l2 * Uc.x, ec.y + l2 * Uc.y};
-            const V2 poly[6] = {ea, eb, {ea.x + ua.x, ea.y + ua.y}, {ea.x + ub.x, ea.y + ub.y},
-                                {eb.x + ua.x, eb.y + ua.y}, {eb.x + ub.x, eb.y + ub.y}};
-            for (int k = 0; k < m && !haz; ++k) {
-                const V2 c = {0.5 * (s_sq[k][0] + s_sq[k][2]), 0.5 * (s_sq[k][1] + s_sq[k][3])};
-                const double hx = 0.5 * (s_sq[k][2] - s_sq[k][0]), hy = 0.5 * (s_sq[k][3] - s_sq[k][1]);
-                double gap = axis_gap(V2{1.0, 0.0}, poly, c, hx, hy);
-                gap = fmax(gap, axis_gap(V2{0.0, 1.0}, poly, c, hx, hy));
-                gap = fmax(gap, axis_gap(n2c, poly, c, hx, hy));
-                gap = fmax(gap, axis_gap(n2a, poly, c, hx, hy));
-                gap = fmax(gap, axis_gap(n2b, poly, c, hx, hy));
-                gap = fmax(gap, axis_gap(n1c, poly, c, hx, hy));
-#pragma unroll 1
-                for (int j = 0; j < 8; ++j) {                                     // corner -> centre pose's end effector / elbow
-                    const double qx = (j & 1) ? s_sq[k][2] : s_sq[k][0], qy = (j & 2) ? s_sq[k][3] : s_sq[k][1];
-                    const V2 from = (j & 4) ? ec : gc;
-                    const double vx = from.x - qx, vy = from.y - qy, nv = sqrt(vx * vx + vy * vy);
-                    if (nv > 1.0e-9) gap = fmax(gap, axis_gap(V2{vx / nv, vy / nv}, poly, c, hx, hy) * (1.0 - 1.0e-12));
-                }
-                if (!(gap > infl)) haz = true;
-            }
-            // ---- the target box (scene_0.py:129-130) against the box of the swept end effector
-            {
-                const double gx0 = fmin(fmin(poly[2].x, poly[3].x), fmin(poly[4].x, poly[5].x)) - infl;
-                const double gx1 = fmax(fmax(poly[2].x, poly[3].x), fmax(poly[4].x, poly[5].x)) + infl;
-                const double gy0 = fmin(fmin(poly[2].y, poly[3].y), fmin(poly[4].y, poly[5].y)) - infl;
-                const double gy1 = fmax(fmax(poly[2].y, poly[3].y), fmax(poly[4].y, poly[5].y)) + infl;
-                const double e = fabs(P.reach_eps);
-                if (!(gx0 > P.target_x + e || gx1 < P.target_x - e || gy0 > P.target_y + e || gy1 < P.target_y - e)) haz = true;
-            }
-            const uint32_t word = __ballot_sync(0xFFFFFFFFu, haz);
-            if ((threadIdx.x & 31) == 0) buf[CMAP_HDR_WORDS + (bin >> 5)] = word;
-        }
-    }
-    // the last block of this launch publishes the key (blocks that skipped count too: the map they saw was complete)
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        if (atomicAdd(&H->done[slot], 1u) == gridDim.x - 1) {
-            H->done[slot] = 0;
-            *reinterpret_cast<volatile unsigned long long *>(&H->key) = s_key;
-            __threadfence();
-        }
-    }
-}
-
-
 // The float32 arm from the tables (see the header of this file): elbow, half of link 2, link 1's hazard bit.
 struct TableArm { float2 ev, hv; uint32_t hazard; };
 __device__ __forceinline__ TableArm table_arm(double q1, double q2, double phase_scale, uint32_t lut1_a, uint32_t lut2_a) {
-    const uint32_t x1 = (uint32_t)__double2loint(fma(q1, phase_scale, PHASE_MAGIC));
-    const uint32_t x2 = (uint32_t)__double2loint(fma(q2, phase_scale, PHASE_MAGIC));
+    const uint32_t x1 = cmap_phase(q1, phase_scale), x2 = cmap_phase(q2, phase_scale);
     const float2 t1 = lds_f2(lut1_a + ((x1 >> (29 - B1)) & (uint32_t)((N1 - 1) << 3)));
     const float2 t2 = lds_f2(lut2_a + ((x2 >> (29 - B2)) & (uint32_t)((N2 - 1) << 3)));
     const float dA = fmaf(__uint_as_float((x1 & ((1u << (32 - B1)) - 1u)) | 0x4B000000u), RAD_PER_UNIT, C0_1);
@@ -553,9 +330,7 @@ k_rollout_lut(const __grid_constant__ ag_params P, const __grid_constant__ GridD
         build_fast_list(G, V, &s_fl);
     }
     if constexpr (CMAP) {                                                        // ---- the map: global -> shared
-        const uint4 *src = reinterpret_cast<const uint4 *>(L.cmap);
-        uint4 *dst = reinterpret_cast<uint4 *>(smem_grid + L.cmap_off);
-        for (int i = threadIdx.x; i < CMAP_WORDS / 4; i += LB) dst[i] = src[i];
+        cmap_to_shared(smem_grid + L.cmap_off, L.cmap, LB);
     } else {                                                                     // ---- the two tables
         const int m = s_fl.m;
         if ((int)threadIdx.x < m) hazard_interval(s_fl.sq[threadIdx.x], P.link_1, 2.0e-6, s_hz[2 * threadIdx.x], s_hz[2 * threadIdx.x + 1]);
@@ -681,12 +456,9 @@ k_rollout_lut(const __grid_constant__ ag_params P, const __grid_constant__ GridD
                 d2 = __dmul_rn(__dsub_rn(u1, 0.5), P.action_scale);              // :85
             }
             q1 = __dadd_rn(q1, d1); q2 = __dadd_rn(q2, d2);                      // two_joint_robot.py:71-72
-            const bool inr = (fabs(q1) < 1048576.0) && (fabs(q2) < 1048576.0);   // NaN-safe: NaN is slow
+            const bool inr = cmap_in_range(q1) && cmap_in_range(q2);              // NaN-safe: NaN is slow
             if constexpr (CMAP) {
-                const uint32_t x1 = (uint32_t)__double2loint(fma(q1, L.phase_scale, PHASE_MAGIC));
-                const uint32_t x2 = (uint32_t)__double2loint(fma(q2, L.phase_scale, PHASE_MAGIC));
-                const uint32_t bit = ((x1 >> (32 - CB1)) << CB2) | (x2 >> (32 - CB2));
-                const uint32_t w = lds_u32(cmap_a + ((bit >> 3) & ~3u));
+                const bool set = cmap_bit(cmap_a, cmap_phase(q1, L.phase_scale), cmap_phase(q2, L.phase_scale));
                 l_inr = inr;
                 if (RECORD) {
                     __stcs(reinterpret_cast<float *>(p1), (float)q1);
@@ -694,7 +466,7 @@ k_rollout_lut(const __grid_constant__ ag_params P, const __grid_constant__ GridD
                     p1 += sr; p2 += sr;
                 }
                 // a set bit, sticky state (thr == INF), or an angle outside the phase's range (also NaN)
-                return (((w >> (bit & 31u)) & 1u) != 0) || !(thr < INF) || !inr;
+                return set || !(thr < INF) || !inr;
             }
             const TableArm ta = table_arm(q1, q2, L.phase_scale, lut1_a, lut2_a);
             const float2 ev = ta.ev, hv = ta.hv;
@@ -865,21 +637,14 @@ k_rollout_lut(const __grid_constant__ ag_params P, const __grid_constant__ GridD
     }
 }
 
-int sm_slots(const void *kernel, size_t smem) {
-    int dev = 0, sms = 0, occ = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return 0;
-    if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, LB, smem) != cudaSuccess) return 0;
-    return sms * occ;
-}
-
 template <bool HA, bool REC, bool M3, bool CM>
 ag_status launch_t(const ag_params &P, const GridDev &G, const RolloutDev &A, const LutConst &L, size_t smem, cudaStream_t s) {
     auto k = k_rollout_lut<HA, REC, M3, CM>;
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (ag_status)e;
-    const int slots = sm_slots(reinterpret_cast<const void *>(k), smem);
-    if (slots <= 0) return (ag_status)cudaGetLastError();
+    int slots = 0;
+    const ag_status st = resident_blocks(k, LB, smem, &slots);
+    if (st != AG_OK) return st;
     const int64_t want = (L.n_tiles + LW - 1) / LW;
     const unsigned blocks = (unsigned)(want < slots ? want : slots);
     k<<<blocks, LB, smem, s>>>(P, G, make_fast_const(P, G), A, L);
@@ -899,104 +664,9 @@ bool rollout_lut_applies(const ag_params &P, const GridDev &G, const RolloutDev 
     return !legacy && cspace_map_applies(G, A.max_occupied) && !P.choose_j_tar && (!rec || A.zfill) && budget;
 }
 
-// ---- the library-owned buffers of the configuration-space maps: up to 32 entries (33 KB each) per process, found by (device, grid
-// pointers, parameters); the CONTENT is validated on the device by every launch (k_cspace_build), so a grid that was
-// rewritten in place, or a new grid at a recycled address, just rebuilds the entry.
-namespace {
-struct CmapEntry {
-    int dev = -1;
-    const void *bits = nullptr, *min_x = nullptr;
-    double par[6] = {0, 0, 0, 0, 0, 0};
-    int S = 0;
-    uint32_t *buf = nullptr;
-    unsigned long long last_use = 0;
-};
-constexpr int CMAP_ENTRIES = 32;
-std::mutex g_cmap_mutex;
-CmapEntry g_cmap[CMAP_ENTRIES];
-unsigned long long g_cmap_clock = 0;
-
-// the entry's device buffer (header + map), or nullptr when the map form cannot be used for this launch
-uint32_t *cmap_buffer(const ag_params &P, const GridDev &G, cudaStream_t s) {
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return nullptr;
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    if (cudaStreamIsCapturing(s, &cap) != cudaSuccess) { cudaGetLastError(); return nullptr; }
-    const bool capturing = cap != cudaStreamCaptureStatusNone;
-    const double par[6] = {P.link_1, P.link_2, P.target_x, P.target_y, P.reach_eps, G.side};
-    std::lock_guard<std::mutex> lock(g_cmap_mutex);
-    CmapEntry *hit = nullptr, *lru = &g_cmap[0];
-    for (CmapEntry &e : g_cmap) {
-        if (e.buf != nullptr && e.dev == dev && e.bits == G.bits && e.min_x == G.min_x && e.S == G.S &&
-            std::memcmp(e.par, par, sizeof(par)) == 0) { hit = &e; break; }
-        if (e.last_use < lru->last_use) lru = &e;
-    }
-    if (hit == nullptr) {
-        if (capturing) return nullptr;                        // no allocation / synchronisation inside a stream capture
-        if (lru->buf != nullptr) {
-            // the buffer changes hands: launches that still read the old map (any stream of its device) must be done
-            int cur = dev;
-            if (lru->dev != cur && cudaSetDevice(lru->dev) != cudaSuccess) return nullptr;
-            cudaDeviceSynchronize();
-            if (lru->dev != cur) { cudaFree(lru->buf); lru->buf = nullptr; cudaSetDevice(cur); }
-        }
-        if (lru->buf == nullptr && cudaMalloc(&lru->buf, (size_t)(CMAP_HDR_WORDS + CMAP_WORDS) * 4) != cudaSuccess) {
-            cudaGetLastError();
-            lru->buf = nullptr; lru->dev = -1;
-            return nullptr;
-        }
-        if (cudaMemsetAsync(lru->buf, 0, CMAP_HDR_WORDS * 4, s) != cudaSuccess) { cudaGetLastError(); return nullptr; }
-        lru->dev = dev; lru->bits = G.bits; lru->min_x = G.min_x; lru->S = G.S;
-        std::memcpy(lru->par, par, sizeof(par));
-        hit = lru;
-    }
-    hit->last_use = ++g_cmap_clock;
-    return hit->buf;
-}
-}  // namespace
-
-bool cspace_map_applies(const GridDev &G, int32_t max_occupied) {
-    return G.stage && G.n_grids == 1 && G.S <= 32 && max_occupied >= 0 && max_occupied <= AG_LIST_MAX;
-}
-
-ag_status cspace_map_for_launch(const ag_params &P, const GridDev &G, cudaStream_t s, const uint32_t **map) {
-    *map = nullptr;
-    uint32_t *buf = cmap_buffer(P, G, s);
-    if (buf == nullptr) return AG_OK;
-    static std::atomic<unsigned> next_build{0};
-    k_cspace_build<<<CMAP_BUILD_BLOCKS, 256, 0, s>>>(P, G, buf, next_build.fetch_add(1, std::memory_order_relaxed) % CMAP_SLOTS);
-    ag_note_launch();
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return (ag_status)e;
-    *map = buf + CMAP_HDR_WORDS;
-    return AG_OK;
-}
-
-int64_t cspace_map_words(int32_t *b1, int32_t *b2) {
-    if (b1) *b1 = CB1;
-    if (b2) *b2 = CB2;
-    return CMAP_WORDS;
-}
-
-// the map alone, into a caller's buffer (ag_cspace_map): built in a scratch buffer with the header in front
-ag_status launch_cspace_map(const ag_params &P, const GridDev &G, uint32_t *map, cudaStream_t s) {
-    uint32_t *buf = nullptr;
-    cudaError_t e = cudaMallocAsync(&buf, (size_t)(CMAP_HDR_WORDS + CMAP_WORDS) * 4, s);
-    if (e != cudaSuccess) return (ag_status)e;
-    e = cudaMemsetAsync(buf, 0, CMAP_HDR_WORDS * 4, s);
-    if (e == cudaSuccess) {
-        k_cspace_build<<<CMAP_BUILD_BLOCKS, 256, 0, s>>>(P, G, buf, 0);
-        ag_note_launch();
-        e = cudaGetLastError();
-    }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(map, buf + CMAP_HDR_WORDS, (size_t)CMAP_WORDS * 4, cudaMemcpyDeviceToDevice, s);
-    cudaFreeAsync(buf, s);
-    return (ag_status)e;
-}
-
 ag_status launch_rollout_lut(const ag_params &P, const GridDev &G, const RolloutDev &A, size_t smem_grid, cudaStream_t s) {
     LutConst L;
-    L.phase_scale = 4294967296.0 / TWO_PI;
+    L.phase_scale = PHASE_SCALE;
     L.thr_c = (float)P.reach_eps + (AG_DELTA_P + 2.0e-7f);
     L.n_tiles = (A.n + 31) / 32;
     static std::atomic<unsigned> next_slot{0};
@@ -1006,17 +676,13 @@ ag_status launch_rollout_lut(const ag_params &P, const GridDev &G, const Rollout
     const bool ha = A.actions != nullptr, rec = A.rec_j1 != nullptr;
     // the unrolled form tests three squares (scene_0's map); fewer are padded with far-away ones in the kernel
     const bool m3 = A.max_occupied >= 0 && A.max_occupied <= 3;
-    // The map form: scene-wide target only (the map holds the target box), |link| small enough for the build's margins
-    static const bool no_cmap = std::getenv("AG_ROLLOUT_NO_CMAP") != nullptr;
-    L.cmap = nullptr; L.cmap_off = 0;
-    if (!no_cmap && A.targets == nullptr) {
-        const ag_status st = cspace_map_for_launch(P, G, s, &L.cmap);
+    // The map form: scene-wide target only (the map holds the target box)
+    CmapLaunch cm = {nullptr, 0, smem};
+    if (A.targets == nullptr) {
+        const ag_status st = cspace_map_for_launch(P, G, A.max_occupied, smem, s, &cm);
         if (st != AG_OK) return st;
-        if (L.cmap != nullptr) {
-            L.cmap_off = (uint32_t)((smem + 15) & ~(size_t)15);
-            smem = (size_t)L.cmap_off + (size_t)CMAP_WORDS * 4;
-        }
     }
+    L.cmap = cm.map; L.cmap_off = cm.off; smem = cm.smem;
 #define AG_LUT(HA, REC) (L.cmap ? launch_t<HA, REC, false, true>(P, G, A, L, smem, s) \
                                 : (m3 ? launch_t<HA, REC, true, false>(P, G, A, L, smem, s) : launch_t<HA, REC, false, false>(P, G, A, L, smem, s)))
     if (ha) return rec ? AG_LUT(true, true) : AG_LUT(true, false);

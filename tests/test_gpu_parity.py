@@ -1343,11 +1343,13 @@ def test_grid_forms_rollout_vs_oracle(ag, torch_, oracle, form, monkeypatch):
 def test_map_form_random_scenes_vs_oracle(ag, torch_, oracle):
     """the headline kernel's configuration-space map on random scene_0-class scenes: random small maps (1..8 occupied
     cells, 5..32 cells per side), random link lengths and targets -- every recorded flag, reward, joint, the
-    final state and the episode counters against the oracle.  AG_SOAK=<n> runs n scenes instead of 6."""
+    final state and the episode counters against the oracle.  AG_SOAK=<n> runs n scenes instead of 6.
+    One more scene has scene_0's obstacles and every other scripted reset candidate at u in [-1e6, -6e5]: such a pose
+    (q = 2 pi u) is outside the range of the map's phase, so the map must not accept it as free."""
     rng = np.random.default_rng(2024)
     n_scenes = int(os.environ.get("AG_SOAK", "6"))
     n, K = 4096, 24
-    for it in range(n_scenes):
+    for it in range(n_scenes + 1):
         S = int(rng.integers(5, 33))
         occ = np.zeros((S, S), np.uint8)
         m = int(rng.integers(1, 9))
@@ -1359,6 +1361,11 @@ def test_map_form_random_scenes_vs_oracle(ag, torch_, oracle):
         j1, j2 = rng.uniform(0, 2 * np.pi, n), rng.uniform(0, 2 * np.pi, n)
         actions = ((rng.random((K, n, 2)) - 0.5) * 0.1).astype(np.float32)
         reset_u = rng.random((n, 40, 2))
+        if it == n_scenes:
+            S, m, l1, l2 = 9, 3, 0.4, 0.3
+            occ = np.zeros((S, S), np.uint8)
+            occ[[5, 5, 2], [6, 7, 3]] = 1
+            reset_u[:, ::2] = rng.uniform(-1.0e6, -6.0e5, (n, 20, 2))
         grid = ag.OccupancyGrid(size=9, random_obstacle=False)
         grid.load_from_matrix(occ)
         robot = ag.BatchedTwoJointRobot(torch_.as_tensor(j1, device="cuda"), torch_.as_tensor(j2, device="cuda"), link_1=l1, link_2=l2)

@@ -3,6 +3,9 @@
 #   tools/ab_build.sh NAME "-DAG_LUT_BLOCKS_PER_SM=3 ..." [TU=ag_rollout_lut]
 # compiles csrc/$TU.cu with the extra flags and links it with the in-tree objects of the other units
 # (abstract_gym_b200/build/*.o from `python -m abstract_gym_b200.build`) into build_ab/NAME.so.
+# A flag that more than one unit reads needs a full build instead: -DAG_CMAP_B1/B2 changes the map's layout, which
+# ag_cmap.cu (the producer) and ag_rollout_lut.cu, ag_motion.cu, ag_cspace.cu (the readers) must agree on:
+#   AG_NVCC_EXTRA="-DAG_CMAP_B1=11" python -m abstract_gym_b200.build --out build_ab/NAME.so
 set -e
 name=$1; flags=$2; tu=${3:-ag_rollout_lut}
 here=$(cd "$(dirname "$0")/.." && pwd)
