@@ -16,7 +16,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 INCLUDE = os.path.join(HERE, "..", "include")
 LIB = os.environ.get("AG_LIB_PATH") or os.path.join(HERE, "libabstract_gym_b200.so")   # AG_LIB_PATH: A/B builds
-SOURCES = ["ag_kernels.cu", "ag_rollout_lut.cu", "ag_cmap.cu", "ag_dense.cu", "ag_motion.cu", "ag_cspace.cu", "ag_host.cu"]
+SOURCES = ["ag_kernels.cu", "ag_rollout_lut.cu", "ag_cmap.cu", "ag_motion.cu", "ag_cspace.cu", "ag_host.cu"]
 HEADERS = ["ag_device.cuh", "ag_fast.cuh", "ag_rollout.cuh", "ag_cmap.cuh", os.path.join(INCLUDE, "abstract_gym_b200.h")]
 OBJDIR = os.path.join(HERE, "build")
 DEBUG_LIB = os.path.join(HERE, "libabstract_gym_b200_debug.so")

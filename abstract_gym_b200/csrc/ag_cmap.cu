@@ -4,12 +4,10 @@
 #include <cstring>
 #include <mutex>
 
-#include "ag_fast.cuh"
 #include "ag_cmap.cuh"
+#include "ag_rollout.cuh"
 
 using namespace agd;
-
-void ag_note_launch();
 
 namespace {
 
@@ -250,9 +248,8 @@ ag_status cspace_map_for_launch(const ag_params &P, const GridDev &G, int32_t ma
     if (buf == nullptr) return AG_OK;
     static std::atomic<unsigned> next_build{0};
     k_cspace_build<<<CMAP_BUILD_BLOCKS, 256, 0, s>>>(P, G, buf, next_build.fetch_add(1, std::memory_order_relaxed) % CMAP_SLOTS);
-    ag_note_launch();
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return (ag_status)e;
+    const ag_status st = launched();
+    if (st != AG_OK) return st;
     out->map = buf + CMAP_HDR_WORDS;
     out->off = (uint32_t)((smem + 15) & ~(size_t)15);
     out->smem = (size_t)out->off + (size_t)CMAP_WORDS * 4;
@@ -273,8 +270,7 @@ ag_status launch_cspace_map(const ag_params &P, const GridDev &G, uint32_t *map,
     e = cudaMemsetAsync(buf, 0, CMAP_HDR_WORDS * 4, s);
     if (e == cudaSuccess) {
         k_cspace_build<<<CMAP_BUILD_BLOCKS, 256, 0, s>>>(P, G, buf, 0);
-        ag_note_launch();
-        e = cudaGetLastError();
+        e = (cudaError_t)launched();
     }
     if (e == cudaSuccess) e = cudaMemcpyAsync(map, buf + CMAP_HDR_WORDS, (size_t)CMAP_WORDS * 4, cudaMemcpyDeviceToDevice, s);
     cudaFreeAsync(buf, s);

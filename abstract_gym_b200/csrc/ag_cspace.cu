@@ -23,8 +23,6 @@
 
 using namespace agd;
 
-void ag_note_launch();
-
 namespace {
 
 // words (of 32 poses) per unit: the row form tests link 1 once per 128 poses.  FAST shares nothing along a row, but
@@ -126,12 +124,10 @@ k_cspace(const __grid_constant__ ag_params P, const __grid_constant__ GridDev G,
 template <int ENGINE, bool MAP>
 ag_status launch(const ag_params &P, const GridDev &G, const CspaceDev &D0, size_t smem, cudaStream_t s) {
     auto k = k_cspace<ENGINE, MAP>;
-    if (smem > 0) {
-        const cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return (ag_status)e;
-    }
+    ag_status st = set_smem(k, smem);
+    if (st != AG_OK) return st;
     int slots = 0;
-    const ag_status st = resident_blocks(k, AG_BLOCK, smem, &slots);
+    st = resident_blocks(k, AG_BLOCK, smem, &slots);
     if (st != AG_OK) return st;
     // Blocks per grid: one unit per warp at most; otherwise about one wave of blocks in all (map form: every block
     // copies the 32 KB map once) or four (the other forms: grids differ in cost, so finer blocks balance better).
@@ -141,8 +137,7 @@ ag_status launch(const ag_params &P, const GridDev &G, const CspaceDev &D0, size
     const int64_t per_grid = (want + G.n_grids - 1) / G.n_grids, most = (D.units + WARPS - 1) / WARPS;
     D.blocks_per_grid = per_grid < most ? per_grid : most;
     k<<<(unsigned)(D.blocks_per_grid * G.n_grids), AG_BLOCK, smem, s>>>(P, G, make_fast_const(P, G), D);
-    ag_note_launch();
-    return (ag_status)cudaGetLastError();
+    return launched();
 }
 
 }  // namespace

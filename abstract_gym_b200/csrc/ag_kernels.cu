@@ -3,7 +3,6 @@
 #include <atomic>
 #include <climits>
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 
 #include "ag_rollout.cuh"
@@ -23,9 +22,6 @@ ag_status launch_check_motion(const ag_params &P, const GridDev &G, int32_t max_
 ag_status launch_cspace_occupancy(const ag_params &P, const GridDev &G, int32_t max_occupied, double lo1, double step1,
                                   int32_t b1, double lo2, double step2, int32_t b2, uint32_t *bits, int64_t *free_count,
                                   int32_t engine, size_t smem, cudaStream_t s);
-// ag_dense.cu: the warp-cooperative kernel for grids that go through the cell traversal (needs the transposed planes)
-bool rollout_coop_applies(const ag_params &P, const GridDev &G, const RolloutDev &A);
-ag_status launch_rollout_coop(const ag_params &P, const GridDev &G, const RolloutDev &A, size_t smem, cudaStream_t s);
 
 namespace {
 
@@ -512,10 +508,7 @@ k_rollout(const __grid_constant__ ag_params P, const __grid_constant__ GridDev G
                         const float2 an = s_ring[((uint32_t)t & (AG_RING - 1)) * BLOCK + threadIdx.x];
                         d1 = (double)an.x; d2 = (double)an.y;
                     } else {
-                        double u0, u1;
-                        philox_uniform2(A.seed, gid, sc0 + (uint32_t)t, 0u, u0, u1);
-                        d1 = __dmul_rn(__dsub_rn(u0, 0.5), P.action_scale);      // scene_0.py:84
-                        d2 = __dmul_rn(__dsub_rn(u1, 0.5), P.action_scale);      // :85
+                        philox_action(P, A.seed, gid, sc0 + (uint32_t)t, d1, d2);
                     }
                     q1 = __dadd_rn(q1, d1); q2 = __dadd_rn(q2, d2);              // two_joint_robot.py:71-72
                     if constexpr (LIST) {
@@ -655,25 +648,14 @@ k_rollout_async(const __grid_constant__ ag_params P, const __grid_constant__ Gri
                     const float2 a = __ldcs(reinterpret_cast<const float2 *>(A.actions) + (int64_t)t * A.row_stride + e);
                     d1 = (double)a.x; d2 = (double)a.y;
                 } else {
-                    double u0, u1;
-                    philox_uniform2(A.seed, gid, sc0 + (uint32_t)t, 0u, u0, u1);
-                    d1 = __dmul_rn(__dsub_rn(u0, 0.5), P.action_scale);          // scene_0.py:84
-                    d2 = __dmul_rn(__dsub_rn(u1, 0.5), P.action_scale);          // :85
+                    philox_action(P, A.seed, gid, sc0 + (uint32_t)t, d1, d2);
                 }
                 q1 = __dadd_rn(q1, d1); q2 = __dadd_rn(q2, d2);                  // two_joint_robot.py:71-72
             } else if (tries >= P.max_reset_tries || (HAS_RESET_U && rc >= (uint32_t)A.R)) {
                 stuck = true;                                                    // give up: keep the last candidate
             } else {                                                             // ---- RESET: scene_0.py:179-181
-                double u0, u1;
-                if (HAS_RESET_U) {
-                    const double2 u = reinterpret_cast<const double2 *>(ru)[rc];
-                    u0 = u.x; u1 = u.y;
-                } else {
-                    philox_uniform2(A.seed, gid, rc, 1u, u0, u1);
-                }
-                ++rc; ++tries;
-                q1 = __dmul_rn(__dmul_rn(u0, 3.141592653589793), 2.0);           // scene_0.py:180  rand()*pi*2.0
-                q2 = __dmul_rn(__dmul_rn(u1, 3.141592653589793), 2.0);           // :181
+                reset_candidate<HAS_RESET_U>(A.seed, gid, rc, ru, q1, q2);
+                ++tries;
             }
             // ---- one pose check per lane and iteration, whatever the mode, with all lanes converged
             __syncwarp(live);
@@ -711,13 +693,8 @@ k_rollout_async(const __grid_constant__ ag_params P, const __grid_constant__ Gri
 }
 
 // ------------------------------------------------------------------------------------- host side
-int stage_max_bytes() {
-    static int v = [] {
-        const char *s = std::getenv("AG_STAGE_MAX_BYTES");
-        return s ? std::atoi(s) : 32768;
-    }();
-    return v;
-}
+// the largest grid footprint (bits, transposed bits, two-level form, cell tables) a block copies to shared memory
+constexpr size_t STAGE_MAX_BYTES = 32768;
 
 ag_status make_grid_dev(const ag_params *p, const ag_grid *g, int64_t env_id0, int engine, GridDev *out,
                         size_t *smem_bytes) {
@@ -746,30 +723,10 @@ ag_status make_grid_dev(const ag_params *p, const ag_grid *g, int64_t env_id0, i
     const bool uniform = g->n_grids == 1 || (g->envs_per_grid % AG_BLOCK == 0 && env_id0 % AG_BLOCK == 0);
     const bool aligned = ((uintptr_t)g->bits % 16 == 0) && ((uintptr_t)g->bits_t % 16 == 0) && ((uintptr_t)g->hier % 16 == 0) &&
                          (g->grid_stride_words % 4 == 0);
-    d.stage = (uniform && aligned && bytes <= (size_t)stage_max_bytes()) ? 1 : 0;
+    d.stage = (uniform && aligned && bytes <= STAGE_MAX_BYTES) ? 1 : 0;
     *smem_bytes = d.stage ? bytes : 0;
     *out = d;
     return AG_OK;
-}
-
-// Without the opt-in a launch may use 48 KB of shared memory INCLUDING the kernel's static part (the 256-thread
-// rollout kernels carry ~22 KB of it), so the attribute is set whenever static + dynamic exceeds 48 KB.
-template <typename Kern>
-ag_status set_smem(Kern k, size_t smem) {
-    if (smem == 0) return AG_OK;
-    cudaFuncAttributes at;
-    cudaError_t e = cudaFuncGetAttributes(&at, k);
-    if (e != cudaSuccess) return (ag_status)e;
-    if (smem + at.sharedSizeBytes > 48 * 1024 && (int)smem > at.maxDynamicSharedSizeBytes) {
-        e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return (ag_status)e;
-    }
-    return AG_OK;
-}
-
-inline ag_status launched() {
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    return (ag_status)cudaGetLastError();
 }
 
 inline unsigned blocks_for(int64_t n) { return (unsigned)((n + AG_BLOCK - 1) / AG_BLOCK); }
@@ -781,6 +738,10 @@ inline unsigned blocks_for(int64_t n) { return (unsigned)((n + AG_BLOCK - 1) / A
         case AG_ENGINE_BRUTE: { constexpr int E = AG_ENGINE_BRUTE; __VA_ARGS__; break; } \
         default: return AG_ERR_MODE;                                      \
     }
+
+// K1 / K2 with first_hit: the FAST engine computes the flag with the EXACT arithmetic (pose_collides, k_step), so those
+// launches run the EXACT kernels
+constexpr int first_hit_engine(int engine) { return engine == AG_ENGINE_FAST ? AG_ENGINE_EXACT : engine; }
 
 template <int E, int BP, bool HA, bool HR, bool REC, bool FULL, int BLOCK>
 ag_status launch_rollout_b(const ag_params &P, const GridDev &G, const RolloutDev &A, size_t smem, cudaStream_t s) {
@@ -810,14 +771,16 @@ ag_status launch_rollout_t(const ag_params &P, const GridDev &G, const RolloutDe
         if (st) return st;
         k<<<blocks_for(A.n), AG_BLOCK, smem, s>>>(P, G, make_fast_const(P, G), A);
         return launched();
+    } else if constexpr (E == AG_ENGINE_FAST) {                      // obstacle list
+        if (G.n_grids == 1) {
+            // complete warps only (n % 32 == 0): the warp votes use a constant full mask
+            if (A.n % 32 == 0) return launch_rollout_b<E, BP, HA, HR, REC, true, AG_SMALL_BLOCK>(P, G, A, smem, s);
+            return launch_rollout_b<E, BP, HA, HR, REC, false, AG_SMALL_BLOCK>(P, G, A, smem, s);
+        }
+        return launch_rollout_b<E, BP, HA, HR, REC, false, AG_BLOCK>(P, G, A, smem, s);
+    } else {                                                         // EXACT / BRUTE
+        return launch_rollout_b<E, BP, HA, HR, REC, false, AG_BLOCK>(P, G, A, smem, s);
     }
-    if (E == AG_ENGINE_FAST && BP == BP_LIST && G.n_grids == 1) {
-        // complete warps only (n % 32 == 0): the warp votes use a constant full mask
-        if (A.n % 32 == 0)
-            return launch_rollout_b<E, BP, HA, HR, REC, E == AG_ENGINE_FAST && BP == BP_LIST, AG_SMALL_BLOCK>(P, G, A, smem, s);
-        return launch_rollout_b<E, BP, HA, HR, REC, false, AG_SMALL_BLOCK>(P, G, A, smem, s);
-    }
-    return launch_rollout_b<E, BP, HA, HR, REC, false, AG_BLOCK>(P, G, A, smem, s);
 }
 
 template <int E, int BP>
@@ -876,7 +839,6 @@ ag_status ag_rollout_impl(const ag_params *p, const ag_grid *g, const ag_rollout
         const bool list = G.stage && g->S <= 32 && g->max_occupied >= 0 && g->max_occupied <= AG_LIST_MAX;
         if (list && rollout_lut_applies(*p, G, A)) return launch_rollout_lut(*p, G, A, smem, s);
         if (list) return launch_rollout_e<AG_ENGINE_FAST, BP_LIST>(*p, G, A, smem, s);
-        if (rollout_coop_applies(*p, G, A)) return launch_rollout_coop(*p, G, A, smem, s);
         return launch_rollout_e<AG_ENGINE_FAST, BP_TRAVERSAL>(*p, G, A, smem, s);
     }
     if (a->engine == AG_ENGINE_EXACT) return launch_rollout_e<AG_ENGINE_EXACT, BP_ANY>(*p, G, A, smem, s);
@@ -967,7 +929,7 @@ ag_status ag_collision_check(const ag_params *p, const ag_grid *g, const double 
     cudaStream_t s = (cudaStream_t)stream;
     AG_DISPATCH_ENGINE(engine, {
         if (first_hit) {
-            auto k = k_collision<E, true>;
+            auto k = k_collision<first_hit_engine(E), true>;
             if ((st = set_smem(k, smem))) return st;
             k<<<blocks_for(n), AG_BLOCK, smem, s>>>(*p, G, j1, j2, hit, first_hit, n, env_id0);
         } else {
@@ -1029,7 +991,7 @@ ag_status ag_step(const ag_params *p, const ag_grid *g, double *j1, double *j2, 
         return AG_ERR_ALIGN;
     cudaStream_t s = (cudaStream_t)stream;
     unsigned long long *ust = reinterpret_cast<unsigned long long *>(stats);
-#define AG_STEP(F32, WF) { auto k = k_step<E, F32, WF>; if ((st = set_smem(k, smem))) return st; \
+#define AG_STEP(F32, WF) { auto k = k_step<(WF ? first_hit_engine(E) : E), F32, WF>; if ((st = set_smem(k, smem))) return st; \
         k<<<blocks_for(n), AG_BLOCK, smem, s>>>(*p, G, j1, j2, actions, reward, flags, ee, dist, first_hit, ust, targets, n, env_id0); }
     AG_DISPATCH_ENGINE(engine, {
         if (actions_f32) { if (first_hit) AG_STEP(true, true) else AG_STEP(true, false) }

@@ -19,8 +19,6 @@
 
 using namespace agd;
 
-void ag_note_launch();
-
 namespace {
 
 struct MotionDev {
@@ -87,20 +85,17 @@ __global__ void __launch_bounds__(AG_BLOCK, 1) k_check_motion(const __grid_const
 template <int ENGINE, bool MAP>
 ag_status launch(const ag_params &P, const GridDev &G, const MotionDev &M, size_t smem, cudaStream_t s) {
     auto k = k_check_motion<ENGINE, MAP>;
-    if (smem > 0) {
-        const cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return (ag_status)e;
-    }
+    ag_status st = set_smem(k, smem);
+    if (st != AG_OK) return st;
     int64_t blocks = (M.m + AG_BLOCK - 1) / AG_BLOCK;
     if (MAP) {                                                                   // persistent: as many blocks as fit at once
         int slots = 0;
-        const ag_status st = resident_blocks(k, AG_BLOCK, smem, &slots);
+        st = resident_blocks(k, AG_BLOCK, smem, &slots);
         if (st != AG_OK) return st;
         blocks = blocks < slots ? blocks : slots;
     }
     k<<<(unsigned)blocks, AG_BLOCK, smem, s>>>(P, G, make_fast_const(P, G), M);
-    ag_note_launch();
-    return (ag_status)cudaGetLastError();
+    return launched();
 }
 
 }  // namespace

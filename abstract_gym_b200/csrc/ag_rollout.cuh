@@ -1,15 +1,40 @@
 // ag_rollout.cuh -- pieces shared by the rollout kernels (ag_kernels.cu: K1..K5 and the general K4;
-// ag_rollout_lut.cu: the persistent scene_0-class K4), motion checking (ag_motion.cu) and occupancy (ag_cspace.cu).
+// ag_rollout_lut.cu: the persistent scene_0-class K4), motion checking (ag_motion.cu) and occupancy (ag_cspace.cu),
+// and the launch helpers every launcher uses (ag_cmap.cu too).
 #pragma once
 #include <climits>
 
 #include "ag_device.cuh"
 #include "ag_fast.cuh"
 
+void ag_note_launch();   // ag_kernels.cu: counts kernel launches (ag_launch_count)
+
 namespace agd {
 
 constexpr int AG_BLOCK = 256;
 static_assert(AG_BLOCK <= AG_TILEQ_COLS, "the tile queue of arm_fast_hier has one column per thread");
+
+// Opt a kernel in to `smem` bytes of dynamic shared memory.  Without the opt-in a launch may use 48 KB INCLUDING the
+// kernel's static part (the 256-thread rollout kernels carry ~22 KB of it), so the attribute is set whenever static +
+// dynamic exceeds 48 KB and the kernel's current limit.
+template <typename Kernel>
+ag_status set_smem(Kernel kernel, size_t smem) {
+    if (smem == 0) return AG_OK;
+    cudaFuncAttributes at;
+    cudaError_t e = cudaFuncGetAttributes(&at, kernel);
+    if (e != cudaSuccess) return (ag_status)e;
+    if (smem + at.sharedSizeBytes > 48 * 1024 && (int)smem > at.maxDynamicSharedSizeBytes) {
+        e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return (ag_status)e;
+    }
+    return AG_OK;
+}
+
+// after a kernel launch: count it and return the launch's error
+inline ag_status launched() {
+    ag_note_launch();
+    return (ag_status)cudaGetLastError();
+}
 
 // the grid of a persistent launch: blocks of `kernel` resident at once (SM count x blocks per SM at `block` threads and
 // `smem` bytes of dynamic shared memory)
@@ -130,6 +155,33 @@ static __device__ __noinline__ bool pose_hit(const ag_params &P, const GridDev &
     return pose_collides<ENGINE, false, BP>(P, G, B, C, q1, q2, fh, axis);
 }
 
+// The in-kernel action of step counter `ctr` (scenario/scene_0.py:84-85): (rand() - 0.5) * action_scale per joint, from
+// Philox stream 0.  BatchedScene.philox_actions draws the same on the host.
+__device__ __forceinline__ void philox_action(const ag_params &P, uint64_t seed, uint64_t gid, uint32_t ctr, double &d1,
+                                              double &d2) {
+    double u0, u1;
+    philox_uniform2(seed, gid, ctr, 0u, u0, u1);
+    d1 = __dmul_rn(__dsub_rn(u0, 0.5), P.action_scale);
+    d2 = __dmul_rn(__dsub_rn(u1, 0.5), P.action_scale);
+}
+
+// Reset candidate number rc (scenario/scene_0.py:180-181): rand()*pi*2.0 per joint, from Philox stream 1 or, with
+// SCRIPTED, from the caller's uniforms reset_u_env[rc]; advances rc.
+template <bool SCRIPTED>
+__device__ __forceinline__ void reset_candidate(uint64_t seed, uint64_t gid, uint32_t &rc, const double *reset_u_env,
+                                                double &j1, double &j2) {
+    double u0, u1;
+    if (SCRIPTED) {
+        const double2 u = reinterpret_cast<const double2 *>(reset_u_env)[rc];
+        u0 = u.x; u1 = u.y;
+    } else {
+        philox_uniform2(seed, gid, rc, 1u, u0, u1);
+    }
+    ++rc;
+    j1 = __dmul_rn(__dmul_rn(u0, 3.141592653589793), 2.0);
+    j2 = __dmul_rn(__dmul_rn(u1, 3.141592653589793), 2.0);
+}
+
 // shared by K3 and K4: scenario/scene_0.py:174-181 with a bound.  `colliding` is the
 // collision_check() of the current pose.
 template <int ENGINE, bool HAS_RESET_U, int BP = BP_ANY>
@@ -143,16 +195,8 @@ __device__ __forceinline__ void resample_pose(const ag_params &P, const GridDev 
             acc32(s_acc, AG_ST_STUCK_RESETS, 1);
             break;
         }
-        double u0, u1;
-        if (HAS_RESET_U) {
-            const double2 u = reinterpret_cast<const double2 *>(reset_u_env)[rc];
-            u0 = u.x; u1 = u.y;
-        } else {
-            philox_uniform2(seed, gid, rc, 1u, u0, u1);
-        }
-        ++rc; ++tries;
-        j1 = __dmul_rn(__dmul_rn(u0, 3.141592653589793), 2.0);    // scene_0.py:180  rand()*pi*2.0
-        j2 = __dmul_rn(__dmul_rn(u1, 3.141592653589793), 2.0);    // :181
+        reset_candidate<HAS_RESET_U>(seed, gid, rc, reset_u_env, j1, j2);
+        ++tries;
         int fh = 0, axis = 0;
         colliding = pose_collides<ENGINE, false, BP>(P, G, B, C, j1, j2, fh, axis);
         if (axis) acc32(s_acc, AG_ST_AXIS_ALIGNED, axis);

@@ -30,14 +30,11 @@
 // consumed on collision), then K steps of
 //   action (cp.async ring, RING - 1 rows ahead) -> 2 DADD -> test -> record (2 F2F + 2 STG) -> vote.
 #include <atomic>
-#include <cstdlib>
 
 #include "ag_cmap.cuh"
 #include "ag_rollout.cuh"
 
 using namespace agd;
-
-void ag_note_launch();
 
 namespace {
 
@@ -450,10 +447,7 @@ k_rollout_lut(const __grid_constant__ ag_params P, const __grid_constant__ GridD
             if (HAS_ACT) {
                 d1 = (double)a.x; d2 = (double)a.y;
             } else {
-                double u0, u1;
-                philox_uniform2(A.seed, gid, sc0 + (uint32_t)t, 0u, u0, u1);
-                d1 = __dmul_rn(__dsub_rn(u0, 0.5), P.action_scale);              // scene_0.py:84
-                d2 = __dmul_rn(__dsub_rn(u1, 0.5), P.action_scale);              // :85
+                philox_action(P, A.seed, gid, sc0 + (uint32_t)t, d1, d2);
             }
             q1 = __dadd_rn(q1, d1); q2 = __dadd_rn(q2, d2);                      // two_joint_robot.py:71-72
             const bool inr = cmap_in_range(q1) && cmap_in_range(q2);              // NaN-safe: NaN is slow
@@ -640,28 +634,26 @@ k_rollout_lut(const __grid_constant__ ag_params P, const __grid_constant__ GridD
 template <bool HA, bool REC, bool M3, bool CM>
 ag_status launch_t(const ag_params &P, const GridDev &G, const RolloutDev &A, const LutConst &L, size_t smem, cudaStream_t s) {
     auto k = k_rollout_lut<HA, REC, M3, CM>;
-    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return (ag_status)e;
+    ag_status st = set_smem(k, smem);
+    if (st != AG_OK) return st;
     int slots = 0;
-    const ag_status st = resident_blocks(k, LB, smem, &slots);
+    st = resident_blocks(k, LB, smem, &slots);
     if (st != AG_OK) return st;
     const int64_t want = (L.n_tiles + LW - 1) / LW;
     const unsigned blocks = (unsigned)(want < slots ? want : slots);
     k<<<blocks, LB, smem, s>>>(P, G, make_fast_const(P, G), A, L);
-    ag_note_launch();
-    return (ag_status)cudaGetLastError();
+    return launched();
 }
 
 }  // namespace
 
 // The persistent kernel serves the FAST engine on one staged small sparse grid (obstacle list), cartesian target.
 bool rollout_lut_applies(const ag_params &P, const GridDev &G, const RolloutDev &A) {
-    static const bool legacy = std::getenv("AG_ROLLOUT_LEGACY") != nullptr;
     const bool rec = A.rec_j1 != nullptr;   // RECORD: complete tiles and zero-filled reward / flags planes only
     // the table arm's error (2.2e-7 m per metre of link 1, 2.8e-7 per metre of link 2, 5e-8 of rounding) must stay
     // inside the float32 filter's budget AG_DELTA_P
     const bool budget = 2.2e-7 * P.link_1 + 2.8e-7 * P.link_2 + 5.0e-8 <= (double)AG_DELTA_P;
-    return !legacy && cspace_map_applies(G, A.max_occupied) && !P.choose_j_tar && (!rec || A.zfill) && budget;
+    return cspace_map_applies(G, A.max_occupied) && !P.choose_j_tar && (!rec || A.zfill) && budget;
 }
 
 ag_status launch_rollout_lut(const ag_params &P, const GridDev &G, const RolloutDev &A, size_t smem_grid, cudaStream_t s) {

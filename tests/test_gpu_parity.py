@@ -1025,36 +1025,6 @@ def test_fullsize_config5_sampled_vs_oracle(ag, torch_, oracle):
 
 
 @pytest.mark.gpu
-def test_dense_pooled_kernel_equals_default(ag, torch_, oracle):
-    """the opt-in warp-cooperative kernel for dense maps (csrc/ag_dense.cu, AG_DENSE_POOLED=1) against the oracle, in a
-    child process (the switch is read once per process)"""
-    import subprocess
-    import sys
-    code = r'''
-import numpy as np, torch, sys
-sys.path.insert(0, %r)
-import abstract_gym_b200 as ag
-from oracle import oracle as orc
-rng = np.random.default_rng(5)
-occs = [(rng.random((256, 256)) < 0.008).astype(np.uint8) for _ in range(4)]
-n, K = 1024, 12
-j1, j2 = rng.uniform(0, 2 * np.pi, n), rng.uniform(0, 2 * np.pi, n)
-g = ag.BatchedOccupancyGrid(torch.as_tensor(np.stack(occs), device="cuda"), 256)
-sc = ag.BatchedScene(ag.BatchedTwoJointRobot(torch.as_tensor(j1, device="cuda"), torch.as_tensor(j2, device="cuda")), g, engine="fast", seed=3)
-rec = sc.rollout(K)
-torch.cuda.synchronize()
-st = orc.RolloutState(j1, j2)
-orec, ostats = orc.rollout(st, K, [orc.grid_squares(o)[0] for o in occs], envs_per_grid=256, seed=3)
-assert np.array_equal(rec["flags"].cpu().numpy(), orec["flags"]) and np.array_equal(rec["j1"].cpu().numpy(), orec["j1"])
-assert np.array_equal(sc.stats.cpu().numpy(), ostats) and np.array_equal(sc.robot.joint_1.cpu().numpy(), st.j1)
-print("pooled ok", int(ostats[0]))
-''' % os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    env = dict(os.environ, AG_DENSE_POOLED="1", AG_GRID_FORM="transposed")   # the pooled kernel walks bits + transposed bits
-    r = subprocess.run([sys.executable, "-c", code], env=env, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=300)
-    assert r.returncode == 0 and "pooled ok" in r.stdout, r.stdout[-2000:]
-
-
-@pytest.mark.gpu
 @pytest.mark.parametrize("grid_kind", ["scene0", "rand64"])
 def test_event_sink_equals_dense_records(ag, torch_, grid_kind):
     """joints-only records + the event list (ag_rollout_args.events) carry exactly what the four dense planes carry"""
@@ -1240,12 +1210,13 @@ def _traps_per_kernel(path):
 
 
 @pytest.mark.gpu
-def test_debug_bounds_build(ag, torch_):
+def test_debug_bounds_build_per_family(ag, torch_):
     """the -DAG_DEBUG_BOUNDS library (csrc/ag_device.cuh AG_CHECK_INDEX): same results as the oracle on list, traversal
     and brute paths with every index assertion compiled in.  That the assertions are there is read from the machine
     code instead of tripping one: a trap is a device fault that ends the CUDA context, and a test does not set one off
     on purpose.  Every rollout, step, reset and collision kernel of the debug library traps on a bad index (the brute
-    collision kernel on the padding bit of a malformed grid); the release library has no trap at all."""
+    collision kernel on the padding bit of a malformed grid); the release library has no trap at all.  The instantiations
+    of each of those kernel families are counted exactly: the launchers build only the forms their dispatch can reach."""
     import subprocess
     import sys
     from abstract_gym_b200 import build as ag_build
@@ -1257,8 +1228,13 @@ def test_debug_bounds_build(ag, torch_):
     assert r.returncode == 0 and "debug parity ok" in r.stdout, r.stdout[-3000:]
     debug, release = _traps_per_kernel(lib), _traps_per_kernel(ag_build.LIB)
     assert sum(release.values()) == 0 and len(release) == len(debug) > 100
-    checked = [k for k in debug if any(s in k for s in ("k_rollout", "k_step", "k_reset", "k_collision"))]
-    assert len(checked) > 100 and all(debug[k] > 0 for k in checked), [k for k in checked if debug[k] == 0]
+    # instantiations per family; a mangled name holds the length-prefixed identifier, then I for the template arguments
+    families = {"k_rollout": 40, "k_rollout_async": 8, "k_rollout_lut": 12, "k_step": 10, "k_step_obs": 6, "k_reset": 6,
+                "k_collision": 5}
+    per_family = {f: [k for k in debug if "%d%sI" % (len(f), f) in k] for f in families}
+    assert {f: len(ks) for f, ks in per_family.items()} == families
+    checked = sum(per_family.values(), [])
+    assert all(debug[k] > 0 for k in checked), [k for k in checked if debug[k] == 0]
     assert any("k_collisionILi2E" in k and debug[k] > 0 for k in debug)       # ENGINE_BRUTE
 
 
