@@ -22,6 +22,9 @@ ag_status launch_check_motion(const ag_params &P, const GridDev &G, int32_t max_
 ag_status launch_cspace_occupancy(const ag_params &P, const GridDev &G, int32_t max_occupied, double lo1, double step1,
                                   int32_t b1, double lo2, double step2, int32_t b2, uint32_t *bits, int64_t *free_count,
                                   int32_t engine, size_t smem, cudaStream_t s);
+// ag_ccl.cu: free-space components of an occupancy image (ag_cspace_components after argument validation)
+ag_status launch_cspace_components(const uint32_t *bits, int64_t n_grids, int32_t b1, int32_t b2, int32_t wrap,
+                                   int32_t *labels, int64_t *n_components, cudaStream_t s);
 
 namespace {
 
@@ -973,6 +976,18 @@ ag_status ag_cspace_occupancy(const ag_params *p, const ag_grid *g, double lo1, 
     if (engine != AG_ENGINE_EXACT && engine != AG_ENGINE_FAST && engine != AG_ENGINE_BRUTE) return AG_ERR_MODE;
     return launch_cspace_occupancy(*p, G, g->max_occupied, lo1, step1, b1, lo2, step2, b2, bits, free_count, engine, smem,
                                    (cudaStream_t)stream);
+}
+
+ag_status ag_cspace_components(const uint32_t *bits, int64_t n_grids, int32_t b1, int32_t b2, int32_t wrap, int32_t *labels,
+                               int64_t *n_components, void *stream) {
+    if (n_grids < 0 || b1 < 1 || b2 < 1) return AG_ERR_SHAPE;
+    const int64_t poses = (int64_t)b1 * b2;
+    if (poses > INT32_MAX || (n_grids > 0 && poses > INT64_MAX / n_grids)) return AG_ERR_SHAPE;   // grid-local int32 labels
+    if (wrap & ~3) return AG_ERR_MODE;
+    if (n_grids == 0) return AG_OK;
+    if (!bits || !labels) return AG_ERR_NULL;
+    if (((uintptr_t)bits % 4) || ((uintptr_t)labels % 4) || ((uintptr_t)n_components % 8)) return AG_ERR_ALIGN;
+    return launch_cspace_components(bits, n_grids, b1, b2, wrap, labels, n_components, (cudaStream_t)stream);
 }
 
 ag_status ag_step(const ag_params *p, const ag_grid *g, double *j1, double *j2, const void *actions,

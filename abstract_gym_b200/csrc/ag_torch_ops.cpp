@@ -138,6 +138,26 @@ void cspace_occupancy(const Tensor &params, const Tensor &bits, const OptTensor 
                  "ag_cspace_occupancy");
 }
 
+// connected components of the free poses of cspace_occupancy's words, per grid -> ag_cspace_components
+void cspace_components(const Tensor &occupancy, int64_t b1, int64_t b2, int64_t wrap, Tensor labels, OptTensor n_components) {
+    const c10::Device dev = labels.device();
+    c10::cuda::CUDAGuard guard(dev);
+    need(occupancy, at::kInt, "occupancy", dev);
+    need(labels, at::kInt, "labels", dev);
+    TORCH_CHECK(b1 >= 1 && b2 >= 1 && b1 <= INT32_MAX && b2 <= INT32_MAX && b1 * b2 <= INT32_MAX,
+                "b1 and b2 must be >= 1 with b1 * b2 < 2^31");
+    const int64_t grid_words = b1 * ((b2 + 31) / 32);
+    TORCH_CHECK(occupancy.numel() % grid_words == 0, "occupancy must be [n_grids, b1, ceil(b2/32)] int32 words");
+    const int64_t n_grids = occupancy.numel() / grid_words;
+    TORCH_CHECK(labels.numel() == n_grids * b1 * b2, "labels must be [n_grids, b1, b2] int32");
+    if (n_components.has_value() && n_components->defined())
+        TORCH_CHECK(n_components->numel() == n_grids, "n_components must be [n_grids]");
+    check_status(ag_cspace_components(reinterpret_cast<const uint32_t *>(occupancy.data_ptr()), n_grids, (int32_t)b1,
+                                      (int32_t)b2, (int32_t)wrap, labels.data_ptr<int32_t>(),
+                                      opt_ptr<int64_t>(n_components, at::kLong, "n_components", dev), stream_of(dev)),
+                 "ag_cspace_components");
+}
+
 // Scene.step (scenario/scene_0.py:88-103) -> ag_step
 void step(const Tensor &params, const Tensor &bits, const OptTensor &bits_t, const OptTensor &hier, const Tensor &min_x, const Tensor &min_y, double side,
           double env_size, int64_t S, int64_t n_grids, int64_t max_occupied, int64_t envs_per_grid, Tensor j1, Tensor j2,
@@ -275,6 +295,7 @@ TORCH_LIBRARY(abstract_gym_b200, m) {
           "Tensor(b!)? first_hit, Tensor(c!)? last_free, int env_id0, int engine) -> ()");
     m.def("cspace_occupancy(" AG_GRID_SCHEMA "float lo1, float step1, int b1, float lo2, float step2, int b2, "
           "Tensor(a!) occupancy, Tensor(b!)? free_count, int engine) -> ()");
+    m.def("cspace_components(Tensor occupancy, int b1, int b2, int wrap, Tensor(a!) labels, Tensor(b!)? n_components) -> ()");
     m.def("step(" AG_GRID_SCHEMA "Tensor(a!) j1, Tensor(b!) j2, Tensor actions, Tensor(c!) reward, Tensor(d!) flags, Tensor(e!)? ee, "
           "Tensor(f!)? dist, Tensor(g!)? first_hit, Tensor(h!)? stats, Tensor? targets, int env_id0, int engine) -> ()");
     m.def("reset(" AG_GRID_SCHEMA "Tensor(a!) j1, Tensor(b!) j2, Tensor(c!) reward, Tensor(d!) flags, Tensor(e!) reset_ctr, Tensor? mask, "
@@ -293,6 +314,7 @@ TORCH_LIBRARY_IMPL(abstract_gym_b200, CUDA, m) {
     m.impl("collision_check", &collision_check);
     m.impl("check_motion", &check_motion);
     m.impl("cspace_occupancy", &cspace_occupancy);
+    m.impl("cspace_components", &cspace_components);
     m.impl("step", &step);
     m.impl("reset", &reset);
     m.impl("rollout", &rollout);

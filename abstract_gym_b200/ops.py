@@ -1,5 +1,5 @@
-"""torch custom ops over the C ABI: `torch.ops.abstract_gym_b200.{collision_check, check_motion, cspace_occupancy, step,
-reset, rollout, step_obs}`.
+"""torch custom ops over the C ABI: `torch.ops.abstract_gym_b200.{collision_check, check_motion, cspace_occupancy,
+cspace_components, step, reset, rollout, step_obs}`.
 
 The ops live in a COMPILED library, libabstract_gym_b200_ops.so (csrc/ag_torch_ops.cpp: TORCH_LIBRARY schemas, CUDA-only
 registration), which validates device / dtype / contiguity / shapes, takes the current CUDA stream and calls the
@@ -55,6 +55,7 @@ load()
 collision_check = torch.ops.abstract_gym_b200.collision_check
 check_motion = torch.ops.abstract_gym_b200.check_motion
 cspace_occupancy = torch.ops.abstract_gym_b200.cspace_occupancy
+cspace_components = torch.ops.abstract_gym_b200.cspace_components
 step = torch.ops.abstract_gym_b200.step
 reset = torch.ops.abstract_gym_b200.reset
 rollout = torch.ops.abstract_gym_b200.rollout

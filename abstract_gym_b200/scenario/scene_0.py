@@ -198,6 +198,71 @@ class BatchedScene:
             words = ((words.unsqueeze(-1) >> shifts) & 1).reshape(n_grids, b1, -1)[:, :, :b2] != 0
         return (words, fc) if free_count else words
 
+    @staticmethod
+    def _lattice(b1, b2, lo, step, wrap):
+        """(lo1, lo2), (step1, step2), wrap bits of cspace_components' lattice (the defaults of cspace_occupancy; wrap=None:
+        both axes when the default steps cover the torus, neither otherwise)"""
+        lo1, lo2 = (float(v) for v in lo)
+        st = (2.0 * math.pi / b1, 2.0 * math.pi / b2) if step is None else tuple(float(v) for v in step)
+        w = (step is None, step is None) if wrap is None else tuple(bool(v) for v in wrap)
+        if len(w) != 2:
+            raise ValueError("wrap must be a pair of bools (joint_1, joint_2)")
+        return (lo1, lo2), st, int(w[0]) | int(w[1]) << 1
+
+    def cspace_components(self, b1, b2=None, lo=(0.0, 0.0), step=None, wrap=None, count=False, engine=None):
+        """Connected components of the free poses of cspace_occupancy(b1, b2, lo, step, engine=engine), per grid: which
+        lattice poses reach which through 4-neighbour steps between free poses.  wrap = (joint_1, joint_2) says which
+        axes wrap (row b1-1 next to row 0, column b2-1 next to column 0); None: both when step is None (the default
+        lattice covers the torus), neither otherwise.  Grids never connect to each other.
+        Returns labels int32 [n_grids, b1, b2]: -1 for a colliding pose, else the smallest row-major index i * b2 + j of
+        its component on that grid; with count=True also int64 [n_grids], the components of each grid.
+        This is connectivity of the lattice image, not of continuous joint space: two adjacent free poses can have a
+        colliding pose between them when the lattice is coarse for the grid's cells (check_motion checks such a step)."""
+        b1 = int(b1)
+        b2 = b1 if b2 is None else int(b2)
+        if b1 < 1 or b2 < 1:
+            raise ValueError("the lattice needs b1, b2 >= 1, got %d x %d" % (b1, b2))
+        lo, st, w = self._lattice(b1, b2, lo, step, wrap)
+        words = self.cspace_occupancy(b1, b2, lo=lo, step=st, packed=True, engine=engine)
+        n_grids = words.shape[0]
+        labels = torch.empty(n_grids, b1, b2, dtype=torch.int32, device=self.device)
+        nc = torch.empty(n_grids, dtype=torch.int64, device=self.device) if count else None
+        _lib.check(self._lib.ag_cspace_components(ptr(words), n_grids, b1, b2, w, ptr(labels), ptr(nc),
+                                                  stream_ptr(self.device)), "ag_cspace_components")
+        return (labels, nc) if count else labels
+
+    def cspace_component_of(self, labels, joints=None, lo=(0.0, 0.0), step=None, wrap=None):
+        """The label (cspace_components) at the nearest lattice pose of each of M poses, on the grid of env m
+        (((env_id0 + m) // envs_per_grid) % n_grids, as check_motion).  joints: [M, 2] float64 (default: the current
+        joints, M = N); lo, step, wrap: those of the call that made `labels`.
+        Per axis, in float64: k = floor((q - lo) / step + 0.5); on a wrapping axis k mod b, on any other k outside [0, b)
+        gives -1, and so does a NaN or infinite q.  Returns int32 [M].
+        Whether env i can reach pose t_i on the lattice: component_of(labels)[i] == component_of(labels, t)[i] >= 0."""
+        n_grids, b1, b2 = labels.shape
+        if n_grids != int(self.grid.n_grids):
+            raise ValueError("labels hold %d grids, the scene %d" % (n_grids, int(self.grid.n_grids)))
+        lo, st, w = self._lattice(b1, b2, lo, step, wrap)
+        if joints is None:
+            q = torch.stack([self.robot.joint_1, self.robot.joint_2], dim=1)
+        else:
+            q = as_f64(joints, self.device).reshape(-1, 2)
+        m = q.shape[0]
+        env = self.env_id0 + torch.arange(m, dtype=torch.int64, device=self.device)
+        g = torch.div(env, int(self.grid.envs_per_grid), rounding_mode="floor") % n_grids
+        ok = torch.ones(m, dtype=torch.bool, device=self.device)
+        idx = []
+        for a, b in enumerate((b1, b2)):
+            k = torch.floor((q[:, a] - lo[a]) / st[a] + 0.5)
+            ok &= torch.isfinite(k)
+            if w >> a & 1:
+                k = torch.fmod(k, b)                          # exact for every integer-valued double
+                k = torch.where(k < 0, k + b, k)
+            else:
+                ok &= (k >= 0) & (k < b)
+            idx.append(torch.where(ok, k, 0.0).to(torch.int64))
+        out = labels.to(self.device)[g, idx[0], idx[1]]
+        return torch.where(ok, out, -1).to(torch.int32)
+
     def check_target_reached(self):
         """scene_0.py:115-133 -> bool [N]"""
         eps = 2e-3

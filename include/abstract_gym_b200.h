@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define AG_ABI_VERSION 7
+#define AG_ABI_VERSION 8
 
 #if defined(__GNUC__)
 #define AG_API __attribute__((visibility("default")))
@@ -215,6 +215,27 @@ AG_API ag_status ag_check_motion(const ag_params *p, const ag_grid *g, const dou
 AG_API ag_status ag_cspace_occupancy(const ag_params *p, const ag_grid *g, double lo1, double step1, int32_t b1, double lo2,
                                      double step2, int32_t b2, uint32_t *bits, int64_t *free_count, int32_t engine,
                                      void *stream);
+
+/* Free-space components: the connected components of the free poses (bit 0) of an occupancy image in the layout
+ * ag_cspace_occupancy writes, per grid g = 0 .. n_grids-1.  No grid or params: this is image work on the words alone.
+ * bits: [n_grids][b1][W] uint32 (device, 4-byte aligned), W = ceil(b2 / 32); pose (i, j) is bit j % 32 of word j / 32 of
+ *       row i, 1 = colliding.  Padding bits (j >= b2) are ignored: those poses do not exist.
+ * Free poses (i, j) and (i+-1, j), (i, j+-1) are adjacent (4-neighbour: a diagonal step would pass a blocked corner).
+ * wrap bit 0: row b1-1 is adjacent to row 0 (joint_1 wraps); bit 1: column b2-1 to column 0 (joint_2 wraps); both: the
+ * torus.  A pose is never its own neighbour (b = 1 adds no edge).  Grids never connect to each other.
+ * labels: [n_grids][b1][b2] int32 (device, 4-byte aligned, no padding): -1 for a colliding pose, else the smallest
+ *       row-major index i * b2 + j (local to the grid) of any pose of its component -- canonical, so the result does not
+ *       depend on scheduling.
+ * n_components: optional [n_grids] int64 (device, 8-byte aligned): the components of each grid, written (not
+ *       accumulated).
+ * This is connectivity of the LATTICE image: two adjacent free poses may have a colliding pose between them when the
+ * lattice is coarse for the grid's cells.  Nothing here checks the motion between them (ag_check_motion does).
+ * Errors, in this order, before anything touches the device: n_grids < 0, b1 < 1 or b2 < 1, b1 * b2 > INT32_MAX or
+ * n_grids * b1 * b2 beyond int64 -> AG_ERR_SHAPE; wrap & ~3 -> AG_ERR_MODE; n_grids == 0 -> AG_OK (nothing launched);
+ * bits or labels NULL -> AG_ERR_NULL; a misaligned pointer -> AG_ERR_ALIGN.  Stream-ordered, no scratch memory, no host
+ * synchronisation (the counts are zeroed by a memset on `stream`): capturable in a CUDA graph. */
+AG_API ag_status ag_cspace_components(const uint32_t *bits, int64_t n_grids, int32_t b1, int32_t b2, int32_t wrap,
+                                      int32_t *labels, int64_t *n_components, void *stream);
 
 /* K1: scenario/scene_0.py:88-103  Scene.step(action).  j1,j2,reward,flags are in/out (sticky
  * semantics).  actions: [n][2] float64 (actions_f32 == 0) or float32.  Optional outputs:
