@@ -231,12 +231,19 @@ ag_status launch(Kernel k, int64_t work, const CclDev &D, cudaStream_t s) {
 
 }  // namespace
 
-// ag_cspace_components after argument validation (ag_kernels.cu): n_grids >= 1, b1 * b2 < 2^31
-ag_status launch_cspace_components(const uint32_t *bits, int64_t n_grids, int32_t b1, int32_t b2, int32_t wrap,
-                                   int32_t *labels, int64_t *n_components, cudaStream_t s) {
+extern "C" ag_status ag_cspace_components(const uint32_t *bits, int64_t n_grids, int32_t b1, int32_t b2, int32_t wrap,
+                                          int32_t *labels, int64_t *n_components, void *stream) {
+    if (n_grids < 0 || b1 < 1 || b2 < 1) return AG_ERR_SHAPE;
+    const int64_t poses = (int64_t)b1 * b2;
+    if (poses > INT32_MAX || (n_grids > 0 && poses > INT64_MAX / n_grids)) return AG_ERR_SHAPE;   // grid-local int32 labels
+    if (wrap & ~3) return AG_ERR_MODE;
+    if (n_grids == 0) return AG_OK;
+    if (!bits || !labels) return AG_ERR_NULL;
+    if (((uintptr_t)bits % 4) || ((uintptr_t)labels % 4) || ((uintptr_t)n_components % 8)) return AG_ERR_ALIGN;
+    cudaStream_t s = (cudaStream_t)stream;
     CclDev D;
     D.bits = bits; D.labels = labels; D.n_components = reinterpret_cast<unsigned long long *>(n_components);
-    D.n_grids = n_grids; D.poses = (int64_t)b1 * b2;
+    D.n_grids = n_grids; D.poses = poses;
     D.b1 = b1; D.b2 = b2; D.W = (b2 + 31) / 32;
     D.tiles_r = (b1 + TH - 1) / TH; D.tiles_c = (b2 + TC - 1) / TC;
     D.nh = D.tiles_r - 1 + ((wrap & 1) && b1 > 1); D.nv = D.tiles_c - 1 + ((wrap & 2) && b2 > 1);   // a pose is never its own neighbour

@@ -1,5 +1,6 @@
-// ag_cmap.cu -- the configuration-space map (layout: ag_cmap.cuh): k_cspace_build, which makes it, and the library's
-// cache of maps, which hands one to each launch that reads it (cspace_map_for_launch).  DESIGN.md "K4, scene_0 class".
+// ag_cmap.cu -- the configuration-space map (layout: ag_cmap.cuh): k_cspace_build, which makes it, the library's cache of
+// maps, which hands one to each launch that reads it (cspace_map_for_launch), and ag_cspace_map, which builds one into a
+// caller's buffer.  DESIGN.md "K4, scene_0 class".
 #include <atomic>
 #include <cstring>
 #include <mutex>
@@ -256,20 +257,28 @@ ag_status cspace_map_for_launch(const ag_params &P, const GridDev &G, int32_t ma
     return AG_OK;
 }
 
-int64_t cspace_map_words(int32_t *b1, int32_t *b2) {
+extern "C" int64_t ag_cspace_map_words(int32_t *b1, int32_t *b2) {
     if (b1) *b1 = CB1;
     if (b2) *b2 = CB2;
     return CMAP_WORDS;
 }
 
-// the map alone, into a caller's buffer (ag_cspace_map): built in a scratch buffer with the header in front
-ag_status launch_cspace_map(const ag_params &P, const GridDev &G, uint32_t *map, cudaStream_t s) {
+// the map alone, into the caller's buffer: built in a scratch buffer with the header in front
+extern "C" ag_status ag_cspace_map(const ag_params *p, const ag_grid *g, uint32_t *map, void *stream) {
+    if (!p || !g || !map) return AG_ERR_NULL;
+    if (g->n_grids != 1 || g->S > 32) return AG_ERR_SHAPE;
+    if ((uintptr_t)map % 16) return AG_ERR_ALIGN;
+    GridDev G;
+    size_t smem;
+    ag_status st = make_grid_dev(p, g, 0, AG_ENGINE_FAST, &G, &smem);
+    if (st) return st;
+    cudaStream_t s = (cudaStream_t)stream;
     uint32_t *buf = nullptr;
     cudaError_t e = cudaMallocAsync(&buf, (size_t)(CMAP_HDR_WORDS + CMAP_WORDS) * 4, s);
     if (e != cudaSuccess) return (ag_status)e;
     e = cudaMemsetAsync(buf, 0, CMAP_HDR_WORDS * 4, s);
     if (e == cudaSuccess) {
-        k_cspace_build<<<CMAP_BUILD_BLOCKS, 256, 0, s>>>(P, G, buf, 0);
+        k_cspace_build<<<CMAP_BUILD_BLOCKS, 256, 0, s>>>(*p, G, buf, 0);
         e = (cudaError_t)launched();
     }
     if (e == cudaSuccess) e = cudaMemcpyAsync(map, buf + CMAP_HDR_WORDS, (size_t)CMAP_WORDS * 4, cudaMemcpyDeviceToDevice, s);

@@ -17,6 +17,7 @@
 //   general form (FAST on every other grid) -- pose_collides<FAST> per pose.  FAST's decision is not a per-link OR
 //     (the float32 filter and the float64 re-evaluation look at the arm as a whole), so it is not factored.
 #include <climits>
+#include <cmath>
 
 #include "ag_cmap.cuh"
 #include "ag_rollout.cuh"
@@ -142,10 +143,22 @@ ag_status launch(const ag_params &P, const GridDev &G, const CspaceDev &D0, size
 
 }  // namespace
 
-// ag_cspace_occupancy after argument validation (ag_kernels.cu): smem = the staged grid's bytes (make_grid_dev, env_id0 0)
-ag_status launch_cspace_occupancy(const ag_params &P, const GridDev &G0, int32_t max_occupied, double lo1, double step1,
-                                  int32_t b1, double lo2, double step2, int32_t b2, uint32_t *bits, int64_t *free_count,
-                                  int32_t engine, size_t smem, cudaStream_t s) {
+extern "C" ag_status ag_cspace_occupancy(const ag_params *p, const ag_grid *g, double lo1, double step1, int32_t b1,
+                                         double lo2, double step2, int32_t b2, uint32_t *bits, int64_t *free_count,
+                                         int32_t engine, void *stream) {
+    if (b1 < 1 || b2 < 1) return AG_ERR_SHAPE;
+    if (!p || !g) return AG_ERR_NULL;
+    GridDev G0;
+    size_t smem;
+    ag_status st = make_grid_dev(p, g, 0, engine, &G0, &smem);   // env_id0 0: K2's staging choice for a grid's own envs
+    if (st) return st;
+    if (!std::isfinite(lo1) || !std::isfinite(step1) || !std::isfinite(lo2) || !std::isfinite(step2)) return AG_ERR_SHAPE;
+    const int64_t row_words = ((int64_t)b2 + 31) / 32;
+    if ((int64_t)b1 * row_words > INT64_MAX / g->n_grids) return AG_ERR_SHAPE;   // n_grids * b1 * W words must fit int64
+    if (!bits) return AG_ERR_NULL;
+    if (((uintptr_t)bits % 4) || ((uintptr_t)free_count % 8)) return AG_ERR_ALIGN;
+    if (engine != AG_ENGINE_EXACT && engine != AG_ENGINE_FAST && engine != AG_ENGINE_BRUTE) return AG_ERR_MODE;
+    cudaStream_t s = (cudaStream_t)stream;
     CspaceDev D;
     D.lo1 = lo1; D.step1 = step1; D.lo2 = lo2; D.step2 = step2;
     D.b1 = b1; D.b2 = b2; D.W = (b2 + 31) / 32; D.spans = (D.W + UNIT_WORDS - 1) / UNIT_WORDS;
@@ -161,13 +174,13 @@ ag_status launch_cspace_occupancy(const ag_params &P, const GridDev &G0, int32_t
     switch (engine) {
         case AG_ENGINE_FAST: {
             CmapLaunch cm;
-            const ag_status st = cspace_map_for_launch(P, G0, max_occupied, smem, s, &cm);
+            st = cspace_map_for_launch(*p, G0, g->max_occupied, smem, s, &cm);
             if (st != AG_OK) return st;
             D.cmap = cm.map; D.cmap_off = cm.off;
-            return cm.map ? launch<AG_ENGINE_FAST, true>(P, G, D, cm.smem, s) : launch<AG_ENGINE_FAST, false>(P, G, D, smem, s);
+            return cm.map ? launch<AG_ENGINE_FAST, true>(*p, G, D, cm.smem, s) : launch<AG_ENGINE_FAST, false>(*p, G, D, smem, s);
         }
-        case AG_ENGINE_EXACT: return launch<AG_ENGINE_EXACT, false>(P, G, D, smem, s);
-        case AG_ENGINE_BRUTE: return launch<AG_ENGINE_BRUTE, false>(P, G, D, smem, s);
+        case AG_ENGINE_EXACT: return launch<AG_ENGINE_EXACT, false>(*p, G, D, smem, s);
+        case AG_ENGINE_BRUTE: return launch<AG_ENGINE_BRUTE, false>(*p, G, D, smem, s);
         default: return AG_ERR_MODE;
     }
 }

@@ -5,10 +5,7 @@
 #include <cstring>
 #include <new>
 
-#include "../../include/abstract_gym_b200.h"
-
-ag_status ag_rollout_impl(const ag_params *p, const ag_grid *g, const ag_rollout_args *a, int64_t row_stride,
-                          void *stream);
+#include "ag_rollout.cuh"
 
 extern "C" {
 

@@ -2,29 +2,11 @@
 // Build: nvcc -gencode arch=compute_100a,code=sm_100a -lineinfo -O3 (abstract_gym_b200/build.py).
 #include <atomic>
 #include <climits>
-#include <cmath>
 #include <cstring>
 
 #include "ag_rollout.cuh"
 
 using namespace agd;
-
-// ag_rollout_lut.cu: the persistent kernel for scene_0-class grids (obstacle list, one grid, cartesian target)
-bool rollout_lut_applies(const ag_params &P, const GridDev &G, const RolloutDev &A);
-ag_status launch_rollout_lut(const ag_params &P, const GridDev &G, const RolloutDev &A, size_t smem, cudaStream_t s);
-int64_t cspace_map_words(int32_t *b1, int32_t *b2);
-ag_status launch_cspace_map(const ag_params &P, const GridDev &G, uint32_t *map, cudaStream_t s);
-// ag_motion.cu: batched motion checking (ag_check_motion after argument validation)
-ag_status launch_check_motion(const ag_params &P, const GridDev &G, int32_t max_occupied, const double *j1, const double *j2,
-                              const double *goal, const int32_t *steps, int32_t *first_collision, int32_t *first_hit,
-                              double *last_free, int64_t m, int64_t env_id0, int32_t engine, size_t smem, cudaStream_t s);
-// ag_cspace.cu: configuration-space occupancy (ag_cspace_occupancy after argument validation)
-ag_status launch_cspace_occupancy(const ag_params &P, const GridDev &G, int32_t max_occupied, double lo1, double step1,
-                                  int32_t b1, double lo2, double step2, int32_t b2, uint32_t *bits, int64_t *free_count,
-                                  int32_t engine, size_t smem, cudaStream_t s);
-// ag_ccl.cu: free-space components of an occupancy image (ag_cspace_components after argument validation)
-ag_status launch_cspace_components(const uint32_t *bits, int64_t n_grids, int32_t b1, int32_t b2, int32_t wrap,
-                                   int32_t *labels, int64_t *n_components, cudaStream_t s);
 
 namespace {
 
@@ -696,44 +678,6 @@ k_rollout_async(const __grid_constant__ ag_params P, const __grid_constant__ Gri
 }
 
 // ------------------------------------------------------------------------------------- host side
-// the largest grid footprint (bits, transposed bits, two-level form, cell tables) a block copies to shared memory
-constexpr size_t STAGE_MAX_BYTES = 32768;
-
-ag_status make_grid_dev(const ag_params *p, const ag_grid *g, int64_t env_id0, int engine, GridDev *out,
-                        size_t *smem_bytes) {
-    if (!g || !g->bits || !g->min_x || !g->min_y) return AG_ERR_NULL;
-    if (g->S < 2 || g->words_per_row != (g->S + 31) / 32 || g->n_grids < 1 || g->envs_per_grid < 1 ||
-        g->grid_stride_words < (int64_t)g->S * g->words_per_row)
-        return AG_ERR_SHAPE;
-    // the FAST engine's error budget (ag_fast.cuh) assumes scene_0-class magnitudes
-    if (engine == AG_ENGINE_FAST && p &&
-        !(p->link_1 > 0 && p->link_2 > 0 && p->link_1 <= 1.0 && p->link_2 <= 1.0 && g->env_size <= 4.0))
-        return AG_ERR_MODE;
-    GridDev d;
-    d.bits = g->bits; d.bits_t = g->bits_t; d.min_x = g->min_x; d.min_y = g->min_y;
-    d.T = (g->S + 7) / 8; d.cwpr = (d.T + 31) / 32;
-    d.hier = d.T <= AG_HIER_MAX_T ? reinterpret_cast<const unsigned char *>(g->hier) : nullptr;   // larger maps: the row walk
-    d.hier_tiles_bytes = (int32_t)((((int64_t)d.T * d.T + 1) & ~(int64_t)1) * 8);
-    d.hier_coarse_words = (int32_t)(((int64_t)d.T * d.cwpr + 3) & ~(int64_t)3);
-    d.hier_bytes = (int32_t)ag_grid_hier_bytes(g->S);
-    d.side = g->side; d.half = g->env_size / 2.0; d.inv_side = 1.0 / g->side;
-    d.margin = 1e-9 * g->env_size;
-    d.S = g->S; d.wpr = g->words_per_row; d.n_grids = g->n_grids;
-    d.stride_words = g->grid_stride_words; d.envs_per_grid = g->envs_per_grid;
-    const int spad = (g->S + 1) & ~1;
-    const size_t bytes = 16 + (size_t)g->grid_stride_words * 4 * (g->bits_t ? 2 : 1) + (d.hier ? (size_t)d.hier_bytes : 0) +
-                         (size_t)spad * 16;
-    const bool uniform = g->n_grids == 1 || (g->envs_per_grid % AG_BLOCK == 0 && env_id0 % AG_BLOCK == 0);
-    const bool aligned = ((uintptr_t)g->bits % 16 == 0) && ((uintptr_t)g->bits_t % 16 == 0) && ((uintptr_t)g->hier % 16 == 0) &&
-                         (g->grid_stride_words % 4 == 0);
-    d.stage = (uniform && aligned && bytes <= STAGE_MAX_BYTES) ? 1 : 0;
-    *smem_bytes = d.stage ? bytes : 0;
-    *out = d;
-    return AG_OK;
-}
-
-inline unsigned blocks_for(int64_t n) { return (unsigned)((n + AG_BLOCK - 1) / AG_BLOCK); }
-
 #define AG_DISPATCH_ENGINE(engine, ...)                                   \
     switch (engine) {                                                     \
         case AG_ENGINE_EXACT: { constexpr int E = AG_ENGINE_EXACT; __VA_ARGS__; break; } \
@@ -801,7 +745,42 @@ ag_status launch_rollout_e(const ag_params &P, const GridDev &G, const RolloutDe
 
 void ag_note_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
 
-// internal (also used by ag_host.cu): rollout with explicit action/record row stride
+// the largest grid footprint (bits, transposed bits, two-level form, cell tables) a block copies to shared memory
+constexpr size_t STAGE_MAX_BYTES = 32768;
+
+ag_status make_grid_dev(const ag_params *p, const ag_grid *g, int64_t env_id0, int engine, GridDev *out,
+                        size_t *smem_bytes) {
+    if (!g || !g->bits || !g->min_x || !g->min_y) return AG_ERR_NULL;
+    if (g->S < 2 || g->words_per_row != (g->S + 31) / 32 || g->n_grids < 1 || g->envs_per_grid < 1 ||
+        g->grid_stride_words < (int64_t)g->S * g->words_per_row)
+        return AG_ERR_SHAPE;
+    // the FAST engine's error budget (ag_fast.cuh) assumes scene_0-class magnitudes
+    if (engine == AG_ENGINE_FAST && p &&
+        !(p->link_1 > 0 && p->link_2 > 0 && p->link_1 <= 1.0 && p->link_2 <= 1.0 && g->env_size <= 4.0))
+        return AG_ERR_MODE;
+    GridDev d;
+    d.bits = g->bits; d.bits_t = g->bits_t; d.min_x = g->min_x; d.min_y = g->min_y;
+    d.T = (g->S + 7) / 8; d.cwpr = (d.T + 31) / 32;
+    d.hier = d.T <= AG_HIER_MAX_T ? reinterpret_cast<const unsigned char *>(g->hier) : nullptr;   // larger maps: the row walk
+    d.hier_tiles_bytes = (int32_t)((((int64_t)d.T * d.T + 1) & ~(int64_t)1) * 8);
+    d.hier_coarse_words = (int32_t)(((int64_t)d.T * d.cwpr + 3) & ~(int64_t)3);
+    d.hier_bytes = (int32_t)ag_grid_hier_bytes(g->S);
+    d.side = g->side; d.half = g->env_size / 2.0; d.inv_side = 1.0 / g->side;
+    d.margin = 1e-9 * g->env_size;
+    d.S = g->S; d.wpr = g->words_per_row; d.n_grids = g->n_grids;
+    d.stride_words = g->grid_stride_words; d.envs_per_grid = g->envs_per_grid;
+    const int spad = (g->S + 1) & ~1;
+    const size_t bytes = 16 + (size_t)g->grid_stride_words * 4 * (g->bits_t ? 2 : 1) + (d.hier ? (size_t)d.hier_bytes : 0) +
+                         (size_t)spad * 16;
+    const bool uniform = g->n_grids == 1 || (g->envs_per_grid % AG_BLOCK == 0 && env_id0 % AG_BLOCK == 0);
+    const bool aligned = ((uintptr_t)g->bits % 16 == 0) && ((uintptr_t)g->bits_t % 16 == 0) && ((uintptr_t)g->hier % 16 == 0) &&
+                         (g->grid_stride_words % 4 == 0);
+    d.stage = (uniform && aligned && bytes <= STAGE_MAX_BYTES) ? 1 : 0;
+    *smem_bytes = d.stage ? bytes : 0;
+    *out = d;
+    return AG_OK;
+}
+
 ag_status ag_rollout_impl(const ag_params *p, const ag_grid *g, const ag_rollout_args *a, int64_t row_stride,
                           void *stream) {
     if (!p || !g || !a) return AG_ERR_NULL;
@@ -944,52 +923,6 @@ ag_status ag_collision_check(const ag_params *p, const ag_grid *g, const double 
     return launched();
 }
 
-ag_status ag_check_motion(const ag_params *p, const ag_grid *g, const double *j1, const double *j2, const double *goal,
-                          const int32_t *steps, int32_t *first_collision, int32_t *first_hit, double *last_free, int64_t m,
-                          int64_t env_id0, int32_t engine, void *stream) {
-    if (m < 0) return AG_ERR_SHAPE;
-    if (!p || !g) return AG_ERR_NULL;
-    GridDev G;
-    size_t smem;
-    ag_status st = make_grid_dev(p, g, env_id0, engine, &G, &smem);
-    if (st) return st;
-    if (m == 0) return AG_OK;
-    if (!j1 || !j2 || !goal || !steps || !first_collision) return AG_ERR_NULL;
-    if (((uintptr_t)goal % 16) || ((uintptr_t)last_free % 16)) return AG_ERR_ALIGN;
-    return launch_check_motion(*p, G, g->max_occupied, j1, j2, goal, steps, first_collision, first_hit, last_free, m, env_id0,
-                               engine, smem, (cudaStream_t)stream);
-}
-
-ag_status ag_cspace_occupancy(const ag_params *p, const ag_grid *g, double lo1, double step1, int32_t b1, double lo2,
-                              double step2, int32_t b2, uint32_t *bits, int64_t *free_count, int32_t engine, void *stream) {
-    if (b1 < 1 || b2 < 1) return AG_ERR_SHAPE;
-    if (!p || !g) return AG_ERR_NULL;
-    GridDev G;
-    size_t smem;
-    ag_status st = make_grid_dev(p, g, 0, engine, &G, &smem);   // env_id0 0: K2's staging choice for a grid's own envs
-    if (st) return st;
-    if (!std::isfinite(lo1) || !std::isfinite(step1) || !std::isfinite(lo2) || !std::isfinite(step2)) return AG_ERR_SHAPE;
-    const int64_t row_words = ((int64_t)b2 + 31) / 32;
-    if ((int64_t)b1 * row_words > INT64_MAX / g->n_grids) return AG_ERR_SHAPE;   // n_grids * b1 * W words must fit int64
-    if (!bits) return AG_ERR_NULL;
-    if (((uintptr_t)bits % 4) || ((uintptr_t)free_count % 8)) return AG_ERR_ALIGN;
-    if (engine != AG_ENGINE_EXACT && engine != AG_ENGINE_FAST && engine != AG_ENGINE_BRUTE) return AG_ERR_MODE;
-    return launch_cspace_occupancy(*p, G, g->max_occupied, lo1, step1, b1, lo2, step2, b2, bits, free_count, engine, smem,
-                                   (cudaStream_t)stream);
-}
-
-ag_status ag_cspace_components(const uint32_t *bits, int64_t n_grids, int32_t b1, int32_t b2, int32_t wrap, int32_t *labels,
-                               int64_t *n_components, void *stream) {
-    if (n_grids < 0 || b1 < 1 || b2 < 1) return AG_ERR_SHAPE;
-    const int64_t poses = (int64_t)b1 * b2;
-    if (poses > INT32_MAX || (n_grids > 0 && poses > INT64_MAX / n_grids)) return AG_ERR_SHAPE;   // grid-local int32 labels
-    if (wrap & ~3) return AG_ERR_MODE;
-    if (n_grids == 0) return AG_OK;
-    if (!bits || !labels) return AG_ERR_NULL;
-    if (((uintptr_t)bits % 4) || ((uintptr_t)labels % 4) || ((uintptr_t)n_components % 8)) return AG_ERR_ALIGN;
-    return launch_cspace_components(bits, n_grids, b1, b2, wrap, labels, n_components, (cudaStream_t)stream);
-}
-
 ag_status ag_step(const ag_params *p, const ag_grid *g, double *j1, double *j2, const void *actions,
                   int32_t actions_f32, float *reward, uint8_t *flags, double *ee, double *dist, int32_t *first_hit,
                   int64_t *stats, const double *targets, int64_t n, int64_t env_id0, int32_t engine, void *stream) {
@@ -1062,19 +995,6 @@ ag_status ag_step_obs(const ag_params *p, const ag_grid *g, double *j1, double *
     AG_DISPATCH_ENGINE(engine, { if (actions_f32) AG_SO(true) else AG_SO(false) });
 #undef AG_SO
     return launched();
-}
-
-int64_t ag_cspace_map_words(int32_t *b1, int32_t *b2) { return cspace_map_words(b1, b2); }
-
-ag_status ag_cspace_map(const ag_params *p, const ag_grid *g, uint32_t *map, void *stream) {
-    if (!p || !g || !map) return AG_ERR_NULL;
-    if (g->n_grids != 1 || g->S > 32) return AG_ERR_SHAPE;
-    if ((uintptr_t)map % 16) return AG_ERR_ALIGN;
-    GridDev G;
-    size_t smem;
-    ag_status st = make_grid_dev(p, g, 0, AG_ENGINE_FAST, &G, &smem);
-    if (st) return st;
-    return launch_cspace_map(*p, G, map, (cudaStream_t)stream);
 }
 
 ag_status ag_rollout(const ag_params *p, const ag_grid *g, const ag_rollout_args *a, void *stream) {

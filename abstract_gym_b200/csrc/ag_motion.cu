@@ -87,23 +87,32 @@ ag_status launch(const ag_params &P, const GridDev &G, const MotionDev &M, size_
     auto k = k_check_motion<ENGINE, MAP>;
     ag_status st = set_smem(k, smem);
     if (st != AG_OK) return st;
-    int64_t blocks = (M.m + AG_BLOCK - 1) / AG_BLOCK;
+    unsigned blocks = blocks_for(M.m);
     if (MAP) {                                                                   // persistent: as many blocks as fit at once
         int slots = 0;
         st = resident_blocks(k, AG_BLOCK, smem, &slots);
         if (st != AG_OK) return st;
-        blocks = blocks < slots ? blocks : slots;
+        blocks = blocks < (unsigned)slots ? blocks : (unsigned)slots;
     }
-    k<<<(unsigned)blocks, AG_BLOCK, smem, s>>>(P, G, make_fast_const(P, G), M);
+    k<<<blocks, AG_BLOCK, smem, s>>>(P, G, make_fast_const(P, G), M);
     return launched();
 }
 
 }  // namespace
 
-// ag_check_motion after argument validation (ag_kernels.cu): smem = the staged grid's bytes (make_grid_dev)
-ag_status launch_check_motion(const ag_params &P, const GridDev &G, int32_t max_occupied, const double *j1, const double *j2,
-                              const double *goal, const int32_t *steps, int32_t *first_collision, int32_t *first_hit,
-                              double *last_free, int64_t m, int64_t env_id0, int32_t engine, size_t smem, cudaStream_t s) {
+extern "C" ag_status ag_check_motion(const ag_params *p, const ag_grid *g, const double *j1, const double *j2,
+                                     const double *goal, const int32_t *steps, int32_t *first_collision, int32_t *first_hit,
+                                     double *last_free, int64_t m, int64_t env_id0, int32_t engine, void *stream) {
+    if (m < 0) return AG_ERR_SHAPE;
+    if (!p || !g) return AG_ERR_NULL;
+    GridDev G;
+    size_t smem;
+    ag_status st = make_grid_dev(p, g, env_id0, engine, &G, &smem);
+    if (st) return st;
+    if (m == 0) return AG_OK;
+    if (!j1 || !j2 || !goal || !steps || !first_collision) return AG_ERR_NULL;
+    if (((uintptr_t)goal % 16) || ((uintptr_t)last_free % 16)) return AG_ERR_ALIGN;
+    cudaStream_t s = (cudaStream_t)stream;
     MotionDev M;
     M.j1 = j1; M.j2 = j2; M.goal = goal; M.steps = steps;
     M.first_collision = first_collision; M.first_hit = first_hit; M.last_free = last_free;
@@ -111,13 +120,13 @@ ag_status launch_check_motion(const ag_params &P, const GridDev &G, int32_t max_
     switch (engine) {
         case AG_ENGINE_FAST: {
             CmapLaunch cm;
-            const ag_status st = cspace_map_for_launch(P, G, max_occupied, smem, s, &cm);
+            st = cspace_map_for_launch(*p, G, g->max_occupied, smem, s, &cm);
             if (st != AG_OK) return st;
             M.cmap = cm.map; M.cmap_off = cm.off;
-            return cm.map ? launch<AG_ENGINE_FAST, true>(P, G, M, cm.smem, s) : launch<AG_ENGINE_FAST, false>(P, G, M, smem, s);
+            return cm.map ? launch<AG_ENGINE_FAST, true>(*p, G, M, cm.smem, s) : launch<AG_ENGINE_FAST, false>(*p, G, M, smem, s);
         }
-        case AG_ENGINE_EXACT: return launch<AG_ENGINE_EXACT, false>(P, G, M, smem, s);
-        case AG_ENGINE_BRUTE: return launch<AG_ENGINE_BRUTE, false>(P, G, M, smem, s);
+        case AG_ENGINE_EXACT: return launch<AG_ENGINE_EXACT, false>(*p, G, M, smem, s);
+        case AG_ENGINE_BRUTE: return launch<AG_ENGINE_BRUTE, false>(*p, G, M, smem, s);
         default: return AG_ERR_MODE;
     }
 }

@@ -1,6 +1,15 @@
-// ag_rollout.cuh -- pieces shared by the rollout kernels (ag_kernels.cu: K1..K5 and the general K4;
-// ag_rollout_lut.cu: the persistent scene_0-class K4), motion checking (ag_motion.cu) and occupancy (ag_cspace.cu),
-// and the launch helpers every launcher uses (ag_cmap.cu too).
+// ag_rollout.cuh -- pieces shared by the kernels of the library, the launch helpers every launcher uses, and the host
+// functions one file calls in another: the grid prologue of every grid-taking entry point (make_grid_dev), the launch
+// counter, the rollout with a row stride (ag_rollout_impl) and its dispatch to the persistent kernel.
+//
+// Each extern "C" entry point is defined next to its kernels:
+//   ag_kernels.cu      K1..K6 and the general K4 (ag_collision_check, ag_step, ag_reset, ag_step_obs, ag_rollout, ...)
+//   ag_rollout_lut.cu  the persistent scene_0-class K4, which ag_rollout dispatches to (launch_rollout_lut)
+//   ag_motion.cu       ag_check_motion
+//   ag_cspace.cu       ag_cspace_occupancy
+//   ag_ccl.cu          ag_cspace_components
+//   ag_cmap.cu         ag_cspace_map, ag_cspace_map_words (and the map cache its readers share, ag_cmap.cuh)
+//   ag_host.cu         the host-only entry points and the pipelined host-buffer executor (ag_rollout_host)
 #pragma once
 #include <climits>
 
@@ -8,6 +17,9 @@
 #include "ag_fast.cuh"
 
 void ag_note_launch();   // ag_kernels.cu: counts kernel launches (ag_launch_count)
+// ag_kernels.cu: ag_rollout with an explicit action / record row stride (ag_host.cu runs it on chunks of a batch)
+ag_status ag_rollout_impl(const ag_params *p, const ag_grid *g, const ag_rollout_args *a, int64_t row_stride,
+                          void *stream);
 
 namespace agd {
 
@@ -47,6 +59,9 @@ ag_status resident_blocks(Kernel kernel, int block, size_t smem, int *blocks) {
     *blocks = sms * occ;
     return (ag_status)e;
 }
+
+// the grid of a launch with one thread per item
+inline unsigned blocks_for(int64_t n) { return (unsigned)((n + AG_BLOCK - 1) / AG_BLOCK); }
 
 struct RolloutDev {
     int64_t n, env_id0, row_stride;
@@ -277,3 +292,13 @@ template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
 }  // namespace agd
+
+// make_grid_dev (ag_kernels.cu): the grid prologue of every entry point that takes an ag_grid.  Checks the grid
+// (NULL pointers -> AG_ERR_NULL, inconsistent shape or stride -> AG_ERR_SHAPE; the FAST engine outside its error
+// budget -> AG_ERR_MODE, other engine values are the caller's to check) and fills *out; *smem_bytes = the dynamic shared
+// memory of a block that stages its grid (0: the grid is read from global memory).  Touches no device.
+ag_status make_grid_dev(const ag_params *p, const ag_grid *g, int64_t env_id0, int engine, agd::GridDev *out,
+                        size_t *smem_bytes);
+// ag_rollout_lut.cu: the persistent kernel for scene_0-class grids (obstacle list, one grid, cartesian target)
+bool rollout_lut_applies(const ag_params &P, const agd::GridDev &G, const agd::RolloutDev &A);
+ag_status launch_rollout_lut(const ag_params &P, const agd::GridDev &G, const agd::RolloutDev &A, size_t smem, cudaStream_t s);
