@@ -306,11 +306,14 @@ __global__ void __launch_bounds__(AG_BLOCK) k_step_obs(const ag_params P, const 
         j1[e] = q1; j2[e] = q2; reward[e] = rw; flags[e] = (uint8_t)fl; ep_len[e] = el;
         write_obs(obs + e * AG_OBS_DIM, q1, q2, A, tx, ty);
         if (crop) {                                                              // local occupancy around the end effector
-            const int r0 = row_of(G, A.gy), c0 = col_of(G, A.gx), hc = crop_size / 2;
+            // the end effector's own cell, not clamped to [-1, S] as row_of / col_of do for the traversal: an arm
+            // that reaches past the grid sees only cells outside it
+            const int64_t r0 = (int64_t)(floor((G.half - A.gy) * G.inv_side) + 1.0), c0 = (int64_t)floor((A.gx + G.half) * G.inv_side);
+            const int hc = crop_size / 2;
             uint8_t *o = crop + e * (int64_t)crop_size * crop_size;
             for (int dr = 0; dr < crop_size; ++dr)
                 for (int dc = 0; dc < crop_size; ++dc) {
-                    const int r = r0 - hc + dr, c = c0 - hc + dc;
+                    const int64_t r = r0 - hc + dr, c = c0 - hc + dc;
                     uint8_t v = 2;
                     if (r >= 0 && r < G.S && c >= 0 && c < G.S) v = (B.V.bits[r * G.wpr + (c >> 5)] >> (c & 31)) & 1u;
                     o[dr * crop_size + dc] = v;

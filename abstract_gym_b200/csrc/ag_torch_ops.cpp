@@ -266,6 +266,14 @@ void step_obs(const Tensor &params, const Tensor &bits, const OptTensor &bits_t,
                 (actions.scalar_type() == at::kFloat || actions.scalar_type() == at::kDouble),
                 "actions must be a contiguous CUDA [N,2] float32 or float64 tensor");
     TORCH_CHECK(obs.numel() == n * AG_OBS_DIM, "obs must be [N,", AG_OBS_DIM, "]");
+    for (const auto &[t, name] : {std::pair<const Tensor *, const char *>{&j2, "j2"}, {&reward, "reward"}, {&flags, "flags"},
+                                  {&reset_ctr, "reset_ctr"}, {&ep_len, "ep_len"}, {&reward_out, "reward_out"},
+                                  {&terminated, "terminated"}, {&collision, "collision"}})
+        TORCH_CHECK(t->numel() == n, name, " must have one element per env (", n, "), got ", t->numel());
+    TORCH_CHECK(stats.numel() == AG_ST_COUNT, "stats must be int64[", AG_ST_COUNT, "], got ", stats.numel(), " elements");
+    if (targets.has_value() && targets->defined()) TORCH_CHECK(targets->numel() == 2 * n, "targets must be [N,2]");
+    if (final_obs.has_value() && final_obs->defined())
+        TORCH_CHECK(final_obs->numel() == n * AG_OBS_DIM, "final_obs must be [N,", AG_OBS_DIM, "]");
     int32_t crop_size = 0;
     if (crop.has_value() && crop->defined()) {
         TORCH_CHECK(crop->dim() == 3 && crop->size(0) == n && crop->size(1) == crop->size(2), "crop must be [N,c,c]");
