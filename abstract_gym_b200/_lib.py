@@ -11,7 +11,7 @@ from . import build as _build
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 
-ABI_VERSION = 8
+ABI_VERSION = 9
 ENGINE_EXACT, ENGINE_FAST, ENGINE_BRUTE = 0, 1, 2
 ENGINES = {"exact": ENGINE_EXACT, "fast": ENGINE_FAST, "brute": ENGINE_BRUTE}
 FLAG_COLLISION, FLAG_DONE = 1, 2
@@ -80,6 +80,8 @@ SYMBOLS = {
     "ag_check_motion": (_i32, [C.POINTER(Params), C.POINTER(Grid), _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i32, _vp]),
     "ag_cspace_occupancy": (_i32, [C.POINTER(Params), C.POINTER(Grid), _dbl, _dbl, _i32, _dbl, _dbl, _i32, _vp, _vp, _i32, _vp]),
     "ag_cspace_components": (_i32, [_vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp]),
+    "ag_cspace_distance": (_i32, [_vp, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp]),
+    "ag_cspace_descend": (_i32, [_vp, _i64, _i32, _i32, _i32, _vp, _vp, _i64, _i32, _vp, _vp, _vp]),
     "ag_step":(_i32, [C.POINTER(Params), C.POINTER(Grid), _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                        _i64, _i64, _i32, _vp]),
     "ag_reset": (_i32, [C.POINTER(Params), C.POINTER(Grid), _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _u64, _i32,

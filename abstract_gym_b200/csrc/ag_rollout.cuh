@@ -8,6 +8,7 @@
 //   ag_motion.cu       ag_check_motion
 //   ag_cspace.cu       ag_cspace_occupancy
 //   ag_ccl.cu          ag_cspace_components
+//   ag_cdist.cu        ag_cspace_distance, ag_cspace_descend
 //   ag_cmap.cu         ag_cspace_map, ag_cspace_map_words (and the map cache its readers share, ag_cmap.cuh)
 //   ag_host.cu         the host-only entry points and the pipelined host-buffer executor (ag_rollout_host)
 #pragma once

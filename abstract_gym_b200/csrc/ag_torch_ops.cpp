@@ -5,7 +5,8 @@
 // point of include/abstract_gym_b200.h in libabstract_gym_b200.so.  There is no CPU dispatch key: the ops are
 // registered for CUDA only, so CPU tensors raise NotImplementedError.  State tensors are mutated in place
 // (declared in the schemas), nothing is allocated and nothing synchronises, so the ops can sit inside CUDA-graph
-// captures next to a policy network.
+// captures next to a policy network -- except cspace_distance, which synchronises with its stream to detect convergence
+// (ag_cspace_distance) and fails inside a capture.
 //
 // Scene constants travel as a float64[13] CPU tensor (ag_params order, see pack_params in ops.py) that is read in
 // place; the grid as its device tensors plus six scalars.  The reference methods each op replaces are cited in the
@@ -158,6 +159,52 @@ void cspace_components(const Tensor &occupancy, int64_t b1, int64_t b2, int64_t 
                  "ag_cspace_components");
 }
 
+// steps from every free pose of cspace_occupancy's words to a goal image in the same layout, per grid -> ag_cspace_distance
+void cspace_distance(const Tensor &occupancy, const Tensor &goals, int64_t b1, int64_t b2, int64_t wrap, Tensor dist,
+                     OptTensor max_dist) {
+    const c10::Device dev = dist.device();
+    c10::cuda::CUDAGuard guard(dev);
+    need(occupancy, at::kInt, "occupancy", dev);
+    need(goals, at::kInt, "goals", dev);
+    need(dist, at::kInt, "dist", dev);
+    TORCH_CHECK(b1 >= 1 && b2 >= 1 && b1 <= INT32_MAX && b2 <= INT32_MAX && b1 * b2 < INT32_MAX,
+                "b1 and b2 must be >= 1 with b1 * b2 < 2^31 - 1");
+    const int64_t grid_words = b1 * ((b2 + 31) / 32);
+    TORCH_CHECK(occupancy.numel() % grid_words == 0, "occupancy must be [n_grids, b1, ceil(b2/32)] int32 words");
+    const int64_t n_grids = occupancy.numel() / grid_words;
+    TORCH_CHECK(goals.numel() == occupancy.numel(), "goals must have the layout of occupancy");
+    TORCH_CHECK(dist.numel() == n_grids * b1 * b2, "dist must be [n_grids, b1, b2] int32");
+    if (max_dist.has_value() && max_dist->defined()) TORCH_CHECK(max_dist->numel() == n_grids, "max_dist must be [n_grids]");
+    check_status(ag_cspace_distance(reinterpret_cast<const uint32_t *>(occupancy.data_ptr()),
+                                    reinterpret_cast<const uint32_t *>(goals.data_ptr()), n_grids, (int32_t)b1, (int32_t)b2,
+                                    (int32_t)wrap, dist.data_ptr<int32_t>(),
+                                    opt_ptr<int32_t>(max_dist, at::kInt, "max_dist", dev), stream_of(dev)),
+                 "ag_cspace_distance");
+}
+
+// lattice paths down a cspace_distance field -> ag_cspace_descend
+void cspace_descend(const Tensor &dist, int64_t b1, int64_t b2, int64_t wrap, const Tensor &start, const Tensor &grid,
+                    int64_t max_len, Tensor path, Tensor length) {
+    const c10::Device dev = path.device();
+    c10::cuda::CUDAGuard guard(dev);
+    need(dist, at::kInt, "dist", dev);
+    need(start, at::kInt, "start", dev);
+    need(grid, at::kLong, "grid", dev);
+    need(path, at::kInt, "path", dev);
+    need(length, at::kInt, "length", dev);
+    TORCH_CHECK(b1 >= 1 && b2 >= 1 && b1 <= INT32_MAX && b2 <= INT32_MAX && b1 * b2 < INT32_MAX,
+                "b1 and b2 must be >= 1 with b1 * b2 < 2^31 - 1");
+    TORCH_CHECK(dist.numel() % (b1 * b2) == 0, "dist must be [n_grids, b1, b2] int32");
+    TORCH_CHECK(max_len >= 1 && max_len <= INT32_MAX, "max_len must be in [1, 2^31)");
+    const int64_t m = start.numel();
+    TORCH_CHECK(grid.numel() == m && length.numel() == m, "start, grid, length must have one element per query");
+    TORCH_CHECK(path.numel() == m * max_len, "path must be [M, max_len] int32");
+    check_status(ag_cspace_descend(dist.data_ptr<int32_t>(), dist.numel() / (b1 * b2), (int32_t)b1, (int32_t)b2,
+                                   (int32_t)wrap, start.data_ptr<int32_t>(), grid.data_ptr<int64_t>(), m, (int32_t)max_len,
+                                   path.data_ptr<int32_t>(), length.data_ptr<int32_t>(), stream_of(dev)),
+                 "ag_cspace_descend");
+}
+
 // Scene.step (scenario/scene_0.py:88-103) -> ag_step
 void step(const Tensor &params, const Tensor &bits, const OptTensor &bits_t, const OptTensor &hier, const Tensor &min_x, const Tensor &min_y, double side,
           double env_size, int64_t S, int64_t n_grids, int64_t max_occupied, int64_t envs_per_grid, Tensor j1, Tensor j2,
@@ -304,6 +351,9 @@ TORCH_LIBRARY(abstract_gym_b200, m) {
     m.def("cspace_occupancy(" AG_GRID_SCHEMA "float lo1, float step1, int b1, float lo2, float step2, int b2, "
           "Tensor(a!) occupancy, Tensor(b!)? free_count, int engine) -> ()");
     m.def("cspace_components(Tensor occupancy, int b1, int b2, int wrap, Tensor(a!) labels, Tensor(b!)? n_components) -> ()");
+    m.def("cspace_distance(Tensor occupancy, Tensor goals, int b1, int b2, int wrap, Tensor(a!) dist, Tensor(b!)? max_dist) -> ()");
+    m.def("cspace_descend(Tensor dist, int b1, int b2, int wrap, Tensor start, Tensor grid, int max_len, Tensor(a!) path, "
+          "Tensor(b!) length) -> ()");
     m.def("step(" AG_GRID_SCHEMA "Tensor(a!) j1, Tensor(b!) j2, Tensor actions, Tensor(c!) reward, Tensor(d!) flags, Tensor(e!)? ee, "
           "Tensor(f!)? dist, Tensor(g!)? first_hit, Tensor(h!)? stats, Tensor? targets, int env_id0, int engine) -> ()");
     m.def("reset(" AG_GRID_SCHEMA "Tensor(a!) j1, Tensor(b!) j2, Tensor(c!) reward, Tensor(d!) flags, Tensor(e!) reset_ctr, Tensor? mask, "
@@ -323,6 +373,8 @@ TORCH_LIBRARY_IMPL(abstract_gym_b200, CUDA, m) {
     m.impl("check_motion", &check_motion);
     m.impl("cspace_occupancy", &cspace_occupancy);
     m.impl("cspace_components", &cspace_components);
+    m.impl("cspace_distance", &cspace_distance);
+    m.impl("cspace_descend", &cspace_descend);
     m.impl("step", &step);
     m.impl("reset", &reset);
     m.impl("rollout", &rollout);

@@ -1,14 +1,17 @@
 """torch custom ops over the C ABI: `torch.ops.abstract_gym_b200.{collision_check, check_motion, cspace_occupancy,
-cspace_components, step, reset, rollout, step_obs}`.
+cspace_components, cspace_distance, cspace_descend, step, reset, rollout, step_obs}`.
 
 The ops live in a COMPILED library, libabstract_gym_b200_ops.so (csrc/ag_torch_ops.cpp: TORCH_LIBRARY schemas, CUDA-only
 registration), which validates device / dtype / contiguity / shapes, takes the current CUDA stream and calls the
 `extern "C"` symbols of include/abstract_gym_b200.h.  This module loads that library and offers the two packing helpers
 the schemas need.  There is no CPU dispatch: a CPU tensor raises NotImplementedError.  The ops mutate their state
 tensors in place (declared in the schemas) and return nothing, so they can sit inside captured graphs next to a policy
-network.
+network.  The one exception is cspace_distance: it synchronises with its stream to detect convergence, so it cannot be
+captured (inside a capture it raises and the capture stays intact).
 
-Every op starts with the same eleven scene / grid arguments:
+The image ops take no scene: cspace_components(occupancy, b1, b2, wrap, labels, n_components?),
+cspace_distance(occupancy, goals, b1, b2, wrap, dist, max_dist?) and cspace_descend(dist, b1, b2, wrap, start, grid,
+max_len, path, length) (include/abstract_gym_b200.h).  Every other op starts with the same eleven scene / grid arguments:
     params        float64[13] CPU tensor  = pack_params(scene.params())      (ag_params)
     grid_bits     int32 [n_grids * stride] CUDA, grid_bits_t (optional transposed planes), grid_hier (optional two-level form, uint8), min_x, min_y float64 [>= S]
     side, env_size, S, n_grids, max_occupied, envs_per_grid                   = grid_args(device_grid)
@@ -56,6 +59,8 @@ collision_check = torch.ops.abstract_gym_b200.collision_check
 check_motion = torch.ops.abstract_gym_b200.check_motion
 cspace_occupancy = torch.ops.abstract_gym_b200.cspace_occupancy
 cspace_components = torch.ops.abstract_gym_b200.cspace_components
+cspace_distance = torch.ops.abstract_gym_b200.cspace_distance
+cspace_descend = torch.ops.abstract_gym_b200.cspace_descend
 step = torch.ops.abstract_gym_b200.step
 reset = torch.ops.abstract_gym_b200.reset
 rollout = torch.ops.abstract_gym_b200.rollout

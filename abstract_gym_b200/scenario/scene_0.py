@@ -26,6 +26,20 @@ def _engine(e):
     return int(e)
 
 
+def _pack_words(img):
+    """bool [n, b1, b2] -> int32 words [n, b1, ceil(b2/32)] in the layout of cspace_occupancy(packed=True): pose (i, j)
+    is bit j % 32 of word j // 32, padding bits 0"""
+    n, b1, b2 = img.shape
+    w = (b2 + 31) // 32
+    pad = torch.zeros(n, b1, w * 32, dtype=torch.uint8, device=img.device)
+    pad[..., :b2] = img
+    # one byte per 8 poses (distinct bits: the sum is an OR), then 4 little-endian bytes per word: 2 bytes of
+    # temporaries per pose
+    shifts = torch.arange(8, dtype=torch.uint8, device=img.device)
+    octets = (pad.view(n, b1, w * 4, 8) << shifts).sum(dim=-1, dtype=torch.uint8)
+    return octets.view(torch.int32)
+
+
 class BatchedScene:
     """N environments sharing one grid (or one grid per block of `envs_per_grid` envs).
 
@@ -231,25 +245,12 @@ class BatchedScene:
                                                   stream_ptr(self.device)), "ag_cspace_components")
         return (labels, nc) if count else labels
 
-    def cspace_component_of(self, labels, joints=None, lo=(0.0, 0.0), step=None, wrap=None):
-        """The label (cspace_components) at the nearest lattice pose of each of M poses, on the grid of env m
-        (((env_id0 + m) // envs_per_grid) % n_grids, as check_motion).  joints: [M, 2] float64 (default: the current
-        joints, M = N); lo, step, wrap: those of the call that made `labels`.
-        Per axis, in float64: k = floor((q - lo) / step + 0.5); on a wrapping axis k mod b, on any other k outside [0, b)
-        gives -1, and so does a NaN or infinite q.  Returns int32 [M].
-        Whether env i can reach pose t_i on the lattice: component_of(labels)[i] == component_of(labels, t)[i] >= 0."""
-        n_grids, b1, b2 = labels.shape
-        if n_grids != int(self.grid.n_grids):
-            raise ValueError("labels hold %d grids, the scene %d" % (n_grids, int(self.grid.n_grids)))
-        lo, st, w = self._lattice(b1, b2, lo, step, wrap)
-        if joints is None:
-            q = torch.stack([self.robot.joint_1, self.robot.joint_2], dim=1)
-        else:
-            q = as_f64(joints, self.device).reshape(-1, 2)
-        m = q.shape[0]
-        env = self.env_id0 + torch.arange(m, dtype=torch.int64, device=self.device)
-        g = torch.div(env, int(self.grid.envs_per_grid), rounding_mode="floor") % n_grids
-        ok = torch.ones(m, dtype=torch.bool, device=self.device)
+    @staticmethod
+    def _nearest(q, b1, b2, lo, st, w):
+        """the nearest lattice pose of each pose q [M, 2] float64: (k1, k2) int64 [M] and ok bool [M].  Per axis, in
+        float64: k = floor((q - lo) / step + 0.5); on a wrapping axis k mod b; on any other, k outside [0, b) is not ok,
+        and neither is a NaN or infinite q (k is 0 where not ok)"""
+        ok = torch.ones(q.shape[0], dtype=torch.bool, device=q.device)
         idx = []
         for a, b in enumerate((b1, b2)):
             k = torch.floor((q[:, a] - lo[a]) / st[a] + 0.5)
@@ -260,8 +261,117 @@ class BatchedScene:
             else:
                 ok &= (k >= 0) & (k < b)
             idx.append(torch.where(ok, k, 0.0).to(torch.int64))
-        out = labels.to(self.device)[g, idx[0], idx[1]]
+        return idx[0], idx[1], ok
+
+    def _snap(self, shape, joints, lo, step, wrap):
+        """grid (the env rule of check_motion), nearest lattice pose (k1, k2) and ok of each of M poses, for a per-grid
+        field of `shape` [n_grids, b1, b2] made with lo, step, wrap; joints None: the current joints (M = N)"""
+        n_grids, b1, b2 = shape
+        if n_grids != int(self.grid.n_grids):
+            raise ValueError("the field holds %d grids, the scene %d" % (n_grids, int(self.grid.n_grids)))
+        lo, st, w = self._lattice(b1, b2, lo, step, wrap)
+        if joints is None:
+            q = torch.stack([self.robot.joint_1, self.robot.joint_2], dim=1)
+        else:
+            q = as_f64(joints, self.device).reshape(-1, 2)
+        env = self.env_id0 + torch.arange(q.shape[0], dtype=torch.int64, device=self.device)
+        g = torch.div(env, int(self.grid.envs_per_grid), rounding_mode="floor") % n_grids
+        return (g,) + self._nearest(q, b1, b2, lo, st, w)
+
+    def _lookup(self, field, joints, lo, step, wrap):
+        """the entry of a per-grid lattice field at the nearest lattice pose of each of M poses, -1 off the lattice"""
+        g, k1, k2, ok = self._snap(field.shape, joints, lo, step, wrap)
+        out = field.to(self.device)[g, k1, k2]
         return torch.where(ok, out, -1).to(torch.int32)
+
+    def cspace_component_of(self, labels, joints=None, lo=(0.0, 0.0), step=None, wrap=None):
+        """The label (cspace_components) at the nearest lattice pose of each of M poses, on the grid of env m
+        (((env_id0 + m) // envs_per_grid) % n_grids, as check_motion).  joints: [M, 2] float64 (default: the current
+        joints, M = N); lo, step, wrap: those of the call that made `labels`.
+        Per axis, in float64: k = floor((q - lo) / step + 0.5); on a wrapping axis k mod b, on any other k outside [0, b)
+        gives -1, and so does a NaN or infinite q.  Returns int32 [M].
+        Whether env i can reach pose t_i on the lattice: component_of(labels)[i] == component_of(labels, t)[i] >= 0."""
+        return self._lookup(labels, joints, lo, step, wrap)
+
+    def cspace_distance(self, b1, b2=None, goals=None, lo=(0.0, 0.0), step=None, wrap=None, max_dist=False, engine=None):
+        """Steps to the goal from every lattice pose, per grid: the fewest 4-neighbour steps through free poses of
+        cspace_occupancy(b1, b2, lo, step, engine=engine) to a free goal pose (a multi-source BFS on the lattice).  The
+        lattice and wrap are those of cspace_components.
+        goals: a bool [n_grids, b1, b2] goal image; or float64 joint poses [G, 2] (goals of every grid) or
+        [n_grids, G, 2], each snapped to its nearest lattice pose by the rule of cspace_component_of (a NaN or
+        off-lattice pose seeds nothing); or None: the scene's own task -- target_j when choose_j_tar is set, else the
+        valid solutions (both elbows) of robot.inverse_kinematic(target_c, corrected=True).  A goal is the lattice pose
+        nearest each such pose, not the box that check_target_reached accepts.  Goals on colliding poses seed nothing.
+        Returns dist int32 [n_grids, b1, b2]: -1 colliding, -2 free but no goal in its component, else the steps to the
+        nearest goal (0 at a goal); with max_dist=True also int32 [n_grids], the largest distance of each grid (-1 if
+        none).  Like cspace_components this is the lattice image, not continuous joint space.  The call synchronises
+        with the current stream (it reads convergence back), so it cannot be captured in a CUDA graph."""
+        b1 = int(b1)
+        b2 = b1 if b2 is None else int(b2)
+        if b1 < 1 or b2 < 1:
+            raise ValueError("the lattice needs b1, b2 >= 1, got %d x %d" % (b1, b2))
+        lo, st, w = self._lattice(b1, b2, lo, step, wrap)
+        words = self.cspace_occupancy(b1, b2, lo=lo, step=st, packed=True, engine=engine)
+        n_grids = words.shape[0]
+        goal_words = _pack_words(self._goal_image(goals, n_grids, b1, b2, lo, st, w))
+        dist = torch.empty(n_grids, b1, b2, dtype=torch.int32, device=self.device)
+        md = torch.empty(n_grids, dtype=torch.int32, device=self.device) if max_dist else None
+        _lib.check(self._lib.ag_cspace_distance(ptr(words), ptr(goal_words), n_grids, b1, b2, w, ptr(dist), ptr(md),
+                                                stream_ptr(self.device)), "ag_cspace_distance")
+        return (dist, md) if max_dist else dist
+
+    def _goal_image(self, goals, n_grids, b1, b2, lo, st, w):
+        """bool [n_grids, b1, b2] goal image of cspace_distance's `goals` argument"""
+        if isinstance(goals, torch.Tensor) and goals.dtype == torch.bool:
+            if tuple(goals.shape) != (n_grids, b1, b2):
+                raise ValueError("a goal image must be [n_grids, b1, b2] = %s, got %s" % ((n_grids, b1, b2), tuple(goals.shape)))
+            return goals.to(self.device)
+        if goals is None:
+            if self.choose_j_tar:
+                goals = torch.tensor([[float(self.target_j[0]), float(self.target_j[1])]], dtype=torch.float64)
+            else:
+                valid, s1, s2 = self.robot.inverse_kinematic([[float(self.target_c.x), float(self.target_c.y)]], corrected=True)
+                goals = torch.cat([s1[valid], s2[valid]])
+        q = as_f64(goals, self.device)
+        if q.dim() == 2 and q.shape[1] == 2:
+            q = q.unsqueeze(0).expand(n_grids, -1, -1)
+        if q.dim() != 3 or q.shape[0] != n_grids or q.shape[2] != 2:
+            raise ValueError("goal poses must be [G, 2] or [n_grids, G, 2], got %s" % (tuple(q.shape),))
+        k1, k2, ok = self._nearest(q.reshape(-1, 2), b1, b2, lo, st, w)
+        g = torch.arange(n_grids, dtype=torch.int64, device=self.device).repeat_interleave(q.shape[1])
+        img = torch.zeros(n_grids * b1 * b2, dtype=torch.bool, device=self.device)
+        img[((g * b1 + k1) * b2 + k2)[ok]] = True
+        return img.view(n_grids, b1, b2)
+
+    def cspace_distance_of(self, dist, joints=None, lo=(0.0, 0.0), step=None, wrap=None):
+        """The distance (cspace_distance) at the nearest lattice pose of each of M poses, on the grid of env m: the rule
+        of cspace_component_of.  -1 for a colliding pose and for a pose off the lattice (or NaN), -2 where no goal is
+        reachable.  Returns int32 [M]."""
+        return self._lookup(dist, joints, lo, step, wrap)
+
+    def cspace_path(self, dist, max_len, joints=None, lo=(0.0, 0.0), step=None, wrap=None):
+        """Lattice paths down a cspace_distance field: from the nearest lattice pose of each of M poses (the snapping
+        rule of cspace_component_of, on the grid of env m), each step goes to the first neighbour, in the order
+        (i+1, j), (i-1, j), (i, j+1), (i, j-1) (across a seam only where the axis wraps), whose distance is one less,
+        until a goal or max_len poses.  joints: [M, 2] float64 (default: the current joints); lo, step, wrap: those of
+        the call that made `dist`.
+        Returns (path int32 [M, max_len], length int32 [M]).  path[m, :length[m]] are grid-local indices k = i * b2 + j,
+        then -1; index k is the joint pose lo + (k // b2, k % b2) * step.  length = min(dist + 1, max_len), 0 for a
+        start that is colliding, unreachable, off the lattice or NaN.  The walk is on the lattice image only."""
+        max_len = int(max_len)
+        if max_len < 1:
+            raise ValueError("max_len must be >= 1, got %d" % max_len)
+        n_grids, b1, b2 = dist.shape
+        g, k1, k2, ok = self._snap(dist.shape, joints, lo, step, wrap)
+        _, _, w = self._lattice(b1, b2, lo, step, wrap)
+        start = torch.where(ok, k1 * b2 + k2, -1).to(torch.int32)
+        m = start.numel()
+        path = torch.empty(m, max_len, dtype=torch.int32, device=self.device)
+        length = torch.empty(m, dtype=torch.int32, device=self.device)
+        d = dist.to(self.device, torch.int32).contiguous()
+        _lib.check(self._lib.ag_cspace_descend(ptr(d), n_grids, b1, b2, w, ptr(start), ptr(g), m, max_len, ptr(path),
+                                               ptr(length), stream_ptr(self.device)), "ag_cspace_descend")
+        return path, length
 
     def check_target_reached(self):
         """scene_0.py:115-133 -> bool [N]"""

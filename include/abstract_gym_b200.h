@@ -12,7 +12,8 @@
  *     nothing throws across the boundary; no hidden global state;
  *   - unless a name ends in _host, every pointer is a DEVICE pointer owned by the caller and all
  *     work is enqueued on `stream` (a cudaStream_t passed as void*); calls are stream-ordered,
- *     re-entrant and never synchronise;
+ *     re-entrant and never synchronise -- except ag_cspace_distance, which synchronises with its stream to
+ *     detect convergence (and so cannot be captured in a CUDA graph);
  *   - *_host entry points take HOST pointers, do their own H2D/D2H copies and return after the
  *     results are in the host buffers;
  *   - there is no CPU implementation behind any of these symbols: without a CUDA device they
@@ -27,7 +28,7 @@
 extern "C" {
 #endif
 
-#define AG_ABI_VERSION 8
+#define AG_ABI_VERSION 9
 
 #if defined(__GNUC__)
 #define AG_API __attribute__((visibility("default")))
@@ -236,6 +237,48 @@ AG_API ag_status ag_cspace_occupancy(const ag_params *p, const ag_grid *g, doubl
  * synchronisation (the counts are zeroed by a memset on `stream`): capturable in a CUDA graph. */
 AG_API ag_status ag_cspace_components(const uint32_t *bits, int64_t n_grids, int32_t b1, int32_t b2, int32_t wrap,
                                       int32_t *labels, int64_t *n_components, void *stream);
+
+/* Free-space distance: the fewest 4-neighbour steps through free poses from every pose of an occupancy image to a goal
+ * pose, per grid g = 0 .. n_grids-1 (a multi-source BFS on the lattice).  No grid or params: image work on the words.
+ * bits, goals: [n_grids][b1][W] uint32 (device, 4-byte aligned), W = ceil(b2 / 32), the layout ag_cspace_occupancy writes:
+ *       pose (i, j) is bit j % 32 of word j / 32 of row i; bits: 1 = colliding; goals: 1 = goal.  Padding bits (j >= b2)
+ *       are ignored, and so are goal bits on colliding poses: neither seeds anything.
+ * Adjacency is that of ag_cspace_components: 4 neighbours, wrap bit 0 joins row b1-1 to row 0, bit 1 column b2-1 to
+ * column 0, a pose is never its own neighbour and grids never connect.
+ * dist: [n_grids][b1][b2] int32 (device, 4-byte aligned, no padding): -1 for a colliding pose; -2 for a free pose whose
+ *       component holds no free goal; else the fewest steps to a free goal (0 at a free goal).  This distance is unique,
+ *       so the result does not depend on scheduling.
+ * max_dist: optional [n_grids] int32 (device, 4-byte aligned): the largest distance of each grid, -1 if no pose reaches a
+ *       goal; written (not accumulated).
+ * Like ag_cspace_components this is the LATTICE image: a step between adjacent free poses may cross a colliding pose in
+ * continuous joint space when the lattice is coarse (ag_check_motion checks such a step).
+ * Errors, in this order, before anything touches the device: n_grids < 0, b1 < 1 or b2 < 1, b1 * b2 > INT32_MAX - 1 or
+ * n_grids * b1 * b2 beyond int64 -> AG_ERR_SHAPE; wrap & ~3 -> AG_ERR_MODE; n_grids == 0 -> AG_OK (nothing launched);
+ * bits, goals or dist NULL -> AG_ERR_NULL; a misaligned pointer -> AG_ERR_ALIGN.
+ * THE ONE EXCEPTION to "never synchronise": this call synchronises with `stream` every few relaxation passes to learn
+ * whether the field has converged.  It returns once it has; the final pass (the -2 marks and max_dist) is enqueued on
+ * `stream` after the last synchronisation, so the results are stream-ordered like those of every other call.  On a stream
+ * that is capturing a CUDA graph it returns cudaErrorStreamCaptureUnsupported before it enqueues anything, and the
+ * capture stays intact.  Scratch memory (tile stamps, change counters) comes from cudaMallocAsync on `stream`. */
+AG_API ag_status ag_cspace_distance(const uint32_t *bits, const uint32_t *goals, int64_t n_grids, int32_t b1, int32_t b2,
+                                    int32_t wrap, int32_t *dist, int32_t *max_dist, void *stream);
+
+/* Lattice descent: m paths down a distance field of ag_cspace_distance (same n_grids, b1, b2, wrap).  Query q starts at
+ * the grid-local row-major index start[q] = i * b2 + j on grid grid[q].  path[q][0] = start; from a pose at distance
+ * d > 0 the next pose is the FIRST neighbour in the order (i+1, j), (i-1, j), (i, j+1), (i, j-1) that exists (across a
+ * seam only where that axis wraps) and has distance d - 1, so the path is canonical.  The walk stops at distance 0 or
+ * after max_len poses.
+ * dist: [n_grids][b1][b2] int32; start: [m] int32; grid: [m] int64 (8-byte aligned); path: [m][max_len] int32;
+ * length: [m] int32 -- all device arrays.  length[q] = min(dist(start) + 1, max_len), and 0 when start is outside
+ * [0, b1 * b2), grid[q] outside [0, n_grids), or the start pose is colliding or unreachable (dist < 0): these are device
+ * data, not errors.  path[q][k] = -1 for k >= length[q].
+ * Errors, in this order, before anything touches the device: n_grids < 0, b1 < 1 or b2 < 1, b1 * b2 > INT32_MAX - 1 or
+ * n_grids * b1 * b2 beyond int64, m < 0, max_len < 1 or m * max_len beyond int64 -> AG_ERR_SHAPE; wrap & ~3 ->
+ * AG_ERR_MODE; m == 0 -> AG_OK (nothing launched); dist, start, grid, path or length NULL -> AG_ERR_NULL; a misaligned
+ * pointer -> AG_ERR_ALIGN.  Stream-ordered, never synchronises: capturable in a CUDA graph. */
+AG_API ag_status ag_cspace_descend(const int32_t *dist, int64_t n_grids, int32_t b1, int32_t b2, int32_t wrap,
+                                   const int32_t *start, const int64_t *grid, int64_t m, int32_t max_len, int32_t *path,
+                                   int32_t *length, void *stream);
 
 /* K1: scenario/scene_0.py:88-103  Scene.step(action).  j1,j2,reward,flags are in/out (sticky
  * semantics).  actions: [n][2] float64 (actions_f32 == 0) or float32.  Optional outputs:
