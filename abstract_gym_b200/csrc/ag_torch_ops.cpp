@@ -38,6 +38,15 @@ void need(const Tensor &t, at::ScalarType dt, const char *name, c10::Device dev)
     TORCH_CHECK(t.is_contiguous(), name, " must be contiguous");
 }
 
+// element counts are checked before anything launches: an undersized tensor would be read or written out of bounds
+void need_numel(const Tensor &t, int64_t count, const char *name) {
+    TORCH_CHECK(t.numel() == count, name, " must have ", count, " elements, got ", t.numel());
+}
+
+void opt_numel(const OptTensor &t, int64_t count, const char *name) {
+    if (t.has_value() && t->defined()) need_numel(*t, count, name);
+}
+
 template <typename T>
 T *opt_ptr(const OptTensor &t, at::ScalarType dt, const char *name, c10::Device dev) {
     if (!t.has_value() || !t->defined()) return nullptr;
@@ -88,6 +97,7 @@ void collision_check(const Tensor &params, const Tensor &bits, const OptTensor &
     c10::cuda::CUDAGuard guard(dev);
     need(j1, at::kDouble, "j1", dev); need(j2, at::kDouble, "j2", dev); need(hit, at::kByte, "hit", dev);
     TORCH_CHECK(j2.numel() == j1.numel() && hit.numel() == j1.numel(), "j1, j2, hit must have one element per env");
+    opt_numel(first_hit, j1.numel(), "first_hit");
     const ag_params p = unpack_params(params);
     const ag_grid g = make_grid(bits, bits_t, hier, min_x, min_y, side, env_size, S, n_grids, max_occupied, envs_per_grid, dev);
     check_status(ag_collision_check(&p, &g, j1.data_ptr<double>(), j2.data_ptr<double>(), hit.data_ptr<uint8_t>(),
@@ -218,6 +228,9 @@ void step(const Tensor &params, const Tensor &bits, const OptTensor &bits_t, con
     TORCH_CHECK(actions.is_cuda() && actions.is_contiguous() && actions.numel() == 2 * n &&
                 (actions.scalar_type() == at::kFloat || actions.scalar_type() == at::kDouble),
                 "actions must be a contiguous CUDA [N,2] float32 or float64 tensor");
+    need_numel(j2, n, "j2"); need_numel(reward, n, "reward"); need_numel(flags, n, "flags");
+    opt_numel(ee, 2 * n, "ee"); opt_numel(dist, 2 * n, "dist"); opt_numel(first_hit, n, "first_hit");
+    opt_numel(stats, AG_ST_COUNT, "stats"); opt_numel(targets, 2 * n, "targets");
     const ag_params p = unpack_params(params);
     const ag_grid g = make_grid(bits, bits_t, hier, min_x, min_y, side, env_size, S, n_grids, max_occupied, envs_per_grid, dev);
     check_status(ag_step(&p, &g, j1.data_ptr<double>(), j2.data_ptr<double>(), actions.data_ptr(),
@@ -243,6 +256,8 @@ void reset(const Tensor &params, const Tensor &bits, const OptTensor &bits_t, co
         TORCH_CHECK(reset_u->dim() == 3 && reset_u->size(0) == n && reset_u->size(2) == 2, "reset_u must be [N,R,2]");
         R = (int32_t)reset_u->size(1);
     }
+    need_numel(j2, n, "j2"); need_numel(reward, n, "reward"); need_numel(flags, n, "flags"); need_numel(reset_ctr, n, "reset_ctr");
+    opt_numel(mask, n, "mask"); opt_numel(stats, AG_ST_COUNT, "stats");
     const ag_params p = unpack_params(params);
     const ag_grid g = make_grid(bits, bits_t, hier, min_x, min_y, side, env_size, S, n_grids, max_occupied, envs_per_grid, dev);
     check_status(ag_reset(&p, &g, j1.data_ptr<double>(), j2.data_ptr<double>(), reward.data_ptr<float>(), flags.data_ptr<uint8_t>(),
@@ -266,6 +281,10 @@ void rollout(const Tensor &params, const Tensor &bits, const OptTensor &bits_t, 
     need(step_ctr, at::kInt, "step_ctr", dev); need(reset_ctr, at::kInt, "reset_ctr", dev); need(ep_len, at::kInt, "ep_len", dev);
     need(stats, at::kLong, "stats", dev);
     const int64_t n = j1.numel();
+    need_numel(j2, n, "j2"); need_numel(reward, n, "reward"); need_numel(flags, n, "flags");
+    need_numel(step_ctr, n, "step_ctr"); need_numel(reset_ctr, n, "reset_ctr"); need_numel(ep_len, n, "ep_len");
+    need_numel(stats, AG_ST_COUNT, "stats"); opt_numel(diag, AG_DIAG_COUNT, "diag"); opt_numel(targets, 2 * n, "targets");
+    opt_numel(event_count, 1, "event_count");
     ag_rollout_args a = {};
     a.n = n; a.env_id0 = env_id0; a.K = (int32_t)K; a.engine = (int32_t)engine; a.seed = (uint64_t)seed;
     if (actions.has_value() && actions->defined())
