@@ -146,63 +146,6 @@ __global__ void __launch_bounds__(AG_BLOCK) k_collision(const ag_params P, const
     if (WANT_FIRST) first_hit[e] = h ? fh : -1;
 }
 
-// ------------------------------------------------------------------------------------------- K1
-// scenario/scene_0.py:88-103.  The float64 arm is always computed here (ee / dist outputs).
-template <int ENGINE, bool ACT_F32, bool WANT_FIRST>
-__global__ void __launch_bounds__(AG_BLOCK) k_step(const ag_params P, const GridDev G, double *__restrict__ j1,
-                                                   double *__restrict__ j2, const void *__restrict__ actions,
-                                                   float *__restrict__ reward, uint8_t *__restrict__ flags,
-                                                   double *__restrict__ ee, double *__restrict__ dist,
-                                                   int32_t *__restrict__ first_hit, unsigned long long *stats,
-                                                   const double *__restrict__ targets, int64_t n, int64_t env_id0) {
-    extern __shared__ __align__(16) unsigned char smem[];
-    __shared__ FastList s_fl;
-    __shared__ unsigned long long s_acc[AG_ST_COUNT];
-    if (threadIdx.x < AG_ST_COUNT) s_acc[threadIdx.x] = 0;
-    const BlockCtx B = block_prologue<ENGINE>(G, env_id0, n, smem, &s_fl);
-    __syncthreads();
-    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e < n) {
-        ag_params Pe = P;                                   // per-env cartesian target (gym-style callers), if given
-        if (targets) {
-            const double2 tg = reinterpret_cast<const double2 *>(targets)[e];
-            Pe.target_x = tg.x; Pe.target_y = tg.y;
-        }
-        double d1, d2;
-        if (ACT_F32) {
-            const float2 a = reinterpret_cast<const float2 *>(actions)[e];
-            d1 = (double)a.x; d2 = (double)a.y;
-        } else {
-            const double2 a = reinterpret_cast<const double2 *>(actions)[e];
-            d1 = a.x; d2 = a.y;
-        }
-        const double q1 = __dadd_rn(j1[e], d1), q2 = __dadd_rn(j2[e], d2);   // two_joint_robot.py:71-72
-        float rw = reward[e];
-        uint8_t fl = flags[e];
-        const Arm A = forward_kinematics(q1, q2, P.link_1, P.link_2);
-        int fh = INT_MAX, axis = 0;
-        bool h;
-        if constexpr (ENGINE == AG_ENGINE_FAST && !WANT_FIRST) {
-            const FastConst C = make_fast_const(P, G);
-            h = fast_arm_collides(P, G, B.V, B.fl, C, A, axis);
-        } else {
-            h = arm_collides<ENGINE == AG_ENGINE_BRUTE ? AG_ENGINE_BRUTE : AG_ENGINE_EXACT, WANT_FIRST>(
-                G, B.V, A, P.section_eps, fh, axis);
-        }
-        if (h) { rw = (float)P.reward_collision; fl |= AG_FLAG_COLLISION; }       // scene_0.py:95-97
-        if (target_reached(Pe, q1, q2, A)) { rw = (float)P.reward_reach; fl |= AG_FLAG_DONE; }   // :98-100
-        j1[e] = q1; j2[e] = q2; reward[e] = rw; flags[e] = fl;
-        if (ee) reinterpret_cast<double2 *>(ee)[e] = make_double2(A.gx, A.gy);
-        if (dist)
-            reinterpret_cast<double2 *>(dist)[e] =
-                make_double2(fabs(__dsub_rn(Pe.target_x, A.gx)), fabs(__dsub_rn(Pe.target_y, A.gy)));
-        if (WANT_FIRST) first_hit[e] = h ? fh : -1;
-        acc32(s_acc, AG_ST_ENV_STEPS, 1);
-        if (axis) acc32(s_acc, AG_ST_AXIS_ALIGNED, axis);
-    }
-    stats_flush(s_acc, stats);
-}
-
 // ------------------------------------------------------------------------------------------- K3
 // scenario/scene_0.py:105-113 (clear_flags) / :174-181
 template <int ENGINE, bool HAS_RESET_U>
@@ -234,93 +177,114 @@ __global__ void __launch_bounds__(AG_BLOCK) k_reset(const ag_params P, const Gri
     stats_flush(s_acc, stats);
 }
 
-// ------------------------------------------------------------------------------------------- K6
-// The gym-style step of scenario/vector_env.py in ONE launch: Scene.step (scene_0.py:88-103), the terminal
-// observation, the episode statistics and Scene.reset() of experiment_0.py:30-34 (same-step auto-reset), and the
-// observation of the pose the env continues from.  obs / final_obs: [n][AG_OBS_DIM] float64 =
-// (joint_1, joint_2, EE_x, EE_y, |target_x - EE_x|, |target_y - EE_y|); crop: optional [n][c][c] uint8 occupancy of
-// the c x c cells centred on the end effector's cell (1 = occupied, 2 = outside the grid), row 0 = top.
+// -------------------------------------------------------------------------------------- K1 / K6
+// One env step per thread: Scene.step (scene_0.py:88-103) behind ag_step, and the gym-style step of
+// scenario/vector_env.py behind ag_step_obs, which adds the terminal observation, the episode statistics and
+// Scene.reset() of experiment_0.py:30-34 (same-step auto-reset), and the observation of the pose the env continues from.
+// obs / final_obs: [n][AG_OBS_DIM] float64 = (joint_1, joint_2, EE_x, EE_y, |target_x - EE_x|, |target_y - EE_y|); crop:
+// [n][c][c] uint8 occupancy of the c x c cells centred on the end effector's cell (1 = occupied, 2 = outside the grid),
+// row 0 = top.
+struct StepDev {
+    double *j1, *j2;                       // in/out
+    const void *actions;                   // [n][2] float32 (ACT_F32) or float64
+    float *reward;                         // in/out, sticky
+    uint8_t *flags;                        // in/out, sticky
+    const double *targets;                 // optional per-env cartesian targets [n][2], or nullptr
+    unsigned long long *stats;             // or nullptr
+    int64_t n, env_id0;
+    // optional outputs of ag_step: the stepped pose's end effector and goal distances [n][2], K2's first_hit [n]
+    double *ee, *dist;
+    int32_t *first_hit;                    // WANT_FIRST only
+    // optional outputs of ag_step_obs: this step's return values, the observations, the crop; reset_ctr with auto_reset
+    uint32_t *reset_ctr, *ep_len;
+    double *obs, *final_obs;
+    float *reward_out;
+    uint8_t *terminated, *collision, *crop;
+    int32_t crop_size, auto_reset;
+    uint64_t seed;
+};
+
 __device__ __forceinline__ void write_obs(double *o, double q1, double q2, const Arm &A, double tx, double ty) {
     reinterpret_cast<double2 *>(o)[0] = make_double2(q1, q2);
     reinterpret_cast<double2 *>(o)[1] = make_double2(A.gx, A.gy);
     reinterpret_cast<double2 *>(o)[2] = make_double2(fabs(__dsub_rn(tx, A.gx)), fabs(__dsub_rn(ty, A.gy)));
 }
 
-template <int ENGINE, bool ACT_F32>
-__global__ void __launch_bounds__(AG_BLOCK) k_step_obs(const ag_params P, const GridDev G, double *__restrict__ j1,
-                                                       double *__restrict__ j2, const void *__restrict__ actions,
-                                                       float *__restrict__ reward, uint8_t *__restrict__ flags,
-                                                       uint32_t *__restrict__ reset_ctr, uint32_t *__restrict__ ep_len,
-                                                       const double *__restrict__ targets, double *__restrict__ obs,
-                                                       float *__restrict__ reward_out, uint8_t *__restrict__ terminated,
-                                                       uint8_t *__restrict__ collision, double *__restrict__ final_obs,
-                                                       uint8_t *__restrict__ crop, int crop_size, unsigned long long *stats,
-                                                       uint64_t seed, int auto_reset, int64_t n, int64_t env_id0) {
+// WANT_FIRST: the collision flag and first_hit with the EXACT (or BRUTE) arithmetic of K2; the launcher runs the EXACT
+// kernel for the FAST engine
+template <int ENGINE, bool ACT_F32, bool WANT_FIRST>
+__global__ void __launch_bounds__(AG_BLOCK) k_step(const __grid_constant__ ag_params P, const __grid_constant__ GridDev G,
+                                                   const __grid_constant__ StepDev D) {
+    static_assert(!(WANT_FIRST && ENGINE == AG_ENGINE_FAST), "first_hit runs the EXACT kernel");
     extern __shared__ __align__(16) unsigned char smem[];
     __shared__ FastList s_fl;
     __shared__ unsigned long long s_acc[AG_ST_COUNT];
     if (threadIdx.x < AG_ST_COUNT) s_acc[threadIdx.x] = 0;
-    const BlockCtx B = block_prologue<ENGINE>(G, env_id0, n, smem, &s_fl);
+    const BlockCtx B = block_prologue<ENGINE>(G, D.env_id0, D.n, smem, &s_fl);
     __syncthreads();
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e < n) {
+    if (e < D.n) {
         const FastConst C = make_fast_const(P, G);
         double tx = P.target_x, ty = P.target_y;
-        if (targets) { const double2 tg = reinterpret_cast<const double2 *>(targets)[e]; tx = tg.x; ty = tg.y; }
+        if (D.targets) { const double2 tg = reinterpret_cast<const double2 *>(D.targets)[e]; tx = tg.x; ty = tg.y; }
         double d1, d2;
-        if (ACT_F32) { const float2 a = reinterpret_cast<const float2 *>(actions)[e]; d1 = (double)a.x; d2 = (double)a.y; }
-        else { const double2 a = reinterpret_cast<const double2 *>(actions)[e]; d1 = a.x; d2 = a.y; }
-        double q1 = __dadd_rn(j1[e], d1), q2 = __dadd_rn(j2[e], d2);          // two_joint_robot.py:71-72
-        float rw = reward[e];
-        uint32_t fl = flags[e];
+        if (ACT_F32) { const float2 a = reinterpret_cast<const float2 *>(D.actions)[e]; d1 = (double)a.x; d2 = (double)a.y; }
+        else { const double2 a = reinterpret_cast<const double2 *>(D.actions)[e]; d1 = a.x; d2 = a.y; }
+        double q1 = __dadd_rn(D.j1[e], d1), q2 = __dadd_rn(D.j2[e], d2);      // two_joint_robot.py:71-72
+        float rw = D.reward[e];
+        uint32_t fl = D.flags[e];
         Arm A = forward_kinematics(q1, q2, P.link_1, P.link_2);
         int fh = INT_MAX, axis = 0;
         bool h;
         if constexpr (ENGINE == AG_ENGINE_FAST) h = fast_arm_collides(P, G, B.V, B.fl, C, A, axis);
-        else h = arm_collides<ENGINE, false>(G, B.V, A, P.section_eps, fh, axis);
+        else h = arm_collides<ENGINE, WANT_FIRST>(G, B.V, A, P.section_eps, fh, axis);
         if (h) { rw = (float)P.reward_collision; fl |= AG_FLAG_COLLISION; }      // scene_0.py:95-97
         const bool reached = P.choose_j_tar ? target_reached_joint(P, q1, q2)
                                             : (fabs(__dsub_rn(tx, A.gx)) < P.reach_eps && fabs(__dsub_rn(ty, A.gy)) < P.reach_eps);
         if (reached) { rw = (float)P.reward_reach; fl |= AG_FLAG_DONE; }         // :98-100
-        reward_out[e] = rw;
-        terminated[e] = fl != 0 ? 1 : 0;
-        collision[e] = (fl & AG_FLAG_COLLISION) ? 1 : 0;
-        if (final_obs) write_obs(final_obs + e * AG_OBS_DIM, q1, q2, A, tx, ty);
-        uint32_t el = ep_len[e] + 1;
+        if (WANT_FIRST) D.first_hit[e] = h ? fh : -1;
+        if (D.ee) reinterpret_cast<double2 *>(D.ee)[e] = make_double2(A.gx, A.gy);
+        if (D.dist) reinterpret_cast<double2 *>(D.dist)[e] = make_double2(fabs(__dsub_rn(tx, A.gx)), fabs(__dsub_rn(ty, A.gy)));
+        if (D.reward_out) D.reward_out[e] = rw;
+        if (D.terminated) D.terminated[e] = fl != 0 ? 1 : 0;
+        if (D.collision) D.collision[e] = (fl & AG_FLAG_COLLISION) ? 1 : 0;
+        if (D.final_obs) write_obs(D.final_obs + e * AG_OBS_DIM, q1, q2, A, tx, ty);
+        uint32_t el = (D.ep_len ? D.ep_len[e] : 0u) + 1;
         acc32(s_acc, AG_ST_ENV_STEPS, 1);
-        if (fl != 0 && auto_reset) {                                             // experiment_0.py:30-34
+        if (fl != 0 && D.auto_reset) {                                           // experiment_0.py:30-34
             acc32(s_acc, AG_ST_EPISODES, 1);
             if (fl & AG_FLAG_COLLISION) acc32(s_acc, AG_ST_COLLISIONS, 1);
             if (fl & AG_FLAG_DONE) acc32(s_acc, AG_ST_SUCCESSES, 1);
             atomicAdd(&s_acc[AG_ST_EP_LEN_SUM], (unsigned long long)el);
             acc32(s_acc, AG_ST_RETURN_MILLI, __float2int_rn(rw * 1e-3f));
             if (h) {                                                             // Scene.reset(): resample only while colliding
-                uint32_t rc = reset_ctr[e];
-                resample_pose<ENGINE, false>(P, G, B, C, true, q1, q2, rc, nullptr, 0, seed, (uint64_t)(env_id0 + e), s_acc);
-                reset_ctr[e] = rc;
+                uint32_t rc = D.reset_ctr[e];
+                resample_pose<ENGINE, false>(P, G, B, C, true, q1, q2, rc, nullptr, 0, D.seed, (uint64_t)(D.env_id0 + e), s_acc);
+                D.reset_ctr[e] = rc;
                 A = forward_kinematics(q1, q2, P.link_1, P.link_2);
             }
             rw = 0.0f; fl = 0; el = 0;                                           // scene_0.py:111-113
         }
         if (axis) acc32(s_acc, AG_ST_AXIS_ALIGNED, axis);
-        j1[e] = q1; j2[e] = q2; reward[e] = rw; flags[e] = (uint8_t)fl; ep_len[e] = el;
-        write_obs(obs + e * AG_OBS_DIM, q1, q2, A, tx, ty);
-        if (crop) {                                                              // local occupancy around the end effector
+        D.j1[e] = q1; D.j2[e] = q2; D.reward[e] = rw; D.flags[e] = (uint8_t)fl;
+        if (D.ep_len) D.ep_len[e] = el;
+        if (D.obs) write_obs(D.obs + e * AG_OBS_DIM, q1, q2, A, tx, ty);
+        if (D.crop) {                                                            // local occupancy around the end effector
             // the end effector's own cell, not clamped to [-1, S] as row_of / col_of do for the traversal: an arm
             // that reaches past the grid sees only cells outside it
             const int64_t r0 = (int64_t)(floor((G.half - A.gy) * G.inv_side) + 1.0), c0 = (int64_t)floor((A.gx + G.half) * G.inv_side);
-            const int hc = crop_size / 2;
-            uint8_t *o = crop + e * (int64_t)crop_size * crop_size;
-            for (int dr = 0; dr < crop_size; ++dr)
-                for (int dc = 0; dc < crop_size; ++dc) {
+            const int hc = D.crop_size / 2;
+            uint8_t *o = D.crop + e * (int64_t)D.crop_size * D.crop_size;
+            for (int dr = 0; dr < D.crop_size; ++dr)
+                for (int dc = 0; dc < D.crop_size; ++dc) {
                     const int64_t r = r0 - hc + dr, c = c0 - hc + dc;
                     uint8_t v = 2;
                     if (r >= 0 && r < G.S && c >= 0 && c < G.S) v = (B.V.bits[r * G.wpr + (c >> 5)] >> (c & 31)) & 1u;
-                    o[dr * crop_size + dc] = v;
+                    o[dr * D.crop_size + dc] = v;
                 }
         }
     }
-    stats_flush(s_acc, stats);
+    stats_flush(s_acc, D.stats);
 }
 
 // ------------------------------------------------------------------------------------------- K4
@@ -693,6 +657,26 @@ k_rollout_async(const __grid_constant__ ag_params P, const __grid_constant__ Gri
 // launches run the EXACT kernels
 constexpr int first_hit_engine(int engine) { return engine == AG_ENGINE_FAST ? AG_ENGINE_EXACT : engine; }
 
+template <int E, bool F32, bool WF>
+ag_status launch_step_k(const ag_params &P, const GridDev &G, const StepDev &D, size_t smem, cudaStream_t s) {
+    auto k = k_step<E, F32, WF>;
+    ag_status st = set_smem(k, smem);
+    if (st) return st;
+    k<<<blocks_for(D.n), AG_BLOCK, smem, s>>>(P, G, D);
+    return launched();
+}
+
+// K1 / K6: the k_step of the engine, the action dtype and first_hit (which only ag_step asks for)
+ag_status launch_step(const ag_params &P, const GridDev &G, const StepDev &D, int engine, bool f32, size_t smem,
+                      cudaStream_t s) {
+    AG_DISPATCH_ENGINE(engine, {
+        constexpr int EF = first_hit_engine(E);
+        if (D.first_hit)
+            return f32 ? launch_step_k<EF, true, true>(P, G, D, smem, s) : launch_step_k<EF, false, true>(P, G, D, smem, s);
+        return f32 ? launch_step_k<E, true, false>(P, G, D, smem, s) : launch_step_k<E, false, false>(P, G, D, smem, s);
+    });
+}
+
 template <int E, int BP, bool HA, bool HR, bool REC, bool FULL, int BLOCK>
 ag_status launch_rollout_b(const ag_params &P, const GridDev &G, const RolloutDev &A, size_t smem, cudaStream_t s) {
     auto k = k_rollout<E, BP, HA, HR, REC, FULL, BLOCK>;
@@ -940,16 +924,9 @@ ag_status ag_step(const ag_params *p, const ag_grid *g, double *j1, double *j2, 
     if (((uintptr_t)actions % (actions_f32 ? 8 : 16)) || ((uintptr_t)ee % 16) || ((uintptr_t)dist % 16) ||
         ((uintptr_t)targets % 16))
         return AG_ERR_ALIGN;
-    cudaStream_t s = (cudaStream_t)stream;
-    unsigned long long *ust = reinterpret_cast<unsigned long long *>(stats);
-#define AG_STEP(F32, WF) { auto k = k_step<(WF ? first_hit_engine(E) : E), F32, WF>; if ((st = set_smem(k, smem))) return st; \
-        k<<<blocks_for(n), AG_BLOCK, smem, s>>>(*p, G, j1, j2, actions, reward, flags, ee, dist, first_hit, ust, targets, n, env_id0); }
-    AG_DISPATCH_ENGINE(engine, {
-        if (actions_f32) { if (first_hit) AG_STEP(true, true) else AG_STEP(true, false) }
-        else             { if (first_hit) AG_STEP(false, true) else AG_STEP(false, false) }
-    });
-#undef AG_STEP
-    return launched();
+    StepDev D{j1, j2, actions, reward, flags, targets, reinterpret_cast<unsigned long long *>(stats), n, env_id0, ee, dist,
+              first_hit};
+    return launch_step(*p, G, D, engine, actions_f32 != 0, smem, (cudaStream_t)stream);
 }
 
 ag_status ag_reset(const ag_params *p, const ag_grid *g, double *j1, double *j2, float *reward, uint8_t *flags,
@@ -990,14 +967,11 @@ ag_status ag_step_obs(const ag_params *p, const ag_grid *g, double *j1, double *
         return AG_ERR_NULL;
     if (((uintptr_t)actions % (actions_f32 ? 8 : 16)) || ((uintptr_t)obs % 16) || ((uintptr_t)final_obs % 16) || ((uintptr_t)targets % 16))
         return AG_ERR_ALIGN;
-    cudaStream_t s = (cudaStream_t)stream;
-    unsigned long long *ust = reinterpret_cast<unsigned long long *>(stats);
-#define AG_SO(F32) { auto k = k_step_obs<E, F32>; if ((st = set_smem(k, smem))) return st; \
-        k<<<blocks_for(n), AG_BLOCK, smem, s>>>(*p, G, j1, j2, actions, reward, flags, reset_ctr, ep_len, targets, obs, reward_out, \
-                                                terminated, collision, final_obs, crop, crop_size, ust, seed, auto_reset, n, env_id0); }
-    AG_DISPATCH_ENGINE(engine, { if (actions_f32) AG_SO(true) else AG_SO(false) });
-#undef AG_SO
-    return launched();
+    StepDev D{j1, j2, actions, reward, flags, targets, reinterpret_cast<unsigned long long *>(stats), n, env_id0};
+    D.reset_ctr = reset_ctr; D.ep_len = ep_len; D.obs = obs; D.final_obs = final_obs; D.reward_out = reward_out;
+    D.terminated = terminated; D.collision = collision; D.crop = crop; D.crop_size = crop_size; D.auto_reset = auto_reset;
+    D.seed = seed;
+    return launch_step(*p, G, D, engine, actions_f32 != 0, smem, (cudaStream_t)stream);
 }
 
 ag_status ag_rollout(const ag_params *p, const ag_grid *g, const ag_rollout_args *a, void *stream) {

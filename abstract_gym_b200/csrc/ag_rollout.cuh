@@ -3,7 +3,7 @@
 // counter, the rollout with a row stride (ag_rollout_impl) and its dispatch to the persistent kernel.
 //
 // Each extern "C" entry point is defined next to its kernels:
-//   ag_kernels.cu      K1..K6 and the general K4 (ag_collision_check, ag_step, ag_reset, ag_step_obs, ag_rollout, ...)
+//   ag_kernels.cu      K1/K6 (one kernel), K2, K3, general K4 (ag_collision_check, ag_step, ag_reset, ag_step_obs, ag_rollout, ...)
 //   ag_rollout_lut.cu  the persistent scene_0-class K4, which ag_rollout dispatches to (launch_rollout_lut)
 //   ag_motion.cu       ag_check_motion
 //   ag_cspace.cu       ag_cspace_occupancy

@@ -1229,7 +1229,7 @@ def test_debug_bounds_build_per_family(ag, torch_):
     debug, release = _traps_per_kernel(lib), _traps_per_kernel(ag_build.LIB)
     assert sum(release.values()) == 0 and len(release) == len(debug) > 100
     # instantiations per family; a mangled name holds the length-prefixed identifier, then I for the template arguments
-    families = {"k_rollout": 40, "k_rollout_async": 8, "k_rollout_lut": 12, "k_step": 10, "k_step_obs": 6, "k_reset": 6,
+    families = {"k_rollout": 40, "k_rollout_async": 8, "k_rollout_lut": 12, "k_step": 10, "k_step_obs": 0, "k_reset": 6,
                 "k_collision": 5}
     per_family = {f: [k for k in debug if "%d%sI" % (len(f), f) in k] for f in families}
     assert {f: len(ks) for f, ks in per_family.items()} == families

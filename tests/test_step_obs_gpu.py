@@ -1,5 +1,5 @@
-"""K6 (`ag_step_obs`, csrc/ag_kernels.cu k_step_obs), the fused gym step behind VectorEnv and the torch op
-`step_obs`, against the CPU oracle on every engine, action dtype, grid form and option.
+"""K6 (`ag_step_obs`, the single-step kernel k_step of csrc/ag_kernels.cu, which ag_step shares), the fused gym step
+behind VectorEnv and the torch op `step_obs`, against the CPU oracle on every engine, action dtype, grid form and option.
 
 Two references, both in oracle/:
   * float32 actions with auto-reset: `oracle.rollout(K=1)` per step, carrying its RolloutState -- K6's step, episode
@@ -470,13 +470,13 @@ def test_vector_env_graph_equals_eager_heterogeneous(ag, torch_, oracle, engine,
     assert a["stats"][0] > 0 and a["stats"][2] > 0
 
 
-_DEMANGLED = re.compile(r"k_step_obs<\s*(\d+)\s*,\s*(true|false)\s*>")
-_MANGLED = re.compile(r"k_step_obsILi(\d+)ELb([01])E")
+_DEMANGLED = re.compile(r"(?<![A-Za-z0-9_])k_step<\s*(\d+)\s*,\s*(true|false)\s*,\s*(true|false)\s*>")
+_MANGLED = re.compile(r"6k_stepILi(\d+)ELb([01])ELb([01])E")
 
 
 def test_every_instantiation_launches(ag, torch_, oracle, ops, monkeypatch):
-    """the dispatch of ag_step_obs reaches all six k_step_obs<engine, float32 actions> instantiations, each from the
-    engine and action dtype it was asked for (kernel names from the profiler's CUDA activity)"""
+    """the dispatch of ag_step_obs reaches all six k_step<engine, float32 actions, first_hit = false> instantiations,
+    each from the engine and action dtype it was asked for (kernel names from the profiler's CUDA activity)"""
     from torch.profiler import ProfilerActivity, profile
     g = Grid(ag, torch_, oracle, "scene0", monkeypatch)
     j1, j2, acts, blocks, params = setup_case(oracle, 64, 1, "cart", False, "f64", 3)
@@ -486,13 +486,13 @@ def test_every_instantiation_launches(ag, torch_, oracle, ops, monkeypatch):
             for f32 in (False, True):
                 f = OpFront(ag, torch_, ops, g, j1, j2, params[0], None, engine, 3, True, 0, 3)
                 f.step(acts[0].astype(np.float32) if f32 else acts[0])
-                want.append((eid, f32))
+                want.append((eid, f32, False))
         torch_.cuda.synchronize()
     got = []
     for e in prof.events():
         m = _DEMANGLED.search(e.name) or _MANGLED.search(e.name)
         if m:
-            got.append((int(m.group(1)), m.group(2) in ("true", "1")))
+            got.append((int(m.group(1)), m.group(2) in ("true", "1"), m.group(3) in ("true", "1")))
     assert Counter(got) == Counter(want), got
     assert len(set(got)) == 6
 
